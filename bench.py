@@ -2,6 +2,7 @@
 """bench.py — COS option prices per second (N=128, FP64) on B200, and the reference CPU path beside it.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c1|c2|c3|c4|c5]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -39,6 +40,13 @@ Numbers on the JSON line:
                calibrations through `calibrate_many_sharded`, result gather inside the timed region.
 `--impl reference` times only the CPU path and prints the same line shape.
 `--workload c3|c4|c5|c1` make those configs the headline of the line instead (same keys).
+`--steps K` is the number of timed steps of the headline workload (calibrations for c1 / c5); `e2e` and `extra` state
+their own step counts.
+`--dump-outputs DIR` writes, after the timed steps, what the headline's last timed step returned to its caller as
+DIR/<name>.npy (float64, rank 0): c2 / c3 `prices`; c4 `params`, `spots`, `model`, `market`, `loss`; c5 the arrays of
+`calibrate_many_sharded`; c1 `parameters`, `model_prices`, `final_loss` of the last calibration.  Outputs larger than
+DUMP_BYTES are cut to the same fixed, seeded sample of rows in every array.  The inputs depend on the arguments only,
+so two builds run with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -111,6 +119,33 @@ def kernel_source_sha() -> str:
             h.update(f.encode())
             h.update(open(os.path.join(csrc, f), "rb").read())
     return h.hexdigest()[:16]
+
+
+DUMP_BYTES = 60 << 20          # --dump-outputs writes at most this much array data (64 MB with room for .npy headers)
+
+
+def output_sample(arrays: dict, budget: int = DUMP_BYTES, seed: int = 0) -> dict:
+    """float64 NumPy copies of `arrays` (NumPy arrays or torch tensors with the same number of rows): whole if they
+    fit `budget` bytes, else the same seeded sample of rows, in row order, from each."""
+    n = len(next(iter(arrays.values())))
+    row_bytes = 8 * sum(int(np.prod(a.shape[1:])) for a in arrays.values())
+    keep = budget // max(1, row_bytes)
+    idx = None if n <= keep else np.sort(np.random.default_rng(seed).choice(n, size=keep, replace=False))
+    out = {}
+    for name, a in arrays.items():
+        if isinstance(a, np.ndarray):
+            a = a if idx is None else a[idx]
+        else:                                                   # torch tensor: gather the rows where they live
+            import torch
+            a = (a if idx is None else a[torch.from_numpy(idx).to(a.device)]).cpu().numpy()
+        out[name] = np.ascontiguousarray(a, dtype=np.float64)
+    return out
+
+
+def write_outputs(path: str, arrays: dict) -> None:
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -478,8 +513,9 @@ def roofline_block(per_gpu_prices_per_s, nK, nT, N, kernel_ms, P, fp64_peak, wor
     return block
 
 
-def run_price_workload(B: Bench, wl, key):
-    """C2 / C3: value (kernel arm), e2e (host-buffer C-ABI call), roofline."""
+def run_price_workload(B: Bench, wl, key, outputs=None):
+    """C2 / C3: value (kernel arm), e2e (host-buffer C-ABI call), roofline.  `outputs` (a dict) receives the prices
+    of the last timed step."""
     torch, ctx, args = B.torch, B.ctx, B.args
     P, N, r = wl["P"], wl["N"], wl["r"]
     strikes, mats = np.array(wl["strikes"]), np.array(wl["maturities"])
@@ -517,6 +553,8 @@ def run_price_workload(B: Bench, wl, key):
     value = B.world * n_prices * args.steps / (total_ms * 1e-3)
     checksum = float(d_out.sum().item())
     checks = B.gather_floats(checksum)             # the ranks' results stay sharded; their checksums travel (NCCL)
+    if outputs is not None:
+        outputs.update(output_sample({"prices": d_out}))
 
     # ---- end-to-end arm: host buffers through the C-ABI -------------------------------------------
     np_params, np_s0, np_out = h_params.numpy(), h_s0.numpy(), h_out.numpy()
@@ -572,10 +610,11 @@ def run_price_workload(B: Bench, wl, key):
     return line
 
 
-def run_sweep(B: Bench, wl, steps, warmup):
+def run_sweep(B: Bench, wl, steps, warmup, outputs=None):
     """C4: the dataset sweep, STRONG scaling — samples [lo, hi) of the counter stream per rank (whole histories),
     drawn, priced, noised and reduced to losses on the device; the per-sample losses are all-gathered inside the
-    timed region (prices and market prices stay sharded, as a dataset writer would leave them)."""
+    timed region (prices and market prices stay sharded, as a dataset writer would leave them).  `outputs` (a dict)
+    receives this rank's samples of the last timed step."""
     torch, ctx, dist = B.torch, B.ctx, B.dist
     from dhj.shard import history_shard
     n_total, path_len = wl["P"], GEN["path_len"]
@@ -615,6 +654,8 @@ def run_sweep(B: Bench, wl, steps, warmup):
     total_ms = B.max_over_ranks(my_ms)
     value = n_total * M * steps / (total_ms * 1e-3)
     loss_mean = float((all_loss if B.world > 1 else bufs["loss"][:n]).sum().item()) / n_total
+    if outputs is not None:
+        outputs.update(output_sample({k: bufs[k][:n] for k in ("params", "spots", "model", "market", "loss")}))
     # the HBM-bound epilogue alone (market prices + per-sample loss): one sweep with it minus one without, no gather
     def timed_once(with_market):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -671,9 +712,10 @@ def run_sweep(B: Bench, wl, steps, warmup):
     }
 
 
-def run_calibrations(B: Bench, wl, steps, warmup):
+def run_calibrations(B: Bench, wl, steps, warmup, outputs=None):
     """C5: 10 000 markets x 3 starts through calibrate_many_sharded; the gather of the results (NCCL) is inside the
-    timed region.  Markets: the first 10 000 samples of the C4 dataset (noisy market prices from the device)."""
+    timed region.  Markets: the first 10 000 samples of the C4 dataset (noisy market prices from the device).
+    `outputs` (a dict) receives the per-market arrays of the last timed step."""
     dhj, ctx = B.dhj, B.ctx
     n = wl["markets"]
     data = ctx.generate(C4_SEED, 0, n, **GEN)
@@ -694,6 +736,10 @@ def run_calibrations(B: Bench, wl, steps, warmup):
         my = time.perf_counter() - t0
         times.append(B.max_over_ranks(my))
     launches = ctx.launch_count - launches0
+    if outputs is not None:
+        outputs.update(output_sample({k: np.asarray(res[k]) for k in ("x", "parameters", "final_loss", "iterations",
+                                                                      "status", "success", "best_start",
+                                                                      "model_prices")}))
     secs = float(np.median(times))
     fl = res["final_loss"]
     split = {k: res.get(k) for k in ("seconds_loss", "seconds_ask", "seconds_tell", "state_rounds", "evaluations")}
@@ -715,10 +761,11 @@ def run_calibrations(B: Bench, wl, steps, warmup):
     }
 
 
-def time_readme_calibration(ctx, repeats=5):
+def time_readme_calibration(ctx, repeats=5, outputs=None):
     """Second half of BASELINE.json's metric: seconds per 15-option calibration, the README configuration (C1):
     DoubleHestonJumpCalibrator(...).calibrate(maxiter=300, multi_start=3) through the drop-in class on the
-    reference suite's market (tests/test_suite.py:274-302)."""
+    reference suite's market (tests/test_suite.py:274-302).  `outputs` (a dict) receives the last calibration's
+    result."""
     for sub in ("models", "calibration"):
         p = os.path.join(PKG, "src", sub)
         if p not in sys.path:
@@ -738,6 +785,10 @@ def time_readme_calibration(ctx, repeats=5):
         res = cal.calibrate(maxiter=300, multi_start=3)
         times.append(time.perf_counter() - t0)
         launches = ctx.launch_count - launches0
+    if outputs is not None:
+        outputs.update(output_sample({"parameters": np.array([[res.parameters[k] for k in cal.param_names]]),
+                                      "model_prices": res.model_prices[None, :],
+                                      "final_loss": np.array([res.final_loss])}))
     # single-call latencies through the drop-in classes: a new (K, T) on every pricing() call
     p = [0.04, 2.0, 0.04, 0.3, -0.5, 0.04, 1.5, 0.04, 0.2, -0.3, 0.1, 0.0, 0.1]
     n_lat = 400
@@ -810,8 +861,9 @@ def run_b200_arm(args, wl, key):
             ref_calibration = reference_calibration_seconds()
 
     B = Bench(args)
+    outputs = {} if args.dump_outputs is not None else None
     if wl["kind"] == "price":
-        line = run_price_workload(B, wl, key)
+        line = run_price_workload(B, wl, key, outputs)
         if key == "c2":
             if rank == 0:
                 calib, latency = time_readme_calibration(B.ctx)
@@ -828,11 +880,11 @@ def run_b200_arm(args, wl, key):
                                                                          "vs_baseline")} | {"metric": v["metric"], "unit": v["unit"]}
                                  for k, v in extra.items()}
     elif wl["kind"] == "sweep":
-        line = run_sweep(B, wl, max(1, min(args.steps, 5)), max(1, min(args.warmup, 3)))
+        line = run_sweep(B, wl, args.steps, max(1, min(args.warmup, 3)), outputs)
     elif wl["kind"] == "calibrations":
-        line = run_calibrations(B, wl, max(1, min(args.steps, 5)), args.warmup)
+        line = run_calibrations(B, wl, args.steps, args.warmup, outputs)
     else:                                                   # c1
-        calib, latency = time_readme_calibration(B.ctx)
+        calib, latency = time_readme_calibration(B.ctx, repeats=args.steps, outputs=outputs)
         if ref_calibration is not None:
             calib["reference_seconds"] = ref_calibration
         line = {"metric": calib["metric"], "value": calib["value"], "unit": "s", "n_gpus": B.world, "steps": calib["repeats"],
@@ -846,20 +898,33 @@ def run_b200_arm(args, wl, key):
     if rank == 0:
         if cpu_baseline is not None:
             line["cpu_baseline"] = cpu_baseline
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     B.close()
 
 
-def main():
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline workload")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="default workload only: skip the C4 / C5 blocks")
-    args = ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline's outputs of the last timed step to DIR/<name>.npy (--impl b200)")
+    args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm keeps no outputs")
+    return args
+
+
+def main():
+    args = parse_args()
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference_arm(args, wl)
