@@ -164,6 +164,36 @@ DHJ_API int dhj_lbfgs_result(const dhj_lbfgs* opt, double* x, double* f, int32_t
 DHJ_API int dhj_lbfgs_minimize_fd(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market, const int32_t* state_market,
                                   int64_t n_states, double h, int64_t* rounds, int64_t* state_rounds, double* seconds);
 
+/* ---- analytic parameter gradient ------------------------------------------------------------
+ * Derivatives with respect to the 13 model parameters (calibrator order) are exact derivatives of the COS price with
+ * the truncation range [a, b] held at its value for the current parameters ("frozen range", the usual convention for
+ * COS sensitivities; [a, b] depends on the parameters only through the cumulants, and that dependence is below the
+ * rounding noise of a finite difference).  Every other step, including the own range of a strike whose +-0.1
+ * widening binds, is as in dhj_price_list.
+ *
+ * dhj_price_jacobian: dhj_price_list's arguments, out_price[P][M] and out_jac[P][M][13] = d price / d param (host
+ * buffers, chunked synchronously through device scratch).
+ *
+ * dhj_loss_grad: dhj_loss_fd's shapes, out_f[C] = compute_loss(x) and out_g[C][13] = the exact gradient in the
+ * unconstrained x (chain rule through the exp / tanh transform: p, 1 - rho^2 or 1 per parameter); out_f has the
+ * bits of dhj_loss_batch (same prices, same reduction order).  The Feller
+ * penalty contributes 1000 (2 sigma dsigma - 2 theta dkappa - 2 kappa dtheta) per factor whose excess
+ * sigma^2 - 2 kappa theta is > 0 and nothing otherwise (0 at the kink).  Where the loss is the 1e10 sentinel
+ * (any price NaN, inf or <= 0), g = 0.  Each state's (f, g) is formed by one thread in a fixed order: it does not
+ * depend on the other states of the call.
+ *
+ * dhj_lbfgs_minimize_grad: the dhj_lbfgs_minimize_fd loop with dhj_loss_grad as the evaluator (one loss evaluation
+ * per request).  n_states must equal the optimiser's state count (state_market[n_states]). */
+DHJ_API int dhj_price_jacobian(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride,
+                               double r, double q, const double* strike, int64_t strike_stride, const double* maturity,
+                               const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price,
+                               double* out_jac);
+DHJ_API int dhj_loss_grad(dhj_ctx* ctx, const dhj_market* market, const double* x, const int32_t* market_index,
+                          int64_t C, double* out_f, double* out_g);
+DHJ_API int dhj_lbfgs_minimize_grad(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market,
+                                    const int32_t* state_market, int64_t n_states, int64_t* rounds,
+                                    int64_t* state_rounds, double* seconds);
+
 /* Threads used by the library's host-side parallel loops (optimiser states in ask / tell, staging copies of pageable
  * buffers); 0 = all cores (default).  Several lock-step pipelines on one host divide the cores with this. */
 DHJ_API int dhj_set_host_threads(int32_t n);

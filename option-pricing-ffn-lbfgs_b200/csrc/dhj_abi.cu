@@ -14,11 +14,13 @@
 
 #include "dhj.h"
 #include "dhj_kernels.cuh"
+#include "dhj_jac.cuh"
 #include "dhj_generate.cuh"
 
 using namespace dhj;
 
 extern "C" int dhj_host_threads();      // dhj_lbfgs.cpp: threads of the host-side parallel loops
+extern "C" int dhj_lbfgs_shape(const dhj_lbfgs* opt, int64_t* n, int32_t* dim);   // dhj_lbfgs.cpp: states, dimension
 
 namespace {
 
@@ -166,7 +168,7 @@ struct dhj_ctx {
   int book_cur = 0;                           // slot of the last upload_book call
   Slot slots[kSlots];
   // loss path
-  DevBuf d_x, d_xv, d_idx, d_f, d_fg, d_counters, d_prices;
+  DevBuf d_x, d_xv, d_idx, d_f, d_fg, d_counters, d_prices, d_jac;
   PinBuf h_x, h_res;
   size_t counters_zeroed = 0;
   DevBuf d_peak;
@@ -560,7 +562,7 @@ int dhj_destroy(dhj_ctx* ctx) {
     if (b.last_use) cudaEventDestroy(b.last_use);
   }
   ctx->d_x.release(); ctx->d_xv.release(); ctx->d_idx.release(); ctx->d_f.release(); ctx->d_fg.release();
-  ctx->d_counters.release(); ctx->d_prices.release(); ctx->h_x.release(); ctx->h_res.release();
+  ctx->d_counters.release(); ctx->d_prices.release(); ctx->d_jac.release(); ctx->h_x.release(); ctx->h_res.release();
   ctx->d_peak.release();
   for (DevBuf& b : ctx->pool) b.release();
   ctx->pool.clear();
@@ -839,6 +841,179 @@ int dhj_lbfgs_minimize_fd(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market
     if (state_market)
       for (int64_t a = 0; a < na; ++a) mi[a] = state_market[idx[a]];
     rc = run_loss(ctx, market, x.data(), state_market ? mi.data() : nullptr, na, 1, h, f.data(), g.data(), nullptr);
+    if (rc) return rc;
+    const double t2 = omp_get_wtime();
+    rc = dhj_lbfgs_tell(opt, na, f.data(), g.data());
+    if (rc) return fail(ctx, rc, "dhj_lbfgs_tell failed (%d)", rc);
+    t_loss += t2 - t1;
+    t_tell += omp_get_wtime() - t2;
+    ++n_rounds;
+    n_state_rounds += na;
+  }
+  if (rounds) *rounds = n_rounds;
+  if (state_rounds) *state_rounds = n_state_rounds;
+  if (seconds) { seconds[0] = t_ask; seconds[1] = t_loss; seconds[2] = t_tell; }
+  return DHJ_OK;
+}
+
+// ---- analytic parameter gradient (dhj_jac.cuh) -------------------------------------------------------
+static int launch_jac(dhj_ctx* ctx, const SliceView& v, const JacArgs& a, cudaStream_t st) {
+  const long long blocks = (a.P * (long long)v.n_slices + kJacWarps - 1) / kJacWarps;
+  k_price_jac<<<(int)std::max<long long>(1, std::min(blocks, 2147483647LL)), 32 * kJacWarps, 0, st>>>(v, a);
+  DHJ_CUDA(ctx, cudaGetLastError());
+  ctx->launches++;
+  return DHJ_OK;
+}
+
+int dhj_price_jacobian(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride, double r,
+                       double q, const double* strike, int64_t strike_stride, const double* maturity,
+                       const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price, double* out_jac) {
+  int rc = check_common(ctx, params, P, S0, N, L, out_price);
+  if (rc) return rc;
+  if (!out_jac) return fail(ctx, DHJ_ERR_ARG, "null array argument");
+  if (M < 0) return fail(ctx, DHJ_ERR_ARG, "M must be >= 0");
+  if (M == 0 || P == 0) return DHJ_OK;
+  if (!strike || !maturity || !is_call) return fail(ctx, DHJ_ERR_ARG, "null option table");
+  if (s0_stride != 0 && s0_stride != 1) return fail(ctx, DHJ_ERR_ARG, "s0_stride must be 0 or 1");
+  if (strike_stride != 0 && strike_stride != M) return fail(ctx, DHJ_ERR_ARG, "strike_stride must be 0 or M");
+  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
+  BookHost book;
+  book.group(maturity, is_call, M);
+  SliceView v;
+  rc = upload_book(ctx, book, strike_stride ? nullptr : strike, strike_stride ? 0 : M, ctx->stream, &v);
+  if (rc) return rc;
+  v.scale_by_spot = 0; v.n_cos = N; v.r = r; v.q = q; v.L = L;
+  // synchronous chunks of ~32 MB through the staging buffers (throughput of this entry point is not a goal)
+  const size_t row_in = kNumParams + (s0_stride ? 1 : 0) + (strike_stride ? (size_t)M : 0);
+  const size_t row_out = (size_t)M * kJacChannels;
+  const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(P, (int64_t)(((size_t)1 << 22) / (row_in + row_out))));
+  const size_t in_bytes = (size_t)chunk * row_in * sizeof(double) + sizeof(double);
+  const size_t out_bytes = (size_t)chunk * row_out * sizeof(double);
+  DHJ_CUDA(ctx, ctx->h_x.reserve(in_bytes));
+  DHJ_CUDA(ctx, ctx->d_x.reserve(in_bytes));
+  DHJ_CUDA(ctx, ctx->d_jac.reserve(out_bytes));
+  DHJ_CUDA(ctx, ctx->h_res.reserve(out_bytes));
+  for (int64_t lo = 0; lo < P; lo += chunk) {
+    const int64_t n = std::min(chunk, P - lo);
+    const size_t pb = (size_t)n * kNumParams * sizeof(double);
+    const size_t s0b = s0_stride ? (size_t)n * sizeof(double) : sizeof(double);
+    const size_t kb = strike_stride ? (size_t)n * M * sizeof(double) : 0;
+    unsigned char* hin = (unsigned char*)ctx->h_x.p;
+    unsigned char* din = (unsigned char*)ctx->d_x.p;
+    host_copy(hin, params + lo * kNumParams, pb);
+    host_copy(hin + pb, s0_stride ? S0 + lo : S0, s0b);
+    if (kb) host_copy(hin + pb + s0b, strike + lo * (int64_t)M, kb);
+    DHJ_CUDA(ctx, cudaMemcpyAsync(din, hin, pb + s0b + kb, cudaMemcpyHostToDevice, ctx->stream));
+    SliceView vv = v;
+    if (strike_stride) { vv.strike = (const double*)(din + pb + s0b); vv.strike_stride = M; }
+    double* d_out = (double*)ctx->d_jac.p;
+    JacArgs a;
+    a.params = (const double*)din; a.S0 = (const double*)(din + pb); a.s0_stride = s0_stride ? 1 : 0;
+    a.row_index = nullptr; a.P = n; a.out_price = d_out; a.out_jac = d_out + n * (int64_t)M;
+    rc = launch_jac(ctx, vv, a, ctx->stream);
+    if (rc) return rc;
+    const size_t ob = (size_t)n * row_out * sizeof(double);
+    DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, d_out, ob, cudaMemcpyDeviceToHost, ctx->stream));
+    DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    const double* res = (const double*)ctx->h_res.p;
+    host_copy(out_price + lo * (int64_t)M, res, (size_t)n * M * sizeof(double));
+    host_copy(out_jac + lo * (int64_t)M * kNumParams, res + n * (int64_t)M, (size_t)n * M * kNumParams * sizeof(double));
+  }
+  return book_used(ctx, ctx->stream);
+}
+
+// f and the analytic g of B loss evaluations: exp/tanh transform (k_fd_expand without a stencil) -> prices of every
+// market option by the pricing kernel (the split loss path's launch: f below has the bits of dhj_loss_batch) and their
+// Jacobian (k_price_jac) -> one thread per state (k_loss_grad_reduce).  States are cut into launches of bounded scratch;
+// each state's (f, g) is computed by one thread in a fixed order, so it does not depend on the cut or on the other
+// states of the call.
+static int run_loss_grad(dhj_ctx* ctx, const dhj_market* mk, const double* x, const int32_t* market_index, int64_t B,
+                         double* out_f, double* out_g) {
+  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
+  const int* d_index = nullptr;
+  int rc = stage_x(ctx, mk, x, market_index, B, &d_index);
+  if (rc) return rc;
+  if (!out_f || !out_g) return fail(ctx, DHJ_ERR_ARG, "null output");
+  if (B == 0) return DHJ_OK;
+  const int M = mk->M;
+  const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(B, (int64_t)(((size_t)1 << 27) / ((size_t)M * kJacChannels))));
+  DHJ_CUDA(ctx, ctx->d_xv.reserve((size_t)B * kNumParams * sizeof(double)));
+  DHJ_CUDA(ctx, ctx->d_idx.reserve((size_t)B * sizeof(int)));
+  DHJ_CUDA(ctx, ctx->d_fg.reserve((size_t)B * kFdPoints * sizeof(double)));
+  DHJ_CUDA(ctx, ctx->d_prices.reserve((size_t)2 * chunk * M * sizeof(double)));   // pricing kernel | k_price_jac
+  DHJ_CUDA(ctx, ctx->d_jac.reserve((size_t)chunk * M * kNumParams * sizeof(double)));
+  double* pv = (double*)ctx->d_xv.p;
+  int* idx = (int*)ctx->d_idx.p;
+  double* fg = (double*)ctx->d_fg.p;
+  k_fd_expand<<<(unsigned)((B + 127) / 128), 128, 0, ctx->stream>>>((const double*)ctx->d_x.p, d_index, B, 0, 0.0, pv,
+                                                                   idx);
+  DHJ_CUDA(ctx, cudaGetLastError());
+  ctx->launches++;
+  for (int64_t lo = 0; lo < B; lo += chunk) {
+    const int64_t n = std::min(chunk, B - lo);
+    double* prices = (double*)ctx->d_prices.p;
+    PriceArgs pa;
+    pa.params = pv + lo * kNumParams; pa.S0 = (const double*)mk->d_S0.p; pa.s0_stride = 1; pa.row_index = idx + lo;
+    pa.P = n; pa.transform = 0; pa.out = prices;
+    rc = launch_price(ctx, mk->view, pa, mk->book.max_slice, ctx->stream);
+    if (rc) return rc;
+    JacArgs a;
+    a.params = pa.params; a.S0 = pa.S0; a.s0_stride = 1; a.row_index = pa.row_index;
+    a.P = n; a.out_price = prices + n * (int64_t)M; a.out_jac = (double*)ctx->d_jac.p;
+    rc = launch_jac(ctx, mk->view, a, ctx->stream);
+    if (rc) return rc;
+    k_loss_grad_reduce<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(
+        prices, a.out_jac, a.params, a.row_index, (const double*)mk->d_price.p, mk->view.pos, M, n,
+        fg + lo * kFdPoints);
+    DHJ_CUDA(ctx, cudaGetLastError());
+    ctx->launches++;
+  }
+  const size_t res_bytes = (size_t)B * kFdPoints * sizeof(double);
+  DHJ_CUDA(ctx, ctx->h_res.reserve(res_bytes));
+  DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, fg, res_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  const double* res = (const double*)ctx->h_res.p;
+#pragma omp parallel for schedule(static) num_threads(copy_threads()) if (B >= 4096)
+  for (int64_t c = 0; c < B; ++c) {
+    out_f[c] = res[c * kFdPoints];
+    memcpy(out_g + c * kNumParams, res + c * kFdPoints + 1, kNumParams * sizeof(double));
+  }
+  return DHJ_OK;
+}
+
+int dhj_loss_grad(dhj_ctx* ctx, const dhj_market* market, const double* x, const int32_t* market_index, int64_t C,
+                  double* out_f, double* out_g) {
+  if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
+  return run_loss_grad(ctx, market, x, market_index, C, out_f, out_g);
+}
+
+int dhj_lbfgs_minimize_grad(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market, const int32_t* state_market,
+                            int64_t n_states, int64_t* rounds, int64_t* state_rounds, double* seconds) {
+  if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
+  if (!opt || !market) return fail(ctx, DHJ_ERR_ARG, "null optimiser or market");
+  int64_t n_opt = 0;
+  int32_t dim = 0;
+  dhj_lbfgs_shape(opt, &n_opt, &dim);
+  // the buffers below receive up to every state of the optimiser per ask
+  if (n_states != n_opt) return fail(ctx, DHJ_ERR_ARG, "n_states (%lld) != the optimiser's state count (%lld)",
+                                     (long long)n_states, (long long)n_opt);
+  if (dim != kNumParams) return fail(ctx, DHJ_ERR_ARG, "the optimiser's dimension is %d, not %d", dim, kNumParams);
+  std::vector<int64_t> idx((size_t)n_states);
+  std::vector<int32_t> mi((size_t)n_states);
+  std::vector<double> x((size_t)n_states * kNumParams), f((size_t)n_states), g((size_t)n_states * kNumParams);
+  int64_t n_rounds = 0, n_state_rounds = 0;
+  double t_ask = 0.0, t_loss = 0.0, t_tell = 0.0;
+  for (;;) {
+    const double t0 = omp_get_wtime();
+    int64_t na = 0;
+    int rc = dhj_lbfgs_ask(opt, &na, idx.data(), x.data());
+    if (rc) return fail(ctx, rc, "dhj_lbfgs_ask failed (%d)", rc);
+    const double t1 = omp_get_wtime();
+    t_ask += t1 - t0;
+    if (na == 0) break;
+    if (state_market)
+      for (int64_t a = 0; a < na; ++a) mi[a] = state_market[idx[a]];
+    rc = run_loss_grad(ctx, market, x.data(), state_market ? mi.data() : nullptr, na, f.data(), g.data());
     if (rc) return rc;
     const double t2 = omp_get_wtime();
     rc = dhj_lbfgs_tell(opt, na, f.data(), g.data());

@@ -396,6 +396,13 @@ int dhj_lbfgs_tell(dhj_lbfgs* o, int64_t n_active, const double* f, const double
   return DHJ_OK;
 }
 
+// library-internal (not in dhj.h): state count and dimension, for callers that size buffers per ask
+int dhj_lbfgs_shape(const dhj_lbfgs* o, int64_t* n, int32_t* dim) {
+  if (!o || !n || !dim) return DHJ_ERR_ARG;
+  *n = o->n; *dim = o->dim;
+  return DHJ_OK;
+}
+
 int dhj_lbfgs_result(const dhj_lbfgs* o, double* x, double* f, int32_t* nit, int32_t* nfev, int32_t* status) {
   if (!o) return DHJ_ERR_ARG;
   for (int64_t i = 0; i < o->n; ++i) {

@@ -280,6 +280,127 @@ DHJ_HD void cf_exponent(const SetConsts& s, double u, double T, double lamT, con
   }, xr_out, xi_out);
 }
 
+// ---- parameter tangents of the CF exponent (analytic gradient, dhj_jac.cuh) ------------------------------------
+// Forward-mode derivatives of X with respect to the 13 model parameters at one real u, with the truncation range
+// held fixed (the price is linear in exp(X), so dV/dp_i is the COS contraction of Re(dX/dp_i e^{X - iua})).
+struct Cplx { double r, i; };
+DHJ_HD Cplx c_add(Cplx a, Cplx b) { return {a.r + b.r, a.i + b.i}; }
+DHJ_HD Cplx c_sub(Cplx a, Cplx b) { return {a.r - b.r, a.i - b.i}; }
+DHJ_HD Cplx c_mul(Cplx a, Cplx b) { return {fma(a.r, b.r, -(a.i * b.i)), fma(a.r, b.i, a.i * b.r)}; }
+DHJ_HD Cplx c_scale(Cplx a, double f) { return {a.r * f, a.i * f}; }
+
+// Factor j: the same value arithmetic as heston_factor (same bits, without the warp vote: both branches of the csqrt
+// are formed), plus dX/d(v0_j, kappa_j, theta_j, sigma_j, rho_j) -> dX[0..4].  With z_p = dz/dp etc.:
+//   d_p = z_p / (2d),  E_p = -T d_p E,  m_p = beta_p - d_p,  pl_p = beta_p + d_p,  D_p = pl_p - m_p E - m E_p
+//   B = -u (u+i) (1-E) / D             B_p = u (u+i) (E_p + (1-E) D_p/D) / D
+//   Ahat = m T - 2 log(D / (2d))       Ahat_p = m_p T - 2 (D_p/D - d_p/d)
+//   A = c Ahat, c = kappa theta / sigma^2:  dX/dv0 = B,  dX/dtheta = (kappa/sigma^2) Ahat,
+//   dX/dp = c_p Ahat + c Ahat_p + v0 B_p  for p = kappa (c_p = c/kappa), sigma (c_p = -2c/sigma), rho (c_p = 0)
+DHJ_HD void heston_factor_tangents(const Params& mp, const SetConsts& s, int j, double u, double T,
+                                   const fm::Tables* __restrict__ ltab, double& aR, double& aI, double& sli,
+                                   double& xbr, double& xbi, Cplx* dX) {
+  const double kap = s.kappa[j];
+  const double bi = -(s.rs[j] * u);
+  const double s2u = s.s2[j] * u;
+  const double zr = fma(s2u, u, fma(-bi, bi, s.kk[j]));
+  const double zi = fma(s.two_kappa[j], bi, s2u);
+  const double n2 = fma(zr, zr, zi * zi);
+  const double h = n2 * fm::rsqrt(n2);
+  const double x2 = 0.5 * (h + fabs(zr));
+  const double yt = fm::rsqrt(x2);
+  const double t = x2 * yt;
+  const double other = (0.5 * zi) * yt;
+  const bool pos = !(zr < 0.0);
+  const double dr = pos ? t : fabs(other);
+  const double di = pos ? other : copysign(t, zi);
+  const double er = fm::exp_tab_neg_ix(-dr * T, ltab);
+  double sn, cs;
+  fm::sincos_(-di * T, &sn, &cs);
+  const double Er = er * cs, Ei = er * sn;
+  const double mr = kap - dr, mi = bi - di;
+  const double pr = kap + dr, pi_ = bi + di;
+  const double Dr = fma(-mr, Er, fma(mi, Ei, pr));
+  const double Di = fma(-mr, Ei, fma(-mi, Er, pi_));
+  const double nD = fma(Dr, Dr, Di * Di);
+  const double inD = fm::rcp(nD);
+  const double ar = 1.0 - Er, ai = -Ei;
+  const double Nr = fma(ar, Dr, ai * Di), Ni = fma(ai, Dr, -(ar * Di));
+  const double Mr = fma(Nr, u, -Ni), Mi = fma(Ni, u, Nr);
+  const double g = -((s.v0[j] * u) * inD);
+  xbr = fma(Mr, g, xbr);
+  xbi = fma(Mi, g, xbi);
+  const double L = fm::log_tab<false>(h * inD, ltab, 2);
+  const double li = fm::atan2_tab_nz(fma(Di, dr, -(Dr * di)), fma(Dr, dr, Di * di), ltab);
+  const double cT = s.c[j] * T;
+  aR = fma(s.c[j], L, aR);
+  aR = fma(cT, mr, aR);
+  aI = fma(cT, mi, aI);
+  sli = fma(s.c[j], li, sli);
+
+  // tangents
+  const Cplx E = {Er, Ei}, m = {mr, mi}, omE = {ar, ai};
+  const Cplx uu = {u * u, u};                                  // u (u + i)
+  const Cplx invD = {Dr * inD, -(Di * inD)};                   // 1/D
+  const double ih = fm::rcp(h);
+  const Cplx inv2d = {(0.5 * dr) * ih, -((0.5 * di) * ih)};    // 1/(2d) = conj(d) / (2|z|)
+  const Cplx invd = {dr * ih, -(di * ih)};                     // 1/d
+  const double mB = -u * inD;
+  const Cplx B = {Mr * mB, Mi * mB};                           // B_j = (B_j v0_j) / v0_j without the division
+  const Cplx Ahat = {fma(mr, T, L), fma(mi, T, -2.0 * li)};
+  dX[0] = B;
+  dX[2] = c_scale(Ahat, fm::div(kap, s.s2[j]));
+  const double rho = mp.rho[j], sig = mp.sigma[j];
+  const Cplx beta = {kap, bi};
+  Cplx bp[3];                                                  // d beta / d(kappa, sigma, rho)
+  bp[0] = {1.0, 0.0};
+  bp[1] = {0.0, -(rho * u)};
+  bp[2] = {0.0, -(sig * u)};
+  const double cp[3] = {fm::div(s.c[j], kap), fm::div(-2.0 * s.c[j], sig), 0.0};
+  const int slot[3] = {1, 3, 4};
+#pragma unroll
+  for (int q = 0; q < 3; ++q) {
+    Cplx zp = c_scale(c_mul(beta, bp[q]), 2.0);
+    if (q == 1) { zp.r = fma(2.0 * sig, u * u, zp.r); zp.i = fma(2.0 * sig, u, zp.i); }
+    const Cplx dp = c_mul(zp, inv2d);
+    const Cplx Ep = c_scale(c_mul(dp, E), -T);
+    const Cplx mp_ = c_sub(bp[q], dp), plp = c_add(bp[q], dp);
+    const Cplx Dp = c_sub(c_sub(plp, c_mul(mp_, E)), c_mul(m, Ep));
+    const Cplx DpD = c_mul(Dp, invD);
+    const Cplx Bp = c_mul(c_mul(uu, c_add(Ep, c_mul(omE, DpD))), invD);
+    const Cplx Ahp = c_sub(c_scale(mp_, T), c_scale(c_sub(DpD, c_mul(dp, invd)), 2.0));
+    const Cplx Ap = c_add(c_scale(Ahat, cp[q]), c_scale(Ahp, s.c[j]));
+    dX[slot[q]] = c_add(Ap, c_scale(Bp, s.v0[j]));
+  }
+}
+
+// X at u (the same value arithmetic as cf_exponent) and dX/dp_i for the 13 parameters in calibrator order.
+//   jump / drift:  dX/dlam = T (J - 1) - i u T (C - 1),  dX/dmu = i u lam T (J - C),
+//                  dX/dsj = -lam T sj (i u C + u^2 J),   J = exp(i u mu - sj^2 u^2 / 2),  C = exp(mu + sj^2 / 2)
+DHJ_HD void cf_exponent_tangents(const Params& mp, const SetConsts& s, double u, double T,
+                                 const fm::Tables* __restrict__ ltab, double* xr_out, double* xi_out,
+                                 Cplx* dX) {
+  const double lamT = s.lam * T;
+  double aR = 0.0, aI = (s.drift * u) * T, sli = 0.0, xbr = 0.0, xbi = 0.0;
+  heston_factor_tangents(mp, s, 0, u, T, ltab, aR, aI, sli, xbr, xbi, dX);
+  heston_factor_tangents(mp, s, 1, u, T, ltab, aR, aI, sli, xbr, xbi, dX + 5);
+  double xr = aR + xbr;
+  double xi = fma(-2.0, sli, aI) + xbi;
+  double cj, sj;
+  fm::sincos_(u * s.mu, &sj, &cj);
+  const double ej = jump_gauss(s, u, ltab);
+  xr = fma(lamT, fma(ej, cj, -1.0), xr);
+  xi = fma(lamT, ej * sj, xi);
+  *xr_out = xr; *xi_out = xi;
+  const double Jr = ej * cj, Ji = ej * sj;
+  const double C = fm::exp_(s.mu + s.hsj2);
+  const double uT = u * T;
+  dX[10] = {T * (Jr - 1.0), fma(-uT, C - 1.0, T * Ji)};
+  const double ulT = u * lamT;
+  dX[11] = {-(ulT * Ji), ulT * (Jr - C)};
+  const double lts = lamT * mp.sj, u2 = u * u;
+  dX[12] = {-(lts * (u2 * Jr)), -(lts * fma(u, C, u2 * Ji))};
+}
+
 // everything the strike loop needs for one k
 struct KTerm {
   double G;      // w_k Re(phi(u_k) e^{-i u_k a}), w_0 = 1/2     double_heston.py:187-188

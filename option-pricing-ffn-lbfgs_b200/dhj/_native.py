@@ -26,6 +26,7 @@ EXPORTS = (
     "dhj_cf", "dhj_cf_complex", "dhj_truncation_range", "dhj_chi_psi", "dhj_fp64_peak",
     "dhj_lbfgs_create", "dhj_lbfgs_destroy", "dhj_lbfgs_ask", "dhj_lbfgs_tell", "dhj_lbfgs_result", "dhj_lbfgs_minimize_fd",
     "dhj_generator_draws", "dhj_generate_dev", "dhj_generate", "dhj_set_host_threads", "dhj_debug_checks",
+    "dhj_price_jacobian", "dhj_loss_grad", "dhj_lbfgs_minimize_grad",
 )
 
 
@@ -93,6 +94,11 @@ def load_library(path: str | None = None) -> ctypes.CDLL:
         lib.dhj_lbfgs_result.argtypes = [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp]
         lib.dhj_lbfgs_minimize_fd.argtypes = [_c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_f64, ctypes.POINTER(_c_i64),
                                               ctypes.POINTER(_c_i64), _F64]
+        lib.dhj_price_jacobian.argtypes = [_c_vp, _F64, _c_i64, _F64, _c_i64, _c_f64, _c_f64, _F64, _c_i64, _F64,
+                                           _I32, _c_i32, _c_i32, _c_f64, _c_vp, _c_vp]
+        lib.dhj_loss_grad.argtypes = [_c_vp, _c_vp, _F64, _c_vp, _c_i64, _F64, _F64]
+        lib.dhj_lbfgs_minimize_grad.argtypes = [_c_vp, _c_vp, _c_vp, _c_vp, _c_i64, ctypes.POINTER(_c_i64),
+                                                ctypes.POINTER(_c_i64), _F64]
         _U32 = ndpointer(dtype=np.uint32, flags="C_CONTIGUOUS")
         lib.dhj_generator_draws.argtypes = [_U32, _c_i32, _c_i32, _c_f64, _c_i64, _c_i32, _F64, _F64, _c_f64, _c_f64,
                                             _c_f64, _c_f64, _c_f64, _c_i32, _F64, _F64, _F64, _U32,
@@ -171,6 +177,39 @@ class Context:
         return n.value
 
     # -- pricing ----------------------------------------------------------------------------------
+    def price_jacobian(self, params, S0, strike, maturity, is_call, r, q=0.0, N=128, L=10.0):
+        """(prices float64[P, M], jac float64[P, M, 13]) of P parameter sets on an option list: jac[p, o, i] =
+        d price / d param_i with the truncation range held at its value for the current parameters
+        (dhj_price_jacobian)."""
+        params, P, S0, s0_stride, strike, k_stride, maturity, M, call = self._option_list(params, S0, strike, maturity,
+                                                                                        is_call)
+        prices, jac = np.empty((P, M)), np.empty((P, M, N_PARAMS))
+        with self._lock:
+            self._check(self._lib.dhj_price_jacobian(self._h, params, P, S0, s0_stride, float(r), float(q), strike,
+                                                     k_stride, maturity, call, M, int(N), float(L), _ptr(prices),
+                                                     _ptr(jac)), "dhj_price_jacobian")
+        return prices, jac
+
+    @staticmethod
+    def _option_list(params, S0, strike, maturity, is_call):
+        params = _f64(params).reshape(-1, N_PARAMS)
+        P = params.shape[0]
+        maturity = _f64(maturity).reshape(-1)
+        M = maturity.shape[0]
+        S0 = _f64(S0).reshape(-1)
+        if S0.size not in (1, P):
+            raise ValueError("S0 must be a scalar or have one entry per parameter set")
+        s0_stride = 0 if S0.size == 1 else 1
+        strike = _f64(strike)
+        if strike.size == M:
+            strike, k_stride = strike.reshape(M), 0
+        elif strike.size == P * M:
+            strike, k_stride = strike.reshape(P, M), M
+        else:
+            raise ValueError("strike must be [M] or [P, M]")
+        call = np.ascontiguousarray(np.broadcast_to(np.asarray(is_call), (M,)).astype(bool).astype(np.int32))
+        return params, P, S0, s0_stride, strike, k_stride, maturity, M, call
+
     def price_list(self, params, S0, strike, maturity, is_call, r, q=0.0, N=128, L=10.0) -> np.ndarray:
         """Prices float64[P, M] of P parameter sets on an option list (dhj_price_list)."""
         params = _f64(params).reshape(-1, N_PARAMS)
@@ -388,6 +427,18 @@ class Market:
                                         f_all.ctypes.data if want_all else None), "dhj_loss_fd")
         return (f, g, f_all) if want_all else (f, g)
 
+    def loss_grad(self, x, market_index=None):
+        """(f[C], g[C,13]): the loss and its exact gradient in the unconstrained x (dhj_loss_grad; truncation range
+        held fixed, g = 0 where f is the 1e10 sentinel)."""
+        x = _f64(x).reshape(-1, N_PARAMS)
+        C = x.shape[0]
+        idx, pidx = self._index(market_index, C)
+        f, g = np.empty(C), np.empty((C, N_PARAMS))
+        c = self.ctx
+        with c._lock:
+            c._check(c._lib.dhj_loss_grad(c._h, self._h, x, pidx, C, f, g), "dhj_loss_grad")
+        return f, g
+
     def prices(self, x, market_index=None) -> np.ndarray:
         x = _f64(x).reshape(-1, N_PARAMS)
         B = x.shape[0]
@@ -464,6 +515,19 @@ class BatchLBFGS:
             c._check(self._lib.dhj_lbfgs_minimize_fd(self._h, c._h, market._h, None if sm is None else sm.ctypes.data,
                                                      self.n, float(h), ctypes.byref(rounds), ctypes.byref(state_rounds),
                                                      secs), "dhj_lbfgs_minimize_fd")
+        return rounds.value, state_rounds.value, tuple(secs)
+
+    def minimize_grad(self, market: "Market", state_market=None):
+        """minimize_fd with the analytic gradient (dhj_lbfgs_minimize_grad): every round one `dhj_loss_grad` call,
+        one loss evaluation per request.  Returns (rounds, state_rounds, (seconds in ask, loss, tell))."""
+        sm = None if state_market is None else np.ascontiguousarray(np.asarray(state_market, dtype=np.int32).reshape(self.n))
+        rounds, state_rounds, secs = _c_i64(), _c_i64(), np.zeros(3)
+        c = market.ctx
+        with c._lock:
+            c._check(self._lib.dhj_lbfgs_minimize_grad(self._h, c._h, market._h,
+                                                       None if sm is None else sm.ctypes.data, self.n,
+                                                       ctypes.byref(rounds), ctypes.byref(state_rounds), secs),
+                     "dhj_lbfgs_minimize_grad")
         return rounds.value, state_rounds.value, tuple(secs)
 
     def result(self):

@@ -189,8 +189,16 @@ class DoubleHestonJumpCalibrator:
         self._track(loss)
         return loss
 
-    def compute_loss_and_grad(self, x: np.ndarray):
-        """f(x) and scipy's 2-point forward-difference gradient (h = 1e-8) in ONE launch."""
+    def compute_loss_and_grad(self, x: np.ndarray, gradient: str = "fd"):
+        """f(x) and scipy's 2-point forward-difference gradient (h = 1e-8) in ONE launch.  gradient="analytic": the
+        exact gradient instead (truncation range held fixed, g = 0 at the 1e10 sentinel); `n_calls` advances by 1."""
+        if gradient == "analytic":
+            f, g = self._device_market().loss_grad(np.asarray(x, dtype=np.float64).reshape(1, 13))
+            self.n_calls += 1
+            self._track(f[0])
+            return f[0], g[0]
+        if gradient != "fd":
+            raise ValueError(f"gradient must be 'fd' or 'analytic' (got {gradient!r})")
         f, g, f_all = self._device_market().loss_fd(np.asarray(x, dtype=np.float64).reshape(1, 13), _FD_STEP,
                                                     want_all=True)
         self.n_calls += 14
@@ -233,17 +241,23 @@ class DoubleHestonJumpCalibrator:
 
     # -- optimiser driver (:236-336) ----------------------------------------------------------------
     @staticmethod
-    def _minimize(fun_and_grad, x0, maxiter):
+    def _minimize(fun_and_grad, x0, maxiter, maxfun=_MAXFUN_REQUESTS):
         return minimize(fun=fun_and_grad, x0=x0, jac=True, method='L-BFGS-B',
-                        options={'maxiter': maxiter, 'ftol': 1e-9, 'gtol': 1e-6, 'maxfun': _MAXFUN_REQUESTS})
+                        options={'maxiter': maxiter, 'ftol': 1e-9, 'gtol': 1e-6, 'maxfun': maxfun})
 
-    def calibrate(self, maxiter: int = 300, multi_start: int = 3, *, x0=None) -> CalibrationResult:
+    def calibrate(self, maxiter: int = 300, multi_start: int = 3, *, x0=None, gradient: str = "fd") -> CalibrationResult:
         """Calibrate to the market prices with `multi_start` L-BFGS-B runs; the best (lowest loss) wins.
 
         `x0` (keyword-only extension, not in the reference): optional unconstrained starting points
         [multi_start, 13] replacing the built-in guesses — the warm-start hook for an FFN predictor
         (docs/METHODOLOGY.md:112-134 of the reference describes that pipeline; its code is not in the repo).
+
+        `gradient` (keyword-only extension): "fd" (default) is the reference's forward difference; "analytic" answers
+        each scipy request with the exact gradient of the loss (one evaluation, `n_calls` + 1 per request, scipy's
+        default maxfun = 15000 requests).
         """
+        if gradient not in ("fd", "analytic"):
+            raise ValueError(f"gradient must be 'fd' or 'analytic' (got {gradient!r})")
         start_time = time.time()
         market = self._device_market()
 
@@ -262,7 +276,20 @@ class DoubleHestonJumpCalibrator:
                 if v != _SENTINEL and v < counters[i][1]:
                     counters[i][1] = v
 
-        if self.batch_starts and multi_start > 1:
+        if gradient == "analytic":
+            for i in range(multi_start):
+                def fg(x, i=i):
+                    f, g = market.loss_grad(np.asarray(x, dtype=np.float64).reshape(1, 13))
+                    counters[i][0] += 1
+                    if f[0] != _SENTINEL and f[0] < counters[i][1]:
+                        counters[i][1] = f[0]
+                    return f[0], g[0]
+                try:
+                    results[i] = self._minimize(fg, x0s[i], maxiter, maxfun=15000)
+                except Exception as exc:
+                    results[i] = exc
+                finished_at[i] = time.time()
+        elif self.batch_starts and multi_start > 1:
             evaluator = _LockstepEvaluator(market, multi_start)
 
             def worker(i):

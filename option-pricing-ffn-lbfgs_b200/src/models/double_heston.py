@@ -90,3 +90,11 @@ class DoubleHeston():
         price = self._ctx.price_list(self._params(), self.S0, [self.K], [self.T], [self._is_call()],
                                      self.r, self.q, N)
         return np.float64(price[0, 0])
+
+    def pricing_gradient(self, N=128):
+        """float64[13]: d pricing(N) / d(v01, kappa1, theta1, sigma1, rho1, v02, kappa2, theta2, sigma2, rho2,
+        lambda_j, mu_j, sigma_j), exact with the truncation range held at its value for the current parameters
+        (extension, not in the reference) — one kernel launch."""
+        _, jac = self._ctx.price_jacobian(self._params(), self.S0, [self.K], [self.T], [self._is_call()], self.r,
+                                          self.q, N)
+        return jac[0, 0].copy()
