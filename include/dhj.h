@@ -194,6 +194,22 @@ DHJ_API int dhj_lbfgs_minimize_grad(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_mark
                                     const int32_t* state_market, int64_t n_states, int64_t* rounds,
                                     int64_t* state_rounds, double* seconds);
 
+/* ---- Greeks -----------------------------------------------------------------------------------
+ * dhj_price_greeks: dhj_price_list's arguments, out_price[P][M] and out_greeks[P][M][DHJ_N_GREEKS] in the caller's
+ * option order, per option in this order:
+ *   delta = dV/dS0,  gamma = d2V/dS0^2,  theta = -dV/dT (per year, at fixed spot),  rho = dV/dr,  rho_q = dV/dq.
+ * All five are exact derivatives of the COS price with the truncation range [a, b] held at its value for the current
+ * inputs (the frozen range of dhj_price_jacobian).  [a, b] is a range of the log-return and does not move with S0, so
+ * for a strike whose +-0.1 widening does not bind, delta and gamma are the exact derivatives of the price itself.  A
+ * binding strike's own range (log(K/S0) +- 0.1) moves with S0; its frozen-range value is reported.  The discount
+ * exp(-rT) does not depend on q and the truncation range ignores q (as the reference's does), so
+ * rho_q = -(rho + T V).  NaN wherever the price is NaN.  Host buffers, chunked synchronously through device scratch. */
+#define DHJ_N_GREEKS 5
+DHJ_API int dhj_price_greeks(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride,
+                             double r, double q, const double* strike, int64_t strike_stride, const double* maturity,
+                             const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price,
+                             double* out_greeks);
+
 /* Threads used by the library's host-side parallel loops (optimiser states in ask / tell, staging copies of pageable
  * buffers); 0 = all cores (default).  Several lock-step pipelines on one host divide the cores with this. */
 DHJ_API int dhj_set_host_threads(int32_t n);

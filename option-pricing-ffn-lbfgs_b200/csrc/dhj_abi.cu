@@ -14,6 +14,7 @@
 
 #include "dhj.h"
 #include "dhj_kernels.cuh"
+#include "dhj_greeks.cuh"
 #include "dhj_jac.cuh"
 #include "dhj_generate.cuh"
 
@@ -865,12 +866,18 @@ static int launch_jac(dhj_ctx* ctx, const SliceView& v, const JacArgs& a, cudaSt
   return DHJ_OK;
 }
 
-int dhj_price_jacobian(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride, double r,
-                       double q, const double* strike, int64_t strike_stride, const double* maturity,
-                       const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price, double* out_jac) {
+// Prices and n_der derivatives per option of an option list (dhj_price_jacobian, dhj_price_greeks): the argument
+// checks, the maturity book and synchronous chunks of ~32 MB through the staging buffers (throughput of these entry
+// points is not a goal).  launch(view, d_params, d_S0, s0_stride, n, d_price, d_der) enqueues the kernel for n sets.
+extern "C++" {
+template <class Launch>
+static int run_option_list(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride,
+                           double r, double q, const double* strike, int64_t strike_stride, const double* maturity,
+                           const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price, double* out_der,
+                           int n_der, Launch launch) {
   int rc = check_common(ctx, params, P, S0, N, L, out_price);
   if (rc) return rc;
-  if (!out_jac) return fail(ctx, DHJ_ERR_ARG, "null array argument");
+  if (!out_der) return fail(ctx, DHJ_ERR_ARG, "null array argument");
   if (M < 0) return fail(ctx, DHJ_ERR_ARG, "M must be >= 0");
   if (M == 0 || P == 0) return DHJ_OK;
   if (!strike || !maturity || !is_call) return fail(ctx, DHJ_ERR_ARG, "null option table");
@@ -883,9 +890,8 @@ int dhj_price_jacobian(dhj_ctx* ctx, const double* params, int64_t P, const doub
   rc = upload_book(ctx, book, strike_stride ? nullptr : strike, strike_stride ? 0 : M, ctx->stream, &v);
   if (rc) return rc;
   v.scale_by_spot = 0; v.n_cos = N; v.r = r; v.q = q; v.L = L;
-  // synchronous chunks of ~32 MB through the staging buffers (throughput of this entry point is not a goal)
   const size_t row_in = kNumParams + (s0_stride ? 1 : 0) + (strike_stride ? (size_t)M : 0);
-  const size_t row_out = (size_t)M * kJacChannels;
+  const size_t row_out = (size_t)M * (1 + n_der);
   const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(P, (int64_t)(((size_t)1 << 22) / (row_in + row_out))));
   const size_t in_bytes = (size_t)chunk * row_in * sizeof(double) + sizeof(double);
   const size_t out_bytes = (size_t)chunk * row_out * sizeof(double);
@@ -907,19 +913,51 @@ int dhj_price_jacobian(dhj_ctx* ctx, const double* params, int64_t P, const doub
     SliceView vv = v;
     if (strike_stride) { vv.strike = (const double*)(din + pb + s0b); vv.strike_stride = M; }
     double* d_out = (double*)ctx->d_jac.p;
-    JacArgs a;
-    a.params = (const double*)din; a.S0 = (const double*)(din + pb); a.s0_stride = s0_stride ? 1 : 0;
-    a.row_index = nullptr; a.P = n; a.out_price = d_out; a.out_jac = d_out + n * (int64_t)M;
-    rc = launch_jac(ctx, vv, a, ctx->stream);
+    rc = launch(vv, (const double*)din, (const double*)(din + pb), s0_stride ? 1 : 0, n, d_out, d_out + n * (int64_t)M);
     if (rc) return rc;
     const size_t ob = (size_t)n * row_out * sizeof(double);
     DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, d_out, ob, cudaMemcpyDeviceToHost, ctx->stream));
     DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     const double* res = (const double*)ctx->h_res.p;
     host_copy(out_price + lo * (int64_t)M, res, (size_t)n * M * sizeof(double));
-    host_copy(out_jac + lo * (int64_t)M * kNumParams, res + n * (int64_t)M, (size_t)n * M * kNumParams * sizeof(double));
+    host_copy(out_der + lo * (int64_t)M * n_der, res + n * (int64_t)M, (size_t)n * M * n_der * sizeof(double));
   }
   return book_used(ctx, ctx->stream);
+}
+}  // extern "C++"
+
+int dhj_price_jacobian(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride, double r,
+                       double q, const double* strike, int64_t strike_stride, const double* maturity,
+                       const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price, double* out_jac) {
+  return run_option_list(ctx, params, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, N, L,
+                         out_price, out_jac, kNumParams,
+                         [&](const SliceView& vv, const double* d_params, const double* d_S0, long long s0s, int64_t n,
+                             double* d_price, double* d_der) {
+                           JacArgs a;
+                           a.params = d_params; a.S0 = d_S0; a.s0_stride = s0s;
+                           a.row_index = nullptr; a.P = n; a.out_price = d_price; a.out_jac = d_der;
+                           return launch_jac(ctx, vv, a, ctx->stream);
+                         });
+}
+
+// ---- Greeks (dhj_greeks.cuh) --------------------------------------------------------------------------
+int dhj_price_greeks(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride, double r,
+                     double q, const double* strike, int64_t strike_stride, const double* maturity,
+                     const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price, double* out_greeks) {
+  return run_option_list(ctx, params, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, N, L,
+                         out_price, out_greeks, kGreeks,
+                         [&](const SliceView& vv, const double* d_params, const double* d_S0, long long s0s, int64_t n,
+                             double* d_price, double* d_der) {
+                           GreeksArgs a;
+                           a.params = d_params; a.S0 = d_S0; a.s0_stride = s0s;
+                           a.row_index = nullptr; a.P = n; a.out_price = d_price; a.out_greeks = d_der;
+                           const long long blocks = (n * (long long)vv.n_slices + kJacWarps - 1) / kJacWarps;
+                           k_price_greeks<<<(int)std::max<long long>(1, std::min(blocks, 2147483647LL)),
+                                            32 * kJacWarps, 0, ctx->stream>>>(vv, a);
+                           DHJ_CUDA(ctx, cudaGetLastError());
+                           ctx->launches++;
+                           return DHJ_OK;
+                         });
 }
 
 // f and the analytic g of B loss evaluations: exp/tanh transform (k_fd_expand without a stencil) -> prices of every

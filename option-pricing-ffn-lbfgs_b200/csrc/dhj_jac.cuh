@@ -20,6 +20,7 @@
 //     (strike, k) by the three-term recurrence of segment_sums and multiplied into the 14 channels;
 //   * strikes whose +-0.1 widening binds get their own pass with their own (a, b), exactly as in the pricing kernels.
 // Every sum has a fixed order that depends on nothing but the item, so an item's outputs do not depend on the launch.
+// The item loop and the pass are templates on the channel set (JacChannels here; GreeksChannels in dhj_greeks.cuh).
 #pragma once
 #include "dhj_kernels.cuh"
 
@@ -29,24 +30,36 @@ constexpr int kJacChannels = kNumParams + 1;   // channel 0: the price; 1 + i: d
 constexpr int kJacWarps = 2;
 constexpr int kJacChunk = 64;
 
-struct JacWarp {
+// The item loop and the pass below are shared by every kernel that contracts G and some of its tangents against the
+// payoff basis (k_price_jac here, k_price_greeks in dhj_greeks.cuh).  A channel set Ch supplies:
+//   kTangents       complex tangents dX of the CF exponent; channel 0 is G, channel 1 + i is w_k Re(dX_i e^{X - iua})
+//   kStaged         1 + kTangents channels staged per block of 32 k (each with its own A-sums)
+//   kAcc, kChunk    accumulators per strike, strikes per chunk
+//   Args            the kernel's arguments (params, S0, s0_stride, row_index, P and the outputs)
+//   exponent()      X and the kTangents tangents at u
+//   term()          one (strike, k) step: the basis value V_k and everything else the strike accumulates
+//   pass_end()      the strike's constant parts, after the pass's A-sums are complete
+//   write()         the outputs of one option
+template <class Ch>
+struct ChanWarp {
   Params m;
   SetConsts set;
   PassConsts pass;                                 // the pass being contracted: regular, or a binding strike's own
   double S0, disc, a0, b0;
-  double G[kJacChannels][32];                      // stage: channel c of the block's 32 terms
+  double G[Ch::kStaged][32];                       // stage: channel c of the block's 32 terms
   double fP[32], fQ[32], fR[32], f1[32], f2[32];   // P'_k, Q'_k, R'_k, P'_k (t1+t3)_k, R'_k sin(u_k (b-a))
-  double A[3][kJacChannels], g0[kJacChannels];     // A1, A2, A3 and g0 of the pass, per channel
-  double K[kJacChunk], x[kJacChunk], sex[kJacChunk], cth[kJacChunk], sth[kJacChunk];
-  double acc[kJacChunk][kJacChannels];
-  unsigned char call[kJacChunk], bind[kJacChunk];
+  double A[3][Ch::kStaged], g0[Ch::kStaged];       // A1, A2, A3 and g0 of the pass, per channel
+  double K[Ch::kChunk], x[Ch::kChunk], sex[Ch::kChunk], cth[Ch::kChunk], sth[Ch::kChunk];
+  double acc[Ch::kChunk][Ch::kAcc];
+  unsigned char call[Ch::kChunk], bind[Ch::kChunk];
 #if defined(DHJ_CHECKED)
   unsigned wtag[32], rtag[32], epoch;              // as CoefStage: per-slot write epoch, per-lane read epoch
 #endif
 };
 
-struct JacSmem {
-  JacWarp w[kJacWarps];
+template <class Ch>
+struct ChanSmem {
+  ChanWarp<Ch> w[kJacWarps];
   fm::Tables ltab;
 };
 
@@ -60,9 +73,39 @@ struct JacArgs {
   double* out_jac;           // [P][M][13]
 };
 
+// 14 channels (the price and its 13 parameter derivatives), one accumulator each
+struct JacChannels {
+  static constexpr int kTangents = kNumParams, kStaged = kJacChannels, kAcc = kJacChannels, kChunk = kJacChunk;
+  using Args = JacArgs;
+  static __device__ __forceinline__ void exponent(const Params& m, const SetConsts& s, double u, double T,
+                                                  const fm::Tables* __restrict__ ltab, double* xr, double* xi,
+                                                  Cplx* dX) {
+    cf_exponent_tangents(m, s, u, T, ltab, xr, xi, dX);
+  }
+  template <class W>
+  static __device__ __forceinline__ void term(double* acc, const W& w, int i, double c0, double s0, double Kt,
+                                              double sex) {
+    const double V = fma(s0, fma(Kt, w.fR[i], -(sex * w.fQ[i])), -(sex * (w.fP[i] * c0)));
+#pragma unroll
+    for (int c = 0; c < kJacChannels; ++c) acc[c] = fma(w.G[c][i], V, acc[c]);
+  }
+  template <class W>
+  static __device__ __forceinline__ void pass_end(W& w, int t, const PassConsts& pc) {
+    for (int c = 0; c < kJacChannels; ++c)
+      w.acc[t][c] += strike_const_part(w.call[t] != 0, w.S0, w.K[t], w.x[t], pc, w.A[0][c], w.A[1][c], w.A[2][c],
+                                       w.g0[c]);
+  }
+  template <class W>
+  static __device__ __forceinline__ void write(const Args& a, long long at, const W& w, int t, double /*r*/) {
+    a.out_price[at] = w.disc * w.acc[t][0];
+    for (int i = 0; i < kNumParams; ++i) a.out_jac[at * kNumParams + i] = w.disc * w.acc[t][1 + i];
+  }
+};
+
 // lane 0 prepares the item; the other lanes wait at the caller's __syncwarp
-__device__ __forceinline__ void jac_prepare(JacWarp& W, const SliceView& v, const double* __restrict__ pp, double S0,
-                                            double T) {
+template <class Ch>
+__device__ __forceinline__ void chan_prepare(ChanWarp<Ch>& W, const SliceView& v, const double* __restrict__ pp,
+                                             double S0, double T) {
   W.m = load_params(pp);
   W.set = make_set_consts(W.m, v.r, v.q);
   double a0, b0;
@@ -74,23 +117,24 @@ __device__ __forceinline__ void jac_prepare(JacWarp& W, const SliceView& v, cons
 }
 
 // One pass over n_cos terms with W.pass: every strike of the chunk with !bind (only < 0), or strike `only`.
-__device__ __forceinline__ void jac_pass(JacWarp& W, int cnt, int only, int n_cos, int lane,
-                                         const fm::Tables* __restrict__ ltab) {
+template <class Ch>
+__device__ __forceinline__ void chan_pass(ChanWarp<Ch>& W, int cnt, int only, int n_cos, int lane,
+                                          const fm::Tables* __restrict__ ltab) {
   const PassConsts pc = W.pass;
   const double u1 = u_one(pc);
   for (int t = lane; t < cnt; t += 32) {
     if (only < 0 ? W.bind[t] != 0 : t != only) continue;
     fm::sincos_(u1 * (W.x[t] - pc.a), &W.sth[t], &W.cth[t]);
   }
-  if (lane < kJacChannels) { W.A[0][lane] = 0.0; W.A[1][lane] = 0.0; W.A[2][lane] = 0.0; }
+  if (lane < Ch::kStaged) { W.A[0][lane] = 0.0; W.A[1][lane] = 0.0; W.A[2][lane] = 0.0; }
 #pragma unroll 1
   for (int k0 = 0; k0 < n_cos; k0 += 32) {
-    // ---- lane = k: G and its 13 tangents -> stage ----
+    // ---- lane = k: G and its tangent channels -> stage ----
     const int k = k0 + lane;
     const double u = u_of_k(pc, k);
     double xr, xi;
-    Cplx dX[kNumParams];
-    cf_exponent_tangents(W.m, W.set, u, pc.T, ltab, &xr, &xi, dX);
+    Cplx dX[Ch::kTangents];
+    Ch::exponent(W.m, W.set, u, pc.T, ltab, &xr, &xi, dX);
     double sph, cph;
     fm::sincos_(fma(-u, pc.a, xi), &sph, &cph);
     const bool live = k < n_cos;                         // ragged last block: every channel is 0
@@ -118,7 +162,7 @@ __device__ __forceinline__ void jac_pass(JacWarp& W, int cnt, int only, int n_co
 #endif
     W.G[0][lane] = live ? er : 0.0;
 #pragma unroll
-    for (int i = 0; i < kNumParams; ++i) W.G[1 + i][lane] = live ? fma(dX[i].r, er, -(dX[i].i * ei)) : 0.0;
+    for (int i = 0; i < Ch::kTangents; ++i) W.G[1 + i][lane] = live ? fma(dX[i].r, er, -(dX[i].i * ei)) : 0.0;
     W.fP[lane] = pc.tw * kt.inv1;
     W.fQ[lane] = W.fP[lane] * u;
     W.fR[lane] = pc.tw * kt.invu;
@@ -129,7 +173,7 @@ __device__ __forceinline__ void jac_pass(JacWarp& W, int cnt, int only, int n_co
     for (int l = 0; l < 32; ++l) DHJ_CHECK(W.wtag[l] == epoch, kChkReadBeforeWrite);
 #endif
     // ---- strike-independent sums of channel `lane`, k in order ----
-    if (lane < kJacChannels) {
+    if (lane < Ch::kStaged) {
       double s1 = W.A[0][lane], s2 = W.A[1][lane], s3 = W.A[2][lane];
       for (int i = 0; i < 32; ++i) {
         const double gc = W.G[lane][i];
@@ -138,14 +182,14 @@ __device__ __forceinline__ void jac_pass(JacWarp& W, int cnt, int only, int n_co
       W.A[0][lane] = s1; W.A[1][lane] = s2; W.A[2][lane] = s3;
       if (k0 == 0) W.g0[lane] = W.G[lane][0] * pc.tw;
     }
-    // ---- strikes: one basis value per (strike, k), 14 channels ----
+    // ---- strikes: one basis value per (strike, k) into every accumulator ----
     const double u0 = u_of_k(pc, k0);
     for (int t = lane; t < cnt; t += 32) {
       if (only < 0 ? W.bind[t] != 0 : t != only) continue;
-      DHJ_CHECK(t < kJacChunk, kChkSharedIndex);
-      double acc[kJacChannels];
+      DHJ_CHECK(t < Ch::kChunk, kChkSharedIndex);
+      double acc[Ch::kAcc];
 #pragma unroll
-      for (int c = 0; c < kJacChannels; ++c) acc[c] = W.acc[t][c];
+      for (int c = 0; c < Ch::kAcc; ++c) acc[c] = W.acc[t][c];
       double c0, s0;
       fm::sincos_(u0 * (W.x[t] - pc.a), &s0, &c0);
       const double cth = W.cth[t], sth = W.sth[t], two_c = cth + cth;
@@ -153,14 +197,12 @@ __device__ __forceinline__ void jac_pass(JacWarp& W, int cnt, int only, int n_co
       double c1 = fma(c0, cth, -(s0 * sth)), s1 = fma(s0, cth, c0 * sth);
 #pragma unroll 4
       for (int i = 0; i < 32; ++i) {
-        const double V = fma(s0, fma(Kt, W.fR[i], -(sex * W.fQ[i])), -(sex * (W.fP[i] * c0)));
-#pragma unroll
-        for (int c = 0; c < kJacChannels; ++c) acc[c] = fma(W.G[c][i], V, acc[c]);
+        Ch::term(acc, W, i, c0, s0, Kt, sex);
         const double c2 = fma(two_c, c1, -c0), s2 = fma(two_c, s1, -s0);
         c0 = c1; s0 = s1; c1 = c2; s1 = s2;
       }
 #pragma unroll
-      for (int c = 0; c < kJacChannels; ++c) W.acc[t][c] = acc[c];
+      for (int c = 0; c < Ch::kAcc; ++c) W.acc[t][c] = acc[c];
     }
 #if defined(DHJ_CHECKED)
     W.rtag[lane] = W.epoch;
@@ -169,15 +211,15 @@ __device__ __forceinline__ void jac_pass(JacWarp& W, int cnt, int only, int n_co
   __syncwarp();                                          // A-sums complete
   for (int t = lane; t < cnt; t += 32) {
     if (only < 0 ? W.bind[t] != 0 : t != only) continue;
-    for (int c = 0; c < kJacChannels; ++c)
-      W.acc[t][c] += strike_const_part(W.call[t] != 0, W.S0, W.K[t], W.x[t], pc, W.A[0][c], W.A[1][c], W.A[2][c],
-                                       W.g0[c]);
+    Ch::pass_end(W, t, pc);
   }
   __syncwarp();
 }
 
-__global__ void __launch_bounds__(32 * kJacWarps) k_price_jac(SliceView v, JacArgs a) {
-  __shared__ JacSmem sm;
+// The item loop: one warp per (parameter set, maturity slice) item, strikes in chunks of Ch::kChunk.
+template <class Ch>
+__device__ __forceinline__ void chan_items(const SliceView& v, const typename Ch::Args& a) {
+  __shared__ ChanSmem<Ch> sm;
   const int tid = threadIdx.x;
   // (load_log_table assumes >= 65 threads: the block has 64, so the tables are copied in a strided loop)
   for (int i = tid; i < 65; i += 32 * kJacWarps) {
@@ -190,7 +232,7 @@ __global__ void __launch_bounds__(32 * kJacWarps) k_price_jac(SliceView v, JacAr
 #endif
   __syncthreads();
   const int warp = __shfl_sync(kFullMask, tid >> 5, 0), lane = tid & 31;
-  JacWarp& W = sm.w[warp];
+  ChanWarp<Ch>& W = sm.w[warp];
   const long long n_items = a.P * (long long)v.n_slices;
   for (long long item = (long long)blockIdx.x * kJacWarps + warp; item < n_items;
        item += (long long)gridDim.x * kJacWarps) {
@@ -200,11 +242,11 @@ __global__ void __launch_bounds__(32 * kJacWarps) k_price_jac(SliceView v, JacAr
     const double* strike_row = v.strike + row * v.strike_stride;
     const int o_lo = v.slice_off[s], o_hi = v.slice_off[s + 1];
     __syncwarp();                                        // the previous item has left the warp's shared memory
-    if (lane == 0) jac_prepare(W, v, a.params + kNumParams * p, a.S0[row * a.s0_stride], v.slice_T[s]);
+    if (lane == 0) chan_prepare(W, v, a.params + kNumParams * p, a.S0[row * a.s0_stride], v.slice_T[s]);
     __syncwarp();
     const PassConsts regular = W.pass;
-    for (int c_lo = o_lo; c_lo < o_hi; c_lo += kJacChunk) {
-      const int cnt = min(kJacChunk, o_hi - c_lo);
+    for (int c_lo = o_lo; c_lo < o_hi; c_lo += Ch::kChunk) {
+      const int cnt = min(Ch::kChunk, o_hi - c_lo);
       int n_bind = 0;
       for (int t0 = 0; t0 < cnt; t0 += 32) {             // warp-uniform trip count (the ballot needs every lane)
         const int t = t0 + lane;
@@ -216,7 +258,7 @@ __global__ void __launch_bounds__(32 * kJacWarps) k_price_jac(SliceView v, JacAr
           W.K[t] = sc.K; W.x[t] = sc.x; W.sex[t] = W.S0 * sc.ex;
           bind = ((sc.x - 0.1) < W.a0) || ((sc.x + 0.1) > W.b0);
           W.bind[t] = bind; W.call[t] = v.call[c_lo + t];
-          for (int c = 0; c < kJacChannels; ++c) W.acc[t][c] = 0.0;
+          for (int c = 0; c < Ch::kAcc; ++c) W.acc[t][c] = 0.0;
         }
         n_bind += __popc(__ballot_sync(kFullMask, bind));
       }
@@ -224,7 +266,7 @@ __global__ void __launch_bounds__(32 * kJacWarps) k_price_jac(SliceView v, JacAr
       if (n_bind < cnt) {
         if (lane == 0) W.pass = regular;
         __syncwarp();
-        jac_pass(W, cnt, -1, v.n_cos, lane, &sm.ltab);
+        chan_pass(W, cnt, -1, v.n_cos, lane, &sm.ltab);
       }
       if (n_bind > 0) {
         for (int t = 0; t < cnt; ++t) {
@@ -233,20 +275,21 @@ __global__ void __launch_bounds__(32 * kJacWarps) k_price_jac(SliceView v, JacAr
           if (lane == 0) W.pass = make_pass_consts(W.set, py_min(W.a0, W.x[t] - 0.1), py_max(W.b0, W.x[t] + 0.1),
                                                    regular.T);
           __syncwarp();
-          jac_pass(W, cnt, t, v.n_cos, lane, &sm.ltab);
+          chan_pass(W, cnt, t, v.n_cos, lane, &sm.ltab);
         }
       }
       for (int t = lane; t < cnt; t += 32) {
         const int o = v.pos[c_lo + t];
         const long long at = p * (long long)v.n_options + o;
-        DHJ_CHECK(o >= 0 && o < v.n_options && at < a.P * (long long)v.n_options && t < kJacChunk, kChkOutputIndex);
-        a.out_price[at] = W.disc * W.acc[t][0];
-        for (int i = 0; i < kNumParams; ++i) a.out_jac[at * kNumParams + i] = W.disc * W.acc[t][1 + i];
+        DHJ_CHECK(o >= 0 && o < v.n_options && at < a.P * (long long)v.n_options && t < Ch::kChunk, kChkOutputIndex);
+        Ch::write(a, at, W, t, v.r);
       }
       __syncwarp();
     }
   }
 }
+
+__global__ void __launch_bounds__(32 * kJacWarps) k_price_jac(SliceView v, JacArgs a) { chan_items<JacChannels>(v, a); }
 
 // Loss and its analytic gradient in the unconstrained x, one optimiser state per thread, options in slice order as
 // k_loss_reduce visits them; `prices` come from the pricing kernel (f has the bits of the loss path), `jac` from

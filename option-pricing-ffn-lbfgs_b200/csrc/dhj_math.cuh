@@ -289,16 +289,15 @@ DHJ_HD Cplx c_sub(Cplx a, Cplx b) { return {a.r - b.r, a.i - b.i}; }
 DHJ_HD Cplx c_mul(Cplx a, Cplx b) { return {fma(a.r, b.r, -(a.i * b.i)), fma(a.r, b.i, a.i * b.r)}; }
 DHJ_HD Cplx c_scale(Cplx a, double f) { return {a.r * f, a.i * f}; }
 
-// Factor j: the same value arithmetic as heston_factor (same bits, without the warp vote: both branches of the csqrt
-// are formed), plus dX/d(v0_j, kappa_j, theta_j, sigma_j, rho_j) -> dX[0..4].  With z_p = dz/dp etc.:
-//   d_p = z_p / (2d),  E_p = -T d_p E,  m_p = beta_p - d_p,  pl_p = beta_p + d_p,  D_p = pl_p - m_p E - m E_p
-//   B = -u (u+i) (1-E) / D             B_p = u (u+i) (E_p + (1-E) D_p/D) / D
-//   Ahat = m T - 2 log(D / (2d))       Ahat_p = m_p T - 2 (D_p/D - d_p/d)
-//   A = c Ahat, c = kappa theta / sigma^2:  dX/dv0 = B,  dX/dtheta = (kappa/sigma^2) Ahat,
-//   dX/dp = c_p Ahat + c Ahat_p + v0 B_p  for p = kappa (c_p = c/kappa), sigma (c_p = -2c/sigma), rho (c_p = 0)
-DHJ_HD void heston_factor_tangents(const Params& mp, const SetConsts& s, int j, double u, double T,
-                                   const fm::Tables* __restrict__ ltab, double& aR, double& aI, double& sli,
-                                   double& xbr, double& xbi, Cplx* dX) {
+// Factor j's value arithmetic for the tangent functions: heston_factor's operations without the warp vote (both
+// branches of the csqrt are formed), the same running sums, and the intermediates the tangents need.
+struct FactorState {
+  double dr, di, h, Er, Ei, mr, mi, Dr, Di, inD, Mr, Mi, L, li;
+};
+
+DHJ_HD FactorState heston_factor_state(const SetConsts& s, int j, double u, double T,
+                                       const fm::Tables* __restrict__ ltab, double& aR, double& aI, double& sli,
+                                       double& xbr, double& xbi) {
   const double kap = s.kappa[j];
   const double bi = -(s.rs[j] * u);
   const double s2u = s.s2[j] * u;
@@ -336,8 +335,25 @@ DHJ_HD void heston_factor_tangents(const Params& mp, const SetConsts& s, int j, 
   aR = fma(cT, mr, aR);
   aI = fma(cT, mi, aI);
   sli = fma(s.c[j], li, sli);
+  return {dr, di, h, Er, Ei, mr, mi, Dr, Di, inD, Mr, Mi, L, li};
+}
 
-  // tangents
+// Factor j: the value arithmetic of heston_factor_state plus dX/d(v0_j, kappa_j, theta_j, sigma_j, rho_j) -> dX[0..4].
+// With z_p = dz/dp etc.:
+//   d_p = z_p / (2d),  E_p = -T d_p E,  m_p = beta_p - d_p,  pl_p = beta_p + d_p,  D_p = pl_p - m_p E - m E_p
+//   B = -u (u+i) (1-E) / D             B_p = u (u+i) (E_p + (1-E) D_p/D) / D
+//   Ahat = m T - 2 log(D / (2d))       Ahat_p = m_p T - 2 (D_p/D - d_p/d)
+//   A = c Ahat, c = kappa theta / sigma^2:  dX/dv0 = B,  dX/dtheta = (kappa/sigma^2) Ahat,
+//   dX/dp = c_p Ahat + c Ahat_p + v0 B_p  for p = kappa (c_p = c/kappa), sigma (c_p = -2c/sigma), rho (c_p = 0)
+DHJ_HD void heston_factor_tangents(const Params& mp, const SetConsts& s, int j, double u, double T,
+                                   const fm::Tables* __restrict__ ltab, double& aR, double& aI, double& sli,
+                                   double& xbr, double& xbi, Cplx* dX) {
+  const FactorState f = heston_factor_state(s, j, u, T, ltab, aR, aI, sli, xbr, xbi);
+  const double kap = s.kappa[j];
+  const double bi = -(s.rs[j] * u);
+  const double dr = f.dr, di = f.di, h = f.h, Er = f.Er, Ei = f.Ei, mr = f.mr, mi = f.mi, Dr = f.Dr, Di = f.Di;
+  const double inD = f.inD, Mr = f.Mr, Mi = f.Mi, L = f.L, li = f.li;
+  const double ar = 1.0 - Er, ai = -Ei;
   const Cplx E = {Er, Ei}, m = {mr, mi}, omE = {ar, ai};
   const Cplx uu = {u * u, u};                                  // u (u + i)
   const Cplx invD = {Dr * inD, -(Di * inD)};                   // 1/D
@@ -399,6 +415,42 @@ DHJ_HD void cf_exponent_tangents(const Params& mp, const SetConsts& s, double u,
   dX[11] = {-(ulT * Ji), ulT * (Jr - C)};
   const double lts = lamT * mp.sj, u2 = u * u;
   dX[12] = {-(lts * (u2 * Jr)), -(lts * fma(u, C, u2 * Ji))};
+}
+
+// X at u (the value arithmetic of cf_exponent_tangents) and its derivatives in the maturity and the rate, for the
+// Greeks (dhj_greeks.cuh): dX[0] = dX/dT, dX[1] = dX/dr.  beta, d and c do not depend on T; forward mode through
+// E = exp(-d T):
+//   E_T = -d E,  D_T = -m E_T,  B_T = u (u+i) (E_T + (1-E) D_T/D) / D,  Ahat_T = m - 2 D_T/D
+//   dX/dT = sum_j (c_j Ahat_T + v0_j B_T) + i drift u + lam (J - 1),   dX/dr = i u T   (from A0 = i drift u T)
+// (dX/dq = -dX/dr; the truncation range depends on T and r, and is held fixed.)
+DHJ_HD void cf_exponent_time(const SetConsts& s, double u, double T, const fm::Tables* __restrict__ ltab,
+                             double* xr_out, double* xi_out, Cplx* dX) {
+  const double lamT = s.lam * T;
+  double aR = 0.0, aI = (s.drift * u) * T, sli = 0.0, xbr = 0.0, xbi = 0.0;
+  const Cplx uu = {u * u, u};                                  // u (u + i)
+  Cplx dT = {0.0, s.drift * u};
+#pragma unroll
+  for (int j = 0; j < 2; ++j) {
+    const FactorState f = heston_factor_state(s, j, u, T, ltab, aR, aI, sli, xbr, xbi);
+    const Cplx E = {f.Er, f.Ei}, m = {f.mr, f.mi}, omE = {1.0 - f.Er, -f.Ei};
+    const Cplx invD = {f.Dr * f.inD, -(f.Di * f.inD)};
+    const Cplx ET = c_scale(c_mul({f.dr, f.di}, E), -1.0);
+    const Cplx DTD = c_mul(c_scale(c_mul(m, ET), -1.0), invD);
+    const Cplx BT = c_mul(c_mul(uu, c_add(ET, c_mul(omE, DTD))), invD);
+    const Cplx AhT = c_sub(m, c_scale(DTD, 2.0));
+    dT = c_add(dT, c_add(c_scale(AhT, s.c[j]), c_scale(BT, s.v0[j])));
+  }
+  double xr = aR + xbr;
+  double xi = fma(-2.0, sli, aI) + xbi;
+  double cj, sj;
+  fm::sincos_(u * s.mu, &sj, &cj);
+  const double ej = jump_gauss(s, u, ltab);
+  xr = fma(lamT, fma(ej, cj, -1.0), xr);
+  xi = fma(lamT, ej * sj, xi);
+  *xr_out = xr; *xi_out = xi;
+  const double Jr = ej * cj, Ji = ej * sj;
+  dX[0] = {fma(s.lam, Jr - 1.0, dT.r), fma(s.lam, Ji, dT.i)};
+  dX[1] = {0.0, u * T};
 }
 
 // everything the strike loop needs for one k

@@ -15,6 +15,8 @@ import numpy as np
 from numpy.ctypeslib import ndpointer
 
 N_PARAMS = 13
+N_GREEKS = 5
+GREEKS = ("delta", "gamma", "theta", "rho", "rho_q")
 FD_POINTS = 14
 LIB_PATH = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "lib", "libdhj.so")
 
@@ -26,7 +28,7 @@ EXPORTS = (
     "dhj_cf", "dhj_cf_complex", "dhj_truncation_range", "dhj_chi_psi", "dhj_fp64_peak",
     "dhj_lbfgs_create", "dhj_lbfgs_destroy", "dhj_lbfgs_ask", "dhj_lbfgs_tell", "dhj_lbfgs_result", "dhj_lbfgs_minimize_fd",
     "dhj_generator_draws", "dhj_generate_dev", "dhj_generate", "dhj_set_host_threads", "dhj_debug_checks",
-    "dhj_price_jacobian", "dhj_loss_grad", "dhj_lbfgs_minimize_grad",
+    "dhj_price_jacobian", "dhj_loss_grad", "dhj_lbfgs_minimize_grad", "dhj_price_greeks",
 )
 
 
@@ -96,6 +98,7 @@ def load_library(path: str | None = None) -> ctypes.CDLL:
                                               ctypes.POINTER(_c_i64), _F64]
         lib.dhj_price_jacobian.argtypes = [_c_vp, _F64, _c_i64, _F64, _c_i64, _c_f64, _c_f64, _F64, _c_i64, _F64,
                                            _I32, _c_i32, _c_i32, _c_f64, _c_vp, _c_vp]
+        lib.dhj_price_greeks.argtypes = lib.dhj_price_jacobian.argtypes
         lib.dhj_loss_grad.argtypes = [_c_vp, _c_vp, _F64, _c_vp, _c_i64, _F64, _F64]
         lib.dhj_lbfgs_minimize_grad.argtypes = [_c_vp, _c_vp, _c_vp, _c_vp, _c_i64, ctypes.POINTER(_c_i64),
                                                 ctypes.POINTER(_c_i64), _F64]
@@ -189,6 +192,19 @@ class Context:
                                                      k_stride, maturity, call, M, int(N), float(L), _ptr(prices),
                                                      _ptr(jac)), "dhj_price_jacobian")
         return prices, jac
+
+    def price_greeks(self, params, S0, strike, maturity, is_call, r, q=0.0, N=128, L=10.0):
+        """(prices float64[P, M], greeks float64[P, M, 5]) of P parameter sets on an option list: greeks[p, o] =
+        (delta, gamma, theta, rho, rho_q) = (dV/dS0, d2V/dS0^2, -dV/dT, dV/dr, dV/dq), exact with the truncation
+        range held at its value for the current inputs (dhj_price_greeks)."""
+        params, P, S0, s0_stride, strike, k_stride, maturity, M, call = self._option_list(params, S0, strike, maturity,
+                                                                                        is_call)
+        prices, greeks = np.empty((P, M)), np.empty((P, M, N_GREEKS))
+        with self._lock:
+            self._check(self._lib.dhj_price_greeks(self._h, params, P, S0, s0_stride, float(r), float(q), strike,
+                                                   k_stride, maturity, call, M, int(N), float(L), _ptr(prices),
+                                                   _ptr(greeks)), "dhj_price_greeks")
+        return prices, greeks
 
     @staticmethod
     def _option_list(params, S0, strike, maturity, is_call):

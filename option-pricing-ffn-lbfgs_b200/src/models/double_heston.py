@@ -17,7 +17,7 @@ _PKG_ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__fi
 if _PKG_ROOT not in sys.path:
     sys.path.insert(0, _PKG_ROOT)
 
-from dhj import default_context  # noqa: E402
+from dhj import GREEKS, default_context  # noqa: E402
 
 
 class DoubleHeston():
@@ -98,3 +98,11 @@ class DoubleHeston():
         _, jac = self._ctx.price_jacobian(self._params(), self.S0, [self.K], [self.T], [self._is_call()], self.r,
                                           self.q, N)
         return jac[0, 0].copy()
+
+    def greeks(self, N=128):
+        """{"delta", "gamma", "theta", "rho", "rho_q"}: dV/dS0, d2V/dS0^2, -dV/dT (per year), dV/dr and dV/dq of
+        pricing(N), exact with the truncation range held at its value for the current inputs (extension, not in the
+        reference) — one kernel launch."""
+        _, g = self._ctx.price_greeks(self._params(), self.S0, [self.K], [self.T], [self._is_call()], self.r, self.q,
+                                      N)
+        return {name: np.float64(g[0, 0, i]) for i, name in enumerate(GREEKS)}
