@@ -210,6 +210,38 @@ DHJ_API int dhj_price_greeks(dhj_ctx* ctx, const double* params, int64_t P, cons
                              const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price,
                              double* out_greeks);
 
+/* ---- Implied volatility ------------------------------------------------------------------------
+ * Black-Scholes implied volatility of option prices, one thread per option, in the option-list layout of
+ * dhj_price_list: price[P][M], S0 with stride 0 or 1, strike[M] (strike_stride 0) or [P][M] (strike_stride M),
+ * maturity[M], is_call[M] (nonzero: call), scalar r and q (continuous rates).  sigma solves V = BS(S0, K, T, r, q, sigma)
+ * with F = S0 e^{(r-q)T} and discount e^{-rT}.
+ * out_status[P][M] (may be NULL):
+ *   0 ok (a price exactly at the lower bound gives sigma = 0)
+ *   1 price below the no-arbitrage lower bound e^{-rT} max(+-(F - K), 0)             -> NaN
+ *   2 price at or above the upper bound S0 e^{-qT} (call) or K e^{-rT} (put)         -> NaN
+ *   3 invalid input: V, r or q not finite, or S0, K, T not finite and > 0             -> NaN
+ *   4 not converged within 40 solver iterations                                       -> the last iterate
+ * Accuracy: with sigma* the exact implied vol of the double V and vega = dV/dsigma,
+ *   |sigma - sigma*| <= 64 eps (sigma* + V / vega),  eps = 2^-52,
+ * where V / vega is the option's own conditioning (tested for sigma in [0.01, 3], T in [1/365, 10],
+ * |ln(F/K)| / (sigma sqrt T) <= 6, calls and puts in and out of the money).
+ * dhj_implied_vol: host arrays, synchronous chunks through device scratch. */
+DHJ_API int dhj_implied_vol(dhj_ctx* ctx, const double* price, int64_t P, const double* S0, int64_t s0_stride,
+                            double r, double q, const double* strike, int64_t strike_stride, const double* maturity,
+                            const int32_t* is_call, int32_t M, double* out_vol, int32_t* out_status);
+/* DEVICE price / S0 / out / status, HOST tables strike[M], maturity[M], is_call[M]; scale_by_spot != 0 ->
+ * K = strike[j]*S0/100 (so a dhj_price_grid_dev or dhj_generate_dev surface, flattened maturity-major to
+ * M = nT*nK, is inverted without leaving HBM).  Asynchronous on `stream`. */
+DHJ_API int dhj_implied_vol_dev(dhj_ctx* ctx, const double* d_price, int64_t P, const double* d_S0,
+                                int64_t s0_stride, double r, double q, const double* strike, int32_t scale_by_spot,
+                                const double* maturity, const int32_t* is_call, int32_t M, double* d_out_vol,
+                                int32_t* d_out_status, void* stream);
+/* Black-Scholes prices of vol[P][M] (vol quotes -> prices for dhj_market_create; the forward map of the above).
+ * sigma = 0 gives the discounted intrinsic value; NaN for sigma < 0 or NaN and for invalid inputs. */
+DHJ_API int dhj_bs_price(dhj_ctx* ctx, const double* vol, int64_t P, const double* S0, int64_t s0_stride, double r,
+                         double q, const double* strike, int64_t strike_stride, const double* maturity,
+                         const int32_t* is_call, int32_t M, double* out_price);
+
 /* Threads used by the library's host-side parallel loops (optimiser states in ask / tell, staging copies of pageable
  * buffers); 0 = all cores (default).  Several lock-step pipelines on one host divide the cores with this. */
 DHJ_API int dhj_set_host_threads(int32_t n);

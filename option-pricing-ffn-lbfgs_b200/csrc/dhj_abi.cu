@@ -17,6 +17,7 @@
 #include "dhj_greeks.cuh"
 #include "dhj_jac.cuh"
 #include "dhj_generate.cuh"
+#include "dhj_iv.cuh"
 
 using namespace dhj;
 
@@ -306,17 +307,12 @@ int launch_price(dhj_ctx* ctx, const SliceView& v, PriceArgs a, int max_slice, c
   return DHJ_OK;
 }
 
-// Find (or upload into the ring) the packed book image + shared strike table for a pricing call on `stream`.
+// Find (or upload into the ring) a packed table image (an option book + shared strike table for a pricing call, or
+// the option tables of an implied-vol call) on `stream`; *d_image is its device copy.
 // No device-wide synchronisation: a new table goes to the least recently filled slot (after the last launch that
 // read that slot has finished — normally long ago), its copy is ordered before the caller's launches by stream
 // order or an event wait, and launches that still read other slots are not disturbed.
-int upload_book(dhj_ctx* ctx, const BookHost& book, const double* shared_strikes, int n_shared,
-                cudaStream_t stream, SliceView* v) {
-  const size_t bb = book.packed_bytes();
-  const size_t sb = BookHost::align8((size_t)n_shared * sizeof(double));
-  std::vector<unsigned char> image(bb + sb);
-  book.pack(image.data());
-  if (n_shared) memcpy(image.data() + bb, shared_strikes, (size_t)n_shared * sizeof(double));
+int upload_image(dhj_ctx* ctx, std::vector<unsigned char>& image, cudaStream_t stream, const unsigned char** d_image) {
   int hit = -1;
   for (int i = 0; i < kBookSlots && hit < 0; ++i)
     if (ctx->books[i].image == image) hit = i;
@@ -339,9 +335,22 @@ int upload_book(dhj_ctx* ctx, const BookHost& book, const double* shared_strikes
     DHJ_CUDA(ctx, cudaStreamWaitEvent(stream, ctx->books[hit].uploaded, 0));
   }
   ctx->book_cur = hit;
-  const BookSlot& b = ctx->books[hit];
-  book.view(v, (const unsigned char*)b.d.p);
-  v->strike = n_shared ? (const double*)((const unsigned char*)b.d.p + bb) : nullptr;
+  *d_image = (const unsigned char*)ctx->books[hit].d.p;
+  return DHJ_OK;
+}
+
+int upload_book(dhj_ctx* ctx, const BookHost& book, const double* shared_strikes, int n_shared,
+                cudaStream_t stream, SliceView* v) {
+  const size_t bb = book.packed_bytes();
+  const size_t sb = BookHost::align8((size_t)n_shared * sizeof(double));
+  std::vector<unsigned char> image(bb + sb);
+  book.pack(image.data());
+  if (n_shared) memcpy(image.data() + bb, shared_strikes, (size_t)n_shared * sizeof(double));
+  const unsigned char* d_image;
+  int rc = upload_image(ctx, image, stream, &d_image);
+  if (rc) return rc;
+  book.view(v, d_image);
+  v->strike = n_shared ? (const double*)(d_image + bb) : nullptr;
   v->strike_stride = 0;
   return DHJ_OK;
 }
@@ -958,6 +967,136 @@ int dhj_price_greeks(dhj_ctx* ctx, const double* params, int64_t P, const double
                            ctx->launches++;
                            return DHJ_OK;
                          });
+}
+
+// ---- implied volatility (dhj_iv.cuh) ----------------------------------------------------------------
+namespace {
+
+// The option tables of an implied-vol call as one image in the book ring: maturity[M] | strike[M] (shared strikes
+// only) | is_call[M].  Fills the table pointers of *a.
+int upload_iv_tables(dhj_ctx* ctx, const double* strike, bool shared_strike, const double* maturity,
+                     const int32_t* is_call, int32_t M, cudaStream_t st, iv::IvArgs* a) {
+  const size_t db = (size_t)M * sizeof(double);
+  const size_t kb = shared_strike ? db : 0;
+  std::vector<unsigned char> image(db + kb + (size_t)M * sizeof(int32_t));
+  memcpy(image.data(), maturity, db);
+  if (kb) memcpy(image.data() + db, strike, kb);
+  memcpy(image.data() + db + kb, is_call, (size_t)M * sizeof(int32_t));
+  const unsigned char* d;
+  int rc = upload_image(ctx, image, st, &d);
+  if (rc) return rc;
+  a->maturity = (const double*)d;
+  if (kb) { a->strike = (const double*)(d + db); a->strike_stride = 0; }
+  a->is_call = (const int32_t*)(d + db + kb);
+  return DHJ_OK;
+}
+
+// one elementwise launch over a.P x a.M options (grid-stride)
+int launch_iv(dhj_ctx* ctx, const iv::IvArgs& a, bool inverse, cudaStream_t st) {
+  const long long n = a.P * (long long)a.M;
+  const long long blocks = std::max<long long>(1, std::min<long long>((n + 255) / 256, 32LL * ctx->sm_count));
+  if (inverse) iv::k_implied_vol<<<(int)blocks, 256, 0, st>>>(a);
+  else iv::k_bs_price<<<(int)blocks, 256, 0, st>>>(a);
+  DHJ_CUDA(ctx, cudaGetLastError());
+  ctx->launches++;
+  return DHJ_OK;
+}
+
+int check_iv(dhj_ctx* ctx, const void* in, int64_t P, const void* S0, int64_t s0_stride, const void* out, int32_t M) {
+  if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
+  if (!in || !S0 || !out) return fail(ctx, DHJ_ERR_ARG, "null array argument");
+  if (P < 0) return fail(ctx, DHJ_ERR_ARG, "P must be >= 0 (got %lld)", (long long)P);
+  if (M < 0) return fail(ctx, DHJ_ERR_ARG, "M must be >= 0");
+  if (s0_stride != 0 && s0_stride != 1) return fail(ctx, DHJ_ERR_ARG, "s0_stride must be 0 or 1");
+  return DHJ_OK;
+}
+
+// dhj_implied_vol (inverse) and dhj_bs_price: host arrays, synchronous chunks of ~32 MB through the staging buffers
+// (throughput of these entry points is not a goal)
+int run_iv_host(dhj_ctx* ctx, bool inverse, const double* in, int64_t P, const double* S0, int64_t s0_stride,
+                double r, double q, const double* strike, int64_t strike_stride, const double* maturity,
+                const int32_t* is_call, int32_t M, double* out, int32_t* status) {
+  int rc = check_iv(ctx, in, P, S0, s0_stride, out, M);
+  if (rc) return rc;
+  if (M == 0 || P == 0) return DHJ_OK;
+  if (!strike || !maturity || !is_call) return fail(ctx, DHJ_ERR_ARG, "null option table");
+  if (strike_stride != 0 && strike_stride != M) return fail(ctx, DHJ_ERR_ARG, "strike_stride must be 0 or M");
+  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
+  iv::IvArgs a{};
+  rc = upload_iv_tables(ctx, strike, strike_stride == 0, maturity, is_call, M, ctx->stream, &a);
+  if (rc) return rc;
+  a.r = r; a.q = q; a.M = M; a.scale_by_spot = 0; a.s0_stride = s0_stride;
+  const size_t row_in = (size_t)M * sizeof(double) + (s0_stride ? sizeof(double) : 0) +
+                        (strike_stride ? (size_t)M * sizeof(double) : 0);
+  const size_t row_out = (size_t)M * (sizeof(double) + sizeof(int32_t));
+  const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(P, (int64_t)(((size_t)1 << 25) / (row_in + row_out))));
+  const size_t in_bytes = (size_t)chunk * row_in + sizeof(double);
+  const size_t out_bytes = (size_t)chunk * row_out;
+  DHJ_CUDA(ctx, ctx->h_x.reserve(in_bytes));
+  DHJ_CUDA(ctx, ctx->d_x.reserve(in_bytes));
+  DHJ_CUDA(ctx, ctx->d_jac.reserve(out_bytes));
+  DHJ_CUDA(ctx, ctx->h_res.reserve(out_bytes));
+  for (int64_t lo = 0; lo < P; lo += chunk) {
+    const int64_t n = std::min(chunk, P - lo);
+    const size_t vb = (size_t)n * M * sizeof(double);
+    const size_t s0b = s0_stride ? (size_t)n * sizeof(double) : sizeof(double);
+    const size_t kb = strike_stride ? vb : 0;
+    unsigned char* hin = (unsigned char*)ctx->h_x.p;
+    unsigned char* din = (unsigned char*)ctx->d_x.p;
+    host_copy(hin, in + lo * (int64_t)M, vb);
+    host_copy(hin + vb, s0_stride ? S0 + lo : S0, s0b);
+    if (kb) host_copy(hin + vb + s0b, strike + lo * (int64_t)M, kb);
+    DHJ_CUDA(ctx, cudaMemcpyAsync(din, hin, vb + s0b + kb, cudaMemcpyHostToDevice, ctx->stream));
+    unsigned char* dout = (unsigned char*)ctx->d_jac.p;
+    a.in = (const double*)din; a.S0 = (const double*)(din + vb); a.P = n;
+    if (kb) { a.strike = (const double*)(din + vb + s0b); a.strike_stride = M; }
+    a.out = (double*)dout;
+    a.status = (inverse && status) ? (int32_t*)(dout + vb) : nullptr;
+    rc = launch_iv(ctx, a, inverse, ctx->stream);
+    if (rc) return rc;
+    const size_t ob = vb + (a.status ? (size_t)n * M * sizeof(int32_t) : 0);
+    DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, dout, ob, cudaMemcpyDeviceToHost, ctx->stream));
+    DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    const unsigned char* res = (const unsigned char*)ctx->h_res.p;
+    host_copy(out + lo * (int64_t)M, res, vb);
+    if (a.status) host_copy(status + lo * (int64_t)M, res + vb, (size_t)n * M * sizeof(int32_t));
+  }
+  return book_used(ctx, ctx->stream);
+}
+
+}  // namespace
+
+int dhj_implied_vol(dhj_ctx* ctx, const double* price, int64_t P, const double* S0, int64_t s0_stride, double r,
+                    double q, const double* strike, int64_t strike_stride, const double* maturity,
+                    const int32_t* is_call, int32_t M, double* out_vol, int32_t* out_status) {
+  return run_iv_host(ctx, true, price, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, out_vol,
+                     out_status);
+}
+
+int dhj_bs_price(dhj_ctx* ctx, const double* vol, int64_t P, const double* S0, int64_t s0_stride, double r, double q,
+                 const double* strike, int64_t strike_stride, const double* maturity, const int32_t* is_call,
+                 int32_t M, double* out_price) {
+  return run_iv_host(ctx, false, vol, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, out_price,
+                     nullptr);
+}
+
+int dhj_implied_vol_dev(dhj_ctx* ctx, const double* d_price, int64_t P, const double* d_S0, int64_t s0_stride,
+                        double r, double q, const double* strike, int32_t scale_by_spot, const double* maturity,
+                        const int32_t* is_call, int32_t M, double* d_out_vol, int32_t* d_out_status, void* stream) {
+  int rc = check_iv(ctx, d_price, P, d_S0, s0_stride, d_out_vol, M);
+  if (rc) return rc;
+  if (M == 0 || P == 0) return DHJ_OK;
+  if (!strike || !maturity || !is_call) return fail(ctx, DHJ_ERR_ARG, "null option table");
+  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = (cudaStream_t)stream;   // NULL = the default stream
+  iv::IvArgs a{};
+  rc = upload_iv_tables(ctx, strike, true, maturity, is_call, M, st, &a);
+  if (rc) return rc;
+  a.in = d_price; a.S0 = d_S0; a.s0_stride = s0_stride; a.scale_by_spot = scale_by_spot ? 1 : 0;
+  a.r = r; a.q = q; a.P = P; a.M = M; a.out = d_out_vol; a.status = d_out_status;
+  rc = launch_iv(ctx, a, true, st);
+  if (rc) return rc;
+  return book_used(ctx, st);
 }
 
 // f and the analytic g of B loss evaluations: exp/tanh transform (k_fd_expand without a stencil) -> prices of every

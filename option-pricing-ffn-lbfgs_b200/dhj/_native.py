@@ -17,6 +17,8 @@ from numpy.ctypeslib import ndpointer
 N_PARAMS = 13
 N_GREEKS = 5
 GREEKS = ("delta", "gamma", "theta", "rho", "rho_q")
+# status codes of implied_vol (include/dhj.h)
+IV_STATUS = ("ok", "below_lower_bound", "above_upper_bound", "invalid_input", "not_converged")
 FD_POINTS = 14
 LIB_PATH = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "lib", "libdhj.so")
 
@@ -29,6 +31,7 @@ EXPORTS = (
     "dhj_lbfgs_create", "dhj_lbfgs_destroy", "dhj_lbfgs_ask", "dhj_lbfgs_tell", "dhj_lbfgs_result", "dhj_lbfgs_minimize_fd",
     "dhj_generator_draws", "dhj_generate_dev", "dhj_generate", "dhj_set_host_threads", "dhj_debug_checks",
     "dhj_price_jacobian", "dhj_loss_grad", "dhj_lbfgs_minimize_grad", "dhj_price_greeks",
+    "dhj_implied_vol", "dhj_implied_vol_dev", "dhj_bs_price",
 )
 
 
@@ -99,6 +102,12 @@ def load_library(path: str | None = None) -> ctypes.CDLL:
         lib.dhj_price_jacobian.argtypes = [_c_vp, _F64, _c_i64, _F64, _c_i64, _c_f64, _c_f64, _F64, _c_i64, _F64,
                                            _I32, _c_i32, _c_i32, _c_f64, _c_vp, _c_vp]
         lib.dhj_price_greeks.argtypes = lib.dhj_price_jacobian.argtypes
+        lib.dhj_implied_vol.argtypes = [_c_vp, _F64, _c_i64, _F64, _c_i64, _c_f64, _c_f64, _F64, _c_i64, _F64, _I32,
+                                        _c_i32, _c_vp, _c_vp]
+        lib.dhj_implied_vol_dev.argtypes = [_c_vp, _c_vp, _c_i64, _c_vp, _c_i64, _c_f64, _c_f64, _F64, _c_i32, _F64,
+                                            _I32, _c_i32, _c_vp, _c_vp, _c_vp]
+        lib.dhj_bs_price.argtypes = [_c_vp, _F64, _c_i64, _F64, _c_i64, _c_f64, _c_f64, _F64, _c_i64, _F64, _I32,
+                                     _c_i32, _c_vp]
         lib.dhj_loss_grad.argtypes = [_c_vp, _c_vp, _F64, _c_vp, _c_i64, _F64, _F64]
         lib.dhj_lbfgs_minimize_grad.argtypes = [_c_vp, _c_vp, _c_vp, _c_vp, _c_i64, ctypes.POINTER(_c_i64),
                                                 ctypes.POINTER(_c_i64), _F64]
@@ -205,6 +214,69 @@ class Context:
                                                    k_stride, maturity, call, M, int(N), float(L), _ptr(prices),
                                                    _ptr(greeks)), "dhj_price_greeks")
         return prices, greeks
+
+    # -- implied volatility -----------------------------------------------------------------------
+    @staticmethod
+    def _iv_list(values, S0, strike, maturity, is_call):
+        maturity = _f64(maturity).reshape(-1)
+        M = maturity.shape[0]
+        values = _f64(values)
+        if values.ndim == 2 and values.shape[1] == M:
+            P = values.shape[0]
+        elif M and values.size % M == 0:
+            P = values.size // M
+        else:
+            raise ValueError("values must be [M] or [P, M]")
+        values = values.reshape(P, M)
+        S0 = _f64(S0).reshape(-1)
+        if S0.size not in (1, P):
+            raise ValueError("S0 must be a scalar or have one entry per row")
+        strike = _f64(strike)
+        if strike.size == M:
+            strike, k_stride = strike.reshape(M), 0
+        elif strike.size == P * M:
+            strike, k_stride = strike.reshape(P, M), M
+        else:
+            raise ValueError("strike must be [M] or [P, M]")
+        call = np.ascontiguousarray(np.broadcast_to(np.asarray(is_call), (M,)).astype(bool).astype(np.int32))
+        return values, P, S0, 0 if S0.size == 1 else 1, strike, k_stride, maturity, M, call
+
+    def implied_vol(self, price, S0, strike, maturity, is_call, r, q=0.0, return_status=False):
+        """Black–Scholes implied vols float64[P, M] of prices [P, M] (or [M]) on an option list in price_list's layout:
+        S0 scalar or [P], strike [M] or [P, M] (dhj_implied_vol).  NaN outside the no-arbitrage bounds; with
+        return_status also the int32[P, M] status codes (IV_STATUS names them)."""
+        price, P, S0, s0_stride, strike, k_stride, maturity, M, call = self._iv_list(price, S0, strike, maturity,
+                                                                                     is_call)
+        vol, status = np.empty((P, M)), np.empty((P, M), dtype=np.int32)
+        with self._lock:
+            self._check(self._lib.dhj_implied_vol(self._h, price, P, S0, s0_stride, float(r), float(q), strike,
+                                                  k_stride, maturity, call, M, _ptr(vol), _ptr(status)),
+                        "dhj_implied_vol")
+        return (vol, status) if return_status else vol
+
+    def implied_vol_dev(self, d_price: int, P: int, d_S0: int, s0_stride: int, strike, maturity, is_call, r, q,
+                        d_out_vol: int, d_out_status: int = 0, scale_by_spot=False, stream: int = 0):
+        """Asynchronous device-pointer variant (dhj_implied_vol_dev): pointers and the stream are ints, the tables
+        strike[M], maturity[M], is_call[M] host arrays; scale_by_spot: K = strike * S0 / 100."""
+        strike, maturity = _f64(strike).reshape(-1), _f64(maturity).reshape(-1)
+        M = maturity.size
+        if strike.size != M:
+            raise ValueError("strike must be [M]")
+        call = np.ascontiguousarray(np.broadcast_to(np.asarray(is_call), (M,)).astype(bool).astype(np.int32))
+        with self._lock:
+            self._check(self._lib.dhj_implied_vol_dev(self._h, d_price, int(P), d_S0, int(s0_stride), float(r),
+                                                      float(q), strike, int(bool(scale_by_spot)), maturity, call, M,
+                                                      d_out_vol, d_out_status or None, stream or None),
+                        "dhj_implied_vol_dev")
+
+    def bs_price(self, vol, S0, strike, maturity, is_call, r, q=0.0):
+        """Black–Scholes prices float64[P, M] of vols [P, M] (or [M]) in implied_vol's layout (dhj_bs_price)."""
+        vol, P, S0, s0_stride, strike, k_stride, maturity, M, call = self._iv_list(vol, S0, strike, maturity, is_call)
+        out = np.empty((P, M))
+        with self._lock:
+            self._check(self._lib.dhj_bs_price(self._h, vol, P, S0, s0_stride, float(r), float(q), strike, k_stride,
+                                               maturity, call, M, _ptr(out)), "dhj_bs_price")
+        return out
 
     @staticmethod
     def _option_list(params, S0, strike, maturity, is_call):

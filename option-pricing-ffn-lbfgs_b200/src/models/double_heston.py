@@ -106,3 +106,10 @@ class DoubleHeston():
         _, g = self._ctx.price_greeks(self._params(), self.S0, [self.K], [self.T], [self._is_call()], self.r, self.q,
                                       N)
         return {name: np.float64(g[0, 0, i]) for i, name in enumerate(GREEKS)}
+
+    def implied_volatility(self, N=128):
+        """Black–Scholes implied volatility of pricing(N) at the same S0, K, T, r, q and option type (extension, not
+        in the reference): NaN where the COS price lies outside the no-arbitrage bounds — two kernel launches."""
+        price = self._ctx.price_list(self._params(), self.S0, [self.K], [self.T], [self._is_call()], self.r, self.q, N)
+        vol = self._ctx.implied_vol(price, self.S0, [self.K], [self.T], [self._is_call()], self.r, self.q)
+        return np.float64(vol[0, 0])
