@@ -242,6 +242,31 @@ DHJ_API int dhj_bs_price(dhj_ctx* ctx, const double* vol, int64_t P, const doubl
                          double q, const double* strike, int64_t strike_stride, const double* maturity,
                          const int32_t* is_call, int32_t M, double* out_price);
 
+/* ---- Implied-volatility calibration objective ---------------------------------------------------
+ * dhj_market_set_objective selects what dhj_loss_batch, dhj_loss_fd, dhj_loss_grad, dhj_lbfgs_minimize_fd and
+ * dhj_lbfgs_minimize_grad compute on `market`:
+ *   DHJ_OBJECTIVE_PRICE (the default): compute_loss, the mean squared relative price error + Feller penalty;
+ *   DHJ_OBJECTIVE_IV:  f = (1/M_v) sum_{o valid} (sigma_o(x) - sigma^_o)^2 + Feller penalty, where sigma_o(x) is the
+ *                      Black-Scholes implied vol (q = 0, the market's S0, K, T, r) of the model price, sigma^_o that of
+ *                      the market price, and M_v the number of valid options of the market.
+ * Setting DHJ_OBJECTIVE_IV inverts the stored market prices once on the device (dhj_implied_vol's solver); a quote
+ * whose status is not 0 (below the lower bound, at or above the upper bound, invalid, not converged) has no implied
+ * vol and is left out of the objective.  out_market_vol[n_markets][M] (sigma^, NaN where left out) and
+ * out_status[n_markets][M] may be NULL (both are filled on failure too).  A market with no valid option makes the
+ * call fail with DHJ_ERR_ARG; the object's objective and market vols are then left as they were.
+ * On the IV objective f = 1e10 and g = 0 when a valid option has a model price NaN, inf or <= 0, a model-price
+ * implied-vol status != 0 or a vega that is not a positive normal number.  dhj_loss_grad's g is exact with the
+ * truncation range held fixed: (2/M_v) sum (sigma_o - sigma^_o) (dV_o/dp) / vega_o, chained to x as on the price
+ * objective.  f has the same bits on every entry point.
+ * dhj_market_implied_vols: model implied vols out_vol[B][M] and their status out_status[B][M] (may be NULL) at the
+ * transformed x, every option of the selected market (reporting; any objective). */
+#define DHJ_OBJECTIVE_PRICE 0
+#define DHJ_OBJECTIVE_IV 1
+DHJ_API int dhj_market_set_objective(dhj_ctx* ctx, dhj_market* market, int32_t objective, double* out_market_vol,
+                                     int32_t* out_status);
+DHJ_API int dhj_market_implied_vols(dhj_ctx* ctx, const dhj_market* market, const double* x,
+                                    const int32_t* market_index, int64_t B, double* out_vol, int32_t* out_status);
+
 /* Threads used by the library's host-side parallel loops (optimiser states in ask / tell, staging copies of pageable
  * buffers); 0 = all cores (default).  Several lock-step pipelines on one host divide the cores with this. */
 DHJ_API int dhj_set_host_threads(int32_t n);

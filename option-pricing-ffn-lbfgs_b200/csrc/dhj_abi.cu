@@ -18,6 +18,7 @@
 #include "dhj_jac.cuh"
 #include "dhj_generate.cuh"
 #include "dhj_iv.cuh"
+#include "dhj_ivloss.cuh"
 
 using namespace dhj;
 
@@ -171,6 +172,7 @@ struct dhj_ctx {
   Slot slots[kSlots];
   // loss path
   DevBuf d_x, d_xv, d_idx, d_f, d_fg, d_counters, d_prices, d_jac;
+  DevBuf d_ivres;                             // IV objective: model vols | 1 / vega per unit and option
   PinBuf h_x, h_res;
   size_t counters_zeroed = 0;
   DevBuf d_peak;
@@ -204,6 +206,10 @@ struct dhj_market {
   DevBuf d_book, d_strike, d_S0, d_price;
   long long strike_stride = 0;
   SliceView view{};
+  // implied-volatility objective (dhj_market_set_objective): market vols [n_markets][M] (NaN: left out) and the
+  // option tables in the caller's order, maturity[M] | is_call[M] (made on first use)
+  int objective = DHJ_OBJECTIVE_PRICE;
+  DevBuf d_mvol, d_ivtab;
 };
 
 namespace {
@@ -573,7 +579,7 @@ int dhj_destroy(dhj_ctx* ctx) {
   }
   ctx->d_x.release(); ctx->d_xv.release(); ctx->d_idx.release(); ctx->d_f.release(); ctx->d_fg.release();
   ctx->d_counters.release(); ctx->d_prices.release(); ctx->d_jac.release(); ctx->h_x.release(); ctx->h_res.release();
-  ctx->d_peak.release();
+  ctx->d_peak.release(); ctx->d_ivres.release();
   for (DevBuf& b : ctx->pool) b.release();
   ctx->pool.clear();
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -712,12 +718,17 @@ int dhj_market_destroy(dhj_market* mk) {
     cudaStreamSynchronize(mk->ctx->stream);
     mk->ctx->pool_give(&mk->d_book); mk->ctx->pool_give(&mk->d_strike);
     mk->ctx->pool_give(&mk->d_S0); mk->ctx->pool_give(&mk->d_price);
+    mk->ctx->pool_give(&mk->d_mvol); mk->ctx->pool_give(&mk->d_ivtab);
   } else {
     mk->d_book.release(); mk->d_strike.release(); mk->d_S0.release(); mk->d_price.release();
+    mk->d_mvol.release(); mk->d_ivtab.release();
   }
   delete mk;
   return DHJ_OK;
 }
+
+static int launch_iv_residual(dhj_ctx* ctx, const dhj_market* mk, const double* prices, const int* row_index,
+                              long long n_units, double* vol, double* inv_vega, int32_t* status);
 
 static int run_loss(dhj_ctx* ctx, const dhj_market* mk, const double* x, const int32_t* market_index, int64_t B,
                     int fd, double h, double* out_f, double* out_g, double* out_f_all) {
@@ -745,7 +756,8 @@ static int run_loss(dhj_ctx* ctx, const dhj_market* mk, const double* x, const i
     const char* e = getenv("DHJ_DEBUG_SPLIT_UNITS");
     return e ? (int64_t)atoll(e) : (int64_t)8192;
   }();
-  if (mk->book.max_slice <= kBatchMaxStrikes && v.n_slices <= kPriceItems && n_units < kSplitUnits) {
+  const bool iv_objective = mk->objective == DHJ_OBJECTIVE_IV;
+  if (!iv_objective && mk->book.max_slice <= kBatchMaxStrikes && v.n_slices <= kPriceItems && n_units < kSplitUnits) {
     // fused path: one launch
     if (fd) {
       const size_t cb = (size_t)B * sizeof(unsigned int);
@@ -782,10 +794,22 @@ static int run_loss(dhj_ctx* ctx, const dhj_market* mk, const double* x, const i
     ctx->launches++;
     rc = launch_price(ctx, v, pa, mk->book.max_slice, ctx->stream);
     if (rc) return rc;
-    k_loss_reduce<<<(unsigned)((B + 127) / 128), 128, 0, ctx->stream>>>(
-        (const double*)ctx->d_prices.p, (const double*)ctx->d_xv.p, (const int*)ctx->d_idx.p,
-        (const double*)mk->d_price.p, v.pos, mk->M, B, fd, h, (const double*)ctx->d_x.p, (double*)ctx->d_f.p,
-        fd ? (double*)ctx->d_fg.p : nullptr);
+    if (iv_objective) {
+      // IV objective (dhj_ivloss.cuh): always this path; model vols per (point, option), then the reduction
+      DHJ_CUDA(ctx, ctx->d_ivres.reserve((size_t)n_units * mk->M * sizeof(double)));
+      double* vol = (double*)ctx->d_ivres.p;
+      rc = launch_iv_residual(ctx, mk, (const double*)ctx->d_prices.p, (const int*)ctx->d_idx.p, n_units, vol,
+                              nullptr, nullptr);
+      if (rc) return rc;
+      k_loss_iv_reduce<<<(unsigned)((B + 127) / 128), 128, 0, ctx->stream>>>(
+          vol, (const double*)ctx->d_xv.p, (const int*)ctx->d_idx.p, (const double*)mk->d_mvol.p, v.pos, mk->M, B,
+          fd, h, (const double*)ctx->d_x.p, (double*)ctx->d_f.p, fd ? (double*)ctx->d_fg.p : nullptr);
+    } else {
+      k_loss_reduce<<<(unsigned)((B + 127) / 128), 128, 0, ctx->stream>>>(
+          (const double*)ctx->d_prices.p, (const double*)ctx->d_xv.p, (const int*)ctx->d_idx.p,
+          (const double*)mk->d_price.p, v.pos, mk->M, B, fd, h, (const double*)ctx->d_x.p, (double*)ctx->d_f.p,
+          fd ? (double*)ctx->d_fg.p : nullptr);
+    }
     DHJ_CUDA(ctx, cudaGetLastError());
     ctx->launches++;
   }
@@ -1113,12 +1137,14 @@ static int run_loss_grad(dhj_ctx* ctx, const dhj_market* mk, const double* x, co
   if (!out_f || !out_g) return fail(ctx, DHJ_ERR_ARG, "null output");
   if (B == 0) return DHJ_OK;
   const int M = mk->M;
+  const bool iv_objective = mk->objective == DHJ_OBJECTIVE_IV;
   const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(B, (int64_t)(((size_t)1 << 27) / ((size_t)M * kJacChannels))));
   DHJ_CUDA(ctx, ctx->d_xv.reserve((size_t)B * kNumParams * sizeof(double)));
   DHJ_CUDA(ctx, ctx->d_idx.reserve((size_t)B * sizeof(int)));
   DHJ_CUDA(ctx, ctx->d_fg.reserve((size_t)B * kFdPoints * sizeof(double)));
   DHJ_CUDA(ctx, ctx->d_prices.reserve((size_t)2 * chunk * M * sizeof(double)));   // pricing kernel | k_price_jac
   DHJ_CUDA(ctx, ctx->d_jac.reserve((size_t)chunk * M * kNumParams * sizeof(double)));
+  if (iv_objective) DHJ_CUDA(ctx, ctx->d_ivres.reserve((size_t)2 * chunk * M * sizeof(double)));   // vol | 1/vega
   double* pv = (double*)ctx->d_xv.p;
   int* idx = (int*)ctx->d_idx.p;
   double* fg = (double*)ctx->d_fg.p;
@@ -1139,9 +1165,19 @@ static int run_loss_grad(dhj_ctx* ctx, const dhj_market* mk, const double* x, co
     a.P = n; a.out_price = prices + n * (int64_t)M; a.out_jac = (double*)ctx->d_jac.p;
     rc = launch_jac(ctx, mk->view, a, ctx->stream);
     if (rc) return rc;
-    k_loss_grad_reduce<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(
-        prices, a.out_jac, a.params, a.row_index, (const double*)mk->d_price.p, mk->view.pos, M, n,
-        fg + lo * kFdPoints);
+    if (iv_objective) {
+      double* vol = (double*)ctx->d_ivres.p;
+      double* inv_vega = vol + n * (int64_t)M;
+      rc = launch_iv_residual(ctx, mk, prices, a.row_index, n, vol, inv_vega, nullptr);
+      if (rc) return rc;
+      k_loss_iv_grad_reduce<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(
+          vol, inv_vega, a.out_jac, a.params, a.row_index, (const double*)mk->d_mvol.p, mk->view.pos, M, n,
+          fg + lo * kFdPoints);
+    } else {
+      k_loss_grad_reduce<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(
+          prices, a.out_jac, a.params, a.row_index, (const double*)mk->d_price.p, mk->view.pos, M, n,
+          fg + lo * kFdPoints);
+    }
     DHJ_CUDA(ctx, cudaGetLastError());
     ctx->launches++;
   }
@@ -1232,6 +1268,136 @@ int dhj_market_prices(dhj_ctx* ctx, const dhj_market* mk, const double* x, const
   DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, ctx->d_prices.p, ob, cudaMemcpyDeviceToHost, ctx->stream));
   DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   memcpy(out_prices, ctx->h_res.p, ob);
+  return DHJ_OK;
+}
+
+// ---- implied-volatility objective (dhj_ivloss.cuh) ---------------------------------------------------
+// maturity[M] | is_call[M] of the market in the caller's option order, rebuilt from the slice book
+static int ensure_iv_tables(dhj_ctx* ctx, dhj_market* mk) {
+  if (mk->d_ivtab.p) return DHJ_OK;
+  const int M = mk->M;
+  const BookHost& b = mk->book;
+  std::vector<unsigned char> image((size_t)M * (sizeof(double) + sizeof(int32_t)));
+  double* T = (double*)image.data();
+  int32_t* call = (int32_t*)(image.data() + (size_t)M * sizeof(double));
+  for (int s = 0; s < b.n_slices; ++s)
+    for (int d = b.slice_off[s]; d < b.slice_off[s + 1]; ++d) {
+      T[b.pos[d]] = b.slice_T[s];
+      call[b.pos[d]] = b.call[d];
+    }
+  DHJ_CUDA(ctx, ctx->pool_take(&mk->d_ivtab, image.size()));
+  DHJ_CUDA(ctx, cudaMemcpyAsync(mk->d_ivtab.p, image.data(), image.size(), cudaMemcpyHostToDevice, ctx->stream));
+  DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return DHJ_OK;
+}
+
+// k_iv_residual over n_units x M (grid-stride, as launch_iv); status non-null: reporting mode
+static int launch_iv_residual(dhj_ctx* ctx, const dhj_market* mk, const double* prices, const int* row_index,
+                              long long n_units, double* vol, double* inv_vega, int32_t* status) {
+  IvResidualArgs a;
+  a.prices = prices; a.row_index = row_index; a.S0 = (const double*)mk->d_S0.p;
+  a.strike = (const double*)mk->d_strike.p; a.strike_stride = mk->strike_stride;
+  a.maturity = (const double*)mk->d_ivtab.p;
+  a.is_call = (const int32_t*)((const unsigned char*)mk->d_ivtab.p + (size_t)mk->M * sizeof(double));
+  a.mvol = (const double*)mk->d_mvol.p; a.r = mk->r; a.n_units = n_units; a.M = mk->M; a.n_markets = mk->n_markets;
+  a.vol = vol; a.inv_vega = inv_vega; a.status = status;
+  const long long n = n_units * (long long)mk->M;
+  const long long blocks = std::max<long long>(1, std::min<long long>((n + 255) / 256, 32LL * ctx->sm_count));
+  k_iv_residual<<<(int)blocks, 256, 0, ctx->stream>>>(a);
+  DHJ_CUDA(ctx, cudaGetLastError());
+  ctx->launches++;
+  return DHJ_OK;
+}
+
+int dhj_market_set_objective(dhj_ctx* ctx, dhj_market* mk, int32_t objective, double* out_market_vol,
+                             int32_t* out_status) {
+  if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
+  if (!mk) return fail(ctx, DHJ_ERR_ARG, "null market");
+  if (mk->ctx != ctx) return fail(ctx, DHJ_ERR_ARG, "market belongs to another context");
+  if (objective != DHJ_OBJECTIVE_PRICE && objective != DHJ_OBJECTIVE_IV)
+    return fail(ctx, DHJ_ERR_ARG, "unknown objective %d", objective);
+  if (objective == DHJ_OBJECTIVE_PRICE) { mk->objective = objective; return DHJ_OK; }
+  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
+  int rc = ensure_iv_tables(ctx, mk);
+  if (rc) return rc;
+  const int M = mk->M;
+  const size_t n_opt = (size_t)mk->n_markets * M;
+  // the quotes are inverted into scratch: the market's vols and objective change only when the call succeeds
+  DHJ_CUDA(ctx, ctx->d_ivres.reserve(n_opt * (sizeof(double) + sizeof(int32_t))));
+  // the market's quotes through dhj_implied_vol's solver (q = 0, as the market assumes)
+  iv::IvArgs a{};
+  a.in = (const double*)mk->d_price.p; a.S0 = (const double*)mk->d_S0.p; a.s0_stride = 1;
+  a.strike = (const double*)mk->d_strike.p; a.strike_stride = mk->strike_stride; a.scale_by_spot = 0;
+  a.maturity = (const double*)mk->d_ivtab.p;
+  a.is_call = (const int32_t*)((const unsigned char*)mk->d_ivtab.p + (size_t)M * sizeof(double));
+  a.r = mk->r; a.q = 0.0; a.P = mk->n_markets; a.M = M;
+  a.out = (double*)ctx->d_ivres.p; a.status = (int32_t*)((double*)ctx->d_ivres.p + n_opt);
+  rc = launch_iv(ctx, a, true, ctx->stream);
+  if (rc) return rc;
+  std::vector<double> vol(n_opt);
+  std::vector<int32_t> st(n_opt);
+  DHJ_CUDA(ctx, cudaMemcpyAsync(vol.data(), a.out, n_opt * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  DHJ_CUDA(ctx, cudaMemcpyAsync(st.data(), a.status, n_opt * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  // a quote without an implied vol (status != 0; "not converged" returns its last iterate) is left out: NaN
+  int empty = -1;
+  for (int m = 0; m < mk->n_markets; ++m) {
+    int valid = 0;
+    for (int o = 0; o < M; ++o) {
+      const size_t i = (size_t)m * M + o;
+      if (st[i] != iv::kOk) vol[i] = NAN;
+      else ++valid;
+    }
+    if (!valid && empty < 0) empty = m;
+  }
+  if (out_market_vol) memcpy(out_market_vol, vol.data(), n_opt * sizeof(double));
+  if (out_status) memcpy(out_status, st.data(), n_opt * sizeof(int32_t));
+  if (empty >= 0)
+    return fail(ctx, DHJ_ERR_ARG, "market %d has no option with an implied vol (every quote's status is != 0)", empty);
+  if (!mk->d_mvol.p) DHJ_CUDA(ctx, ctx->pool_take(&mk->d_mvol, n_opt * sizeof(double)));
+  DHJ_CUDA(ctx, cudaMemcpyAsync(mk->d_mvol.p, vol.data(), n_opt * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  mk->objective = DHJ_OBJECTIVE_IV;
+  return DHJ_OK;
+}
+
+int dhj_market_implied_vols(dhj_ctx* ctx, const dhj_market* market, const double* x, const int32_t* market_index,
+                            int64_t B, double* out_vol, int32_t* out_status) {
+  if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
+  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
+  const int* d_index = nullptr;
+  int rc = stage_x(ctx, market, x, market_index, B, &d_index);
+  if (rc) return rc;
+  if (!out_vol) return fail(ctx, DHJ_ERR_ARG, "null output");
+  if (B == 0) return DHJ_OK;
+  dhj_market* mk = const_cast<dhj_market*>(market);   // the option tables are a cache of the market's own book
+  rc = ensure_iv_tables(ctx, mk);
+  if (rc) return rc;
+  const int M = mk->M;
+  const size_t nb = (size_t)B * M;
+  DHJ_CUDA(ctx, ctx->d_xv.reserve((size_t)B * kNumParams * sizeof(double)));
+  DHJ_CUDA(ctx, ctx->d_idx.reserve((size_t)B * sizeof(int)));
+  DHJ_CUDA(ctx, ctx->d_prices.reserve(nb * sizeof(double)));
+  DHJ_CUDA(ctx, ctx->d_ivres.reserve(nb * (sizeof(double) + sizeof(int32_t))));
+  DHJ_CUDA(ctx, ctx->h_res.reserve(nb * (sizeof(double) + sizeof(int32_t))));
+  k_fd_expand<<<(unsigned)((B + 127) / 128), 128, 0, ctx->stream>>>((const double*)ctx->d_x.p, d_index, B, 0, 0.0,
+                                                                   (double*)ctx->d_xv.p, (int*)ctx->d_idx.p);
+  DHJ_CUDA(ctx, cudaGetLastError());
+  ctx->launches++;
+  PriceArgs pa;
+  pa.params = (const double*)ctx->d_xv.p; pa.S0 = (const double*)mk->d_S0.p; pa.s0_stride = 1;
+  pa.row_index = (const int*)ctx->d_idx.p; pa.P = B; pa.transform = 0; pa.out = (double*)ctx->d_prices.p;
+  rc = launch_price(ctx, mk->view, pa, mk->book.max_slice, ctx->stream);
+  if (rc) return rc;
+  double* vol = (double*)ctx->d_ivres.p;
+  int32_t* st = (int32_t*)(vol + nb);
+  rc = launch_iv_residual(ctx, mk, pa.out, pa.row_index, B, vol, nullptr, st);
+  if (rc) return rc;
+  DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, vol, nb * (sizeof(double) + sizeof(int32_t)), cudaMemcpyDeviceToHost,
+                                ctx->stream));
+  DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  host_copy(out_vol, ctx->h_res.p, nb * sizeof(double));
+  if (out_status) host_copy(out_status, (const double*)ctx->h_res.p + nb, nb * sizeof(int32_t));
   return DHJ_OK;
 }
 

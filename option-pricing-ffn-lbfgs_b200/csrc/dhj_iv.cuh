@@ -54,6 +54,9 @@ double erfcx_(double z);   // provided by the host emulation
 // e^{-(h^2 + t^2)/2}
 DHJ_HD double gauss2(double h, double t) { return exp(-0.5 * fma(h, h, t * t)); }
 
+// db/ds = e^{-(h^2 + t^2)/2} / sqrt(2 pi) at h = x/s, t = s/2: the normalised vega the solver steps with
+DHJ_HD double vega_norm(double x, double s) { return kInvSqrt2Pi * gauss2(x / s, 0.5 * s); }
+
 // b(x, s) for s < kSeriesMaxS (h = x/s <= 0, t = s/2)
 DHJ_HD double b_series(double h, double t) {
   if (h * h > 1500.0) return 0.0;   // e^{-h^2/2} underflows (and M_k would overflow)
@@ -166,10 +169,13 @@ DHJ_HD double log_moneyness(double S0, double K, double T, double r, double q) {
   return (log(k0) + p) + (k_rem / S0 + fma(d_err, T, p_err));
 }
 
-// Black–Scholes implied volatility of price V; *status as in include/dhj.h, *iters: solver evaluations
+// Black–Scholes implied volatility of price V; *status as in include/dhj.h, *iters: solver evaluations.
+// vega (optional): dV/dsigma at the returned sigma, D sqrt(FK) sqrt(T) vega_norm(x_o, s) from the solver's own x_o
+// and s (0 where sigma = 0, NaN where there is no sigma).
 DHJ_HD double implied_vol(double V, double S0, double K, double T, double r, double q, bool call, int* status,
-                          int* iters) {
+                          int* iters, double* vega = nullptr) {
   *iters = 0;
+  if (vega) *vega = NAN;
   if (!isfinite(V) || !valid_inputs(S0, K, T, r, q)) { *status = kInvalid; return NAN; }
   const double Sq = S0 * exp(-q * T), KD = K * exp(-r * T);
   const double lower = call ? fmax(Sq - KD, 0.0) : fmax(KD - Sq, 0.0);
@@ -177,16 +183,18 @@ DHJ_HD double implied_vol(double V, double S0, double K, double T, double r, dou
   if (V < lower) { *status = kBelowLower; return NAN; }
   if (V >= upper) { *status = kAboveUpper; return NAN; }
   *status = kOk;
+  if (vega) *vega = 0.0;
   if (V == lower) return 0.0;
   const double x = log_moneyness(S0, K, T, r, q);
   const double beta = V / (sqrt(Sq) * sqrt(KD));
   const double iota = ((call ? x : -x) > 0.0) ? 2.0 * sinh(0.5 * fabs(x)) : 0.0;
   const double beta_o = beta - iota, x_o = -fabs(x);
   if (!(beta_o > 0.0)) return 0.0;                          // within rounding of the intrinsic value
-  if (!(beta_o < exp(0.5 * x_o))) { *status = kAboveUpper; return NAN; }
+  if (!(beta_o < exp(0.5 * x_o))) { *status = kAboveUpper; if (vega) *vega = NAN; return NAN; }
   int converged;
   const double s = solve_s(x_o, beta_o, iters, &converged);
   if (!converged) *status = kNotConverged;
+  if (vega) *vega = (sqrt(Sq) * sqrt(KD)) * sqrt(T) * vega_norm(x_o, s);
   return s / sqrt(T);
 }
 

@@ -299,6 +299,25 @@ __global__ void __launch_bounds__(32 * kJacWarps) k_price_jac(SliceView v, JacAr
 //   - 2 kappa dtheta) where the excess sigma^2 - 2 kappa theta is > 0, else 0 (0 at the kink);
 //   dp/dx = p for the exp parameters, 1 - rho^2 for the two tanh parameters, 1 for mu_j.
 // Where the loss is the 1e10 sentinel (a price NaN, inf or <= 0) the gradient is 0.  fg[n][14] = (f, g[13]).
+//
+// loss_grad_tail is the part every analytic-gradient reduction shares (k_loss_grad_reduce here, k_loss_iv_grad_reduce
+// in dhj_ivloss.cuh): gp[13] holds d(data term)/dp; the Feller derivative is added and out[1 + j] = gp_j dp_j/dx_j.
+__device__ __forceinline__ void loss_grad_tail(const double* __restrict__ p, const Params& m, double* gp,
+                                               double* __restrict__ out) {
+  for (int f = 0; f < 2; ++f) {
+    const double e = m.sigma[f] * m.sigma[f] - 2.0 * m.kappa[f] * m.theta[f];
+    if (e > 0.0) {
+      gp[5 * f + 3] += 2000.0 * m.sigma[f];
+      gp[5 * f + 1] -= 2000.0 * m.theta[f];
+      gp[5 * f + 2] -= 2000.0 * m.kappa[f];
+    }
+  }
+  for (int j = 0; j < kNumParams; ++j) {
+    const double dpdx = (j == 4 || j == 9) ? 1.0 - p[j] * p[j] : ((j == 11) ? 1.0 : p[j]);
+    out[1 + j] = gp[j] * dpdx;
+  }
+}
+
 __global__ void k_loss_grad_reduce(const double* __restrict__ prices, const double* __restrict__ jac,
                                    const double* __restrict__ pv, const int* __restrict__ row_index,
                                    const double* __restrict__ market, const int* __restrict__ pos, int M, long long n_x,
@@ -331,18 +350,7 @@ __global__ void k_loss_grad_reduce(const double* __restrict__ prices, const doub
   out[0] = sq / (double)M + feller_penalty(m);
   const double two_m = 2.0 / (double)M;
   for (int j = 0; j < kNumParams; ++j) gp[j] *= two_m;
-  for (int f = 0; f < 2; ++f) {
-    const double e = m.sigma[f] * m.sigma[f] - 2.0 * m.kappa[f] * m.theta[f];
-    if (e > 0.0) {
-      gp[5 * f + 3] += 2000.0 * m.sigma[f];
-      gp[5 * f + 1] -= 2000.0 * m.theta[f];
-      gp[5 * f + 2] -= 2000.0 * m.kappa[f];
-    }
-  }
-  for (int j = 0; j < kNumParams; ++j) {
-    const double dpdx = (j == 4 || j == 9) ? 1.0 - p[j] * p[j] : ((j == 11) ? 1.0 : p[j]);
-    out[1 + j] = gp[j] * dpdx;
-  }
+  loss_grad_tail(p, m, gp, out);
 }
 
 }  // namespace dhj

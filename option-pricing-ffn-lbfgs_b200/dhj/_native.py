@@ -32,7 +32,10 @@ EXPORTS = (
     "dhj_generator_draws", "dhj_generate_dev", "dhj_generate", "dhj_set_host_threads", "dhj_debug_checks",
     "dhj_price_jacobian", "dhj_loss_grad", "dhj_lbfgs_minimize_grad", "dhj_price_greeks",
     "dhj_implied_vol", "dhj_implied_vol_dev", "dhj_bs_price",
+    "dhj_market_set_objective", "dhj_market_implied_vols",
 )
+# calibration objectives of a Market (dhj_market_set_objective)
+OBJECTIVES = {"price": 0, "iv": 1}
 
 
 class NativeError(RuntimeError):
@@ -109,6 +112,8 @@ def load_library(path: str | None = None) -> ctypes.CDLL:
         lib.dhj_bs_price.argtypes = [_c_vp, _F64, _c_i64, _F64, _c_i64, _c_f64, _c_f64, _F64, _c_i64, _F64, _I32,
                                      _c_i32, _c_vp]
         lib.dhj_loss_grad.argtypes = [_c_vp, _c_vp, _F64, _c_vp, _c_i64, _F64, _F64]
+        lib.dhj_market_set_objective.argtypes = [_c_vp, _c_vp, _c_i32, _c_vp, _c_vp]
+        lib.dhj_market_implied_vols.argtypes = [_c_vp, _c_vp, _F64, _c_vp, _c_i64, _F64, _c_vp]
         lib.dhj_lbfgs_minimize_grad.argtypes = [_c_vp, _c_vp, _c_vp, _c_vp, _c_i64, ctypes.POINTER(_c_i64),
                                                 ctypes.POINTER(_c_i64), _F64]
         _U32 = ndpointer(dtype=np.uint32, flags="C_CONTIGUOUS")
@@ -469,6 +474,7 @@ class Market:
             raise ValueError("strike must be [M] or [n_markets, M]")
         call = np.ascontiguousarray(np.broadcast_to(np.asarray(is_call), (M,)).astype(bool).astype(np.int32))
         self.n_markets, self.M, self.N = n, M, int(N)
+        self.objective = "price"
         self._h = _c_vp()
         with ctx._lock:
             ctx._check(ctx._lib.dhj_market_create(ctx._h, n, M, S0, float(r), strike, k_stride, maturity, call, price,
@@ -526,6 +532,39 @@ class Market:
         with c._lock:
             c._check(c._lib.dhj_loss_grad(c._h, self._h, x, pidx, C, f, g), "dhj_loss_grad")
         return f, g
+
+    def set_objective(self, objective: str):
+        """Select what loss_batch, loss_fd, loss_grad and the BatchLBFGS loops compute on this market: "price" (the
+        default: relative price error + Feller) or "iv" (mean squared implied-vol error over the quotes that have an
+        implied vol + Feller; dhj_market_set_objective).  Returns (market_vols[n_markets, M], status[n_markets, M]):
+        the quotes' Black–Scholes implied vols (q = 0; NaN where status != 0: left out of the objective) and their
+        IV_STATUS codes ((None, None) for "price").  A market without any valid quote raises NativeError and the
+        market keeps its objective."""
+        if objective not in OBJECTIVES:
+            raise ValueError(f"objective must be 'price' or 'iv' (got {objective!r})")
+        vol = np.empty((self.n_markets, self.M)) if objective == "iv" else None
+        status = np.empty((self.n_markets, self.M), dtype=np.int32) if objective == "iv" else None
+        c = self.ctx
+        with c._lock:
+            c._check(c._lib.dhj_market_set_objective(c._h, self._h, OBJECTIVES[objective],
+                                                     _ptr(vol) if vol is not None else None,
+                                                     _ptr(status) if status is not None else None),
+                     "dhj_market_set_objective")
+        self.objective = objective
+        return vol, status
+
+    def implied_vols(self, x, market_index=None):
+        """(vol[B, M], status[B, M]): Black–Scholes implied vols (q = 0) of the model prices at the unconstrained x
+        and their IV_STATUS codes, every option (dhj_market_implied_vols)."""
+        x = _f64(x).reshape(-1, N_PARAMS)
+        B = x.shape[0]
+        idx, pidx = self._index(market_index, B)
+        vol, status = np.empty((B, self.M)), np.empty((B, self.M), dtype=np.int32)
+        c = self.ctx
+        with c._lock:
+            c._check(c._lib.dhj_market_implied_vols(c._h, self._h, x, pidx, B, vol, _ptr(status)),
+                     "dhj_market_implied_vols")
+        return vol, status
 
     def prices(self, x, market_index=None) -> np.ndarray:
         x = _f64(x).reshape(-1, N_PARAMS)

@@ -15,7 +15,7 @@ import numpy as np
 
 import os
 
-from ._native import BatchLBFGS, Context, default_context, set_host_threads
+from ._native import BatchLBFGS, Context, NativeError, default_context, set_host_threads
 
 PARAM_NAMES = ('v1_0', 'kappa1', 'theta1', 'sigma1', 'rho1', 'v2_0', 'kappa2', 'theta2', 'sigma2', 'rho2',
                'lambda_j', 'mu_j', 'sigma_j')
@@ -99,7 +99,8 @@ def default_pipelines() -> int:
 
 
 def calibrate_many(spots, risk_free_rate, strikes, maturities, is_call, prices, maxiter=300, multi_start=3,
-                   x0=None, ctx: Context | None = None, return_all_starts=False, pipelines=None, gradient="fd"):
+                   x0=None, ctx: Context | None = None, return_all_starts=False, pipelines=None, gradient="fd",
+                   objective="price"):
     """Calibrate n markets simultaneously.
 
     spots[n]; strikes[M] or [n, M]; maturities[M]; is_call[M]; prices[n, M]; optional x0[n, multi_start, 13].
@@ -116,16 +117,26 @@ def calibrate_many(spots, risk_free_rate, strikes, maturities, is_call, prices, 
     (14 loss evaluations, maxfun 15000 // 14 requests); "analytic" with the exact gradient of the loss (truncation
     range held fixed; one loss evaluation and its Jacobian per request, maxfun 15000 requests as scipy's default
     with a supplied jac).  `evaluations` counts loss evaluations: 14 per request on the FD path, 1 on the analytic.
+
+    `objective`: "price" (default) is the reference's loss; "iv" fits Black–Scholes implied vols (q = 0) instead: per
+    market, the mean squared error of the model's implied vols against the quotes' over the quotes that have one,
+    + Feller (DESIGN.md §6e; `final_loss` is that objective).  A quote whose implied vol has a status != 0 (e.g. a noised
+    price below the intrinsic value) is left out of its market's objective.  The result gains market_vols[n, M] (NaN
+    where left out), model_vols[n, M] (at the chosen x) and excluded_quotes[n].  A market with no valid quote is
+    dropped before the optimiser runs: its x, parameters, final_loss, model prices and vols are NaN, status is 4
+    (the optimiser's "abnormal"), success False and iterations 0; the other markets are unaffected.
     """
     if gradient not in ("fd", "analytic"):
         raise ValueError(f"gradient must be 'fd' or 'analytic' (got {gradient!r})")
+    if objective not in ("price", "iv"):
+        raise ValueError(f"objective must be 'price' or 'iv' (got {objective!r})")
     t0 = time.time()
     n_all = np.asarray(spots).size
     if pipelines is None:
         pipelines = default_pipelines()
     if pipelines > 1 and ctx is None and n_all >= _PIPELINE_MIN_MARKETS:
         return _calibrate_pipelined(spots, risk_free_rate, strikes, maturities, is_call, prices, maxiter, multi_start,
-                                    x0, return_all_starts, t0, int(pipelines), gradient)
+                                    x0, return_all_starts, t0, int(pipelines), gradient, objective)
     ctx = ctx or default_context()
     spots = np.ascontiguousarray(np.asarray(spots, dtype=np.float64).reshape(-1))
     n = spots.size
@@ -134,7 +145,22 @@ def calibrate_many(spots, risk_free_rate, strikes, maturities, is_call, prices, 
     if x0 is None:
         x0 = initial_guesses(spots, strikes, maturities, prices, multi_start)
     x0 = np.asarray(x0, dtype=np.float64).reshape(n * multi_start, 13)
+    iv = objective == "iv"
     market = ctx.market(spots, risk_free_rate, strikes, maturities, is_call, prices)
+    if iv:
+        try:
+            market_vols, market_status = market.set_objective("iv")
+        except NativeError:
+            # some market has no quote with an implied vol (its objective is undefined): it is dropped and the
+            # others run as one batch
+            market.close()
+            _, st = ctx.implied_vol(prices, spots, strikes, maturities, is_call, risk_free_rate, 0.0,
+                                    return_status=True)
+            keep = (st == 0).any(axis=1)
+            if keep.all():
+                raise
+            return _with_dropped(spots, risk_free_rate, strikes, maturities, is_call, prices, maxiter, multi_start,
+                                 x0.reshape(n, multi_start, 13), ctx, return_all_starts, gradient, keep, t0)
     state_market = np.repeat(np.arange(n, dtype=np.int32), multi_start)
     analytic = gradient == "analytic"
     opt = BatchLBFGS(x0, maxiter=maxiter, ftol=1e-9, gtol=1e-6, maxfun=15000 if analytic else 15000 // 14)
@@ -156,6 +182,8 @@ def calibrate_many(spots, risk_free_rate, strikes, maturities, is_call, prices, 
     rows = np.arange(n)
     bx = xs2[rows, best]
     model = market.prices(bx, market_index=np.arange(n, dtype=np.int32)) if n else np.empty((0, maturities.size))
+    if iv:
+        model_vols = market.implied_vols(bx, market_index=np.arange(n, dtype=np.int32))[0]
     market.close()
     out = {
         'x': bx, 'parameters': transform(bx), 'final_loss': fs2[rows, best],
@@ -169,14 +197,54 @@ def calibrate_many(spots, risk_free_rate, strikes, maturities, is_call, prices, 
         'seconds_loss': t_loss, 'seconds_ask': t_ask, 'seconds_tell': t_tell, 'state_rounds': active_sum,
         'seconds_setup': t_setup, 'seconds_loop': t_loop1 - t_loop0,
     }
+    if iv:
+        out.update({'market_vols': market_vols, 'model_vols': model_vols,
+                    'excluded_quotes': (market_status != 0).sum(axis=1)})
     if return_all_starts:
         out.update({'all_x': xs2, 'all_loss': fs2, 'all_nit': nit.reshape(n, multi_start),
                     'all_status': status.reshape(n, multi_start)})
     return out
 
 
+def _with_dropped(spots, risk_free_rate, strikes, maturities, is_call, prices, maxiter, multi_start, x0, ctx,
+                  return_all_starts, gradient, keep, t0):
+    """calibrate_many(objective="iv") when some markets have no valid quote: the others are calibrated as one batch
+    and every per-market array is scattered back; the dropped rows are NaN with status 4 (abnormal)."""
+    n, M = spots.size, maturities.size
+    kept = np.flatnonzero(keep)
+    k_all = strikes if np.asarray(strikes).size == M else np.asarray(strikes, dtype=np.float64).reshape(n, M)
+    out = {}
+    if kept.size:
+        sub = calibrate_many(spots[kept], risk_free_rate, k_all if k_all.ndim == 1 else k_all[kept], maturities,
+                             is_call, prices[kept], maxiter=maxiter, multi_start=multi_start, x0=x0[kept], ctx=ctx,
+                             return_all_starts=return_all_starts, pipelines=1, gradient=gradient, objective="iv")
+    else:
+        sub = {'rounds': 0, 'evaluations': 0, 'seconds_loss': 0.0, 'seconds_ask': 0.0, 'seconds_tell': 0.0,
+               'state_rounds': 0, 'seconds_setup': 0.0, 'seconds_loop': 0.0}
+    fill = {'x': (np.nan, (13,)), 'parameters': (np.nan, (13,)), 'final_loss': (np.nan, ()),
+            'iterations': (0, ()), 'status': (4, ()), 'success': (False, ()), 'best_start': (0, ()),
+            'model_prices': (np.nan, (M,)), 'market_vols': (np.nan, (M,)), 'model_vols': (np.nan, (M,)),
+            'excluded_quotes': (M, ())}
+    if return_all_starts:
+        fill.update({'all_x': (np.nan, (multi_start, 13)), 'all_loss': (np.nan, (multi_start,)),
+                     'all_nit': (0, (multi_start,)), 'all_status': (4, (multi_start,))})
+    dtypes = {'iterations': np.int32, 'status': np.int32, 'success': bool, 'best_start': np.int64,
+              'excluded_quotes': np.int64, 'all_nit': np.int32, 'all_status': np.int32}
+    for key, (value, shape) in fill.items():
+        dtype = sub[key].dtype if key in sub else dtypes.get(key, np.float64)
+        arr = np.full((n,) + shape, value, dtype=dtype)
+        if kept.size:
+            arr[kept] = sub[key]
+        out[key] = arr
+    for key, val in sub.items():
+        if key not in out:
+            out[key] = val
+    out['seconds'] = time.time() - t0
+    return out
+
+
 def _calibrate_pipelined(spots, risk_free_rate, strikes, maturities, is_call, prices, maxiter, multi_start, x0,
-                         return_all_starts, t0, n_pipes=2, gradient="fd"):
+                         return_all_starts, t0, n_pipes=2, gradient="fd", objective="price"):
     import threading
     spots = np.asarray(spots, dtype=np.float64).reshape(-1)
     n = spots.size
@@ -199,7 +267,8 @@ def _calibrate_pipelined(spots, risk_free_rate, strikes, maturities, is_call, pr
             k_local = strikes if strikes.size == maturities.size else strikes.reshape(n, -1)[lo:hi]
             parts[i] = calibrate_many(spots[lo:hi], risk_free_rate, k_local, maturities, is_call, prices[lo:hi],
                                       maxiter=maxiter, multi_start=multi_start, x0=x0[lo:hi], ctx=contexts[i],
-                                      return_all_starts=return_all_starts, pipelines=1, gradient=gradient)
+                                      return_all_starts=return_all_starts, pipelines=1, gradient=gradient,
+                                      objective=objective)
         except BaseException as exc:      # noqa: BLE001  (re-raised in the caller's thread)
             errors.append(exc)
 
@@ -257,7 +326,10 @@ def calibrate_many_sharded(spots, risk_free_rate, strikes, maturities, is_call, 
     local = calibrate_many(spots[lo:hi], risk_free_rate, k_local, maturities, is_call, prices[lo:hi],
                            x0=np.asarray(x0).reshape(n, ms, 13)[lo:hi], **kwargs)
     out = {}
-    for key in ('x', 'parameters', 'final_loss', 'iterations', 'status', 'success', 'best_start', 'model_prices'):
+    keys = ('x', 'parameters', 'final_loss', 'iterations', 'status', 'success', 'best_start', 'model_prices')
+    if kwargs.get('objective', 'price') == 'iv':                    # forwarded to calibrate_many through **kwargs
+        keys += ('market_vols', 'model_vols', 'excluded_quotes')
+    for key in keys:
         arr = np.asarray(local[key])
         out[key] = gather_rows(arr.astype(np.float64) if arr.dtype == bool else arr, n, group, device)
     out['success'] = out['success'].astype(bool)

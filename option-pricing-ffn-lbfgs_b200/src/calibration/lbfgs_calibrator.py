@@ -131,9 +131,23 @@ class DoubleHestonJumpCalibrator:
 
         self._ctx = default_context()        # created once per process, before any timed region
         self._market = None
+        self._iv_market = None               # the same options on the implied-vol objective (objective="iv")
 
     # -- device-side market ------------------------------------------------------------------------
-    def _device_market(self):
+    def _device_market(self, objective: str = "price"):
+        if objective == "iv":
+            if self._iv_market is None:
+                opts = self.market_options
+                is_call = [str(o['option_type']).upper()[0] == 'C' for o in opts]
+                mk = self._ctx.market(
+                    float(self.spot), float(self.risk_free_rate),
+                    [float(o['strike']) for o in opts], [float(o['maturity']) for o in opts], is_call,
+                    [float(o['price']) for o in opts], N=128)
+                mk.set_objective("iv")
+                self._iv_market = mk
+            return self._iv_market
+        if objective != "price":
+            raise ValueError(f"objective must be 'price' or 'iv' (got {objective!r})")
         if self._market is None:
             opts = self.market_options
             is_call = [str(o['option_type']).upper()[0] == 'C' for o in opts]     # double_heston.py:172
@@ -189,18 +203,20 @@ class DoubleHestonJumpCalibrator:
         self._track(loss)
         return loss
 
-    def compute_loss_and_grad(self, x: np.ndarray, gradient: str = "fd"):
+    def compute_loss_and_grad(self, x: np.ndarray, gradient: str = "fd", objective: str = "price"):
         """f(x) and scipy's 2-point forward-difference gradient (h = 1e-8) in ONE launch.  gradient="analytic": the
-        exact gradient instead (truncation range held fixed, g = 0 at the 1e10 sentinel); `n_calls` advances by 1."""
+        exact gradient instead (truncation range held fixed, g = 0 at the 1e10 sentinel); `n_calls` advances by 1.
+        objective="iv": f is the implied-vol objective (mean squared error of the model's Black–Scholes implied vols
+        against the quotes' over the quotes that have one, + Feller; DESIGN.md §6e) instead of compute_loss."""
+        market = self._device_market(objective)
         if gradient == "analytic":
-            f, g = self._device_market().loss_grad(np.asarray(x, dtype=np.float64).reshape(1, 13))
+            f, g = market.loss_grad(np.asarray(x, dtype=np.float64).reshape(1, 13))
             self.n_calls += 1
             self._track(f[0])
             return f[0], g[0]
         if gradient != "fd":
             raise ValueError(f"gradient must be 'fd' or 'analytic' (got {gradient!r})")
-        f, g, f_all = self._device_market().loss_fd(np.asarray(x, dtype=np.float64).reshape(1, 13), _FD_STEP,
-                                                    want_all=True)
+        f, g, f_all = market.loss_fd(np.asarray(x, dtype=np.float64).reshape(1, 13), _FD_STEP, want_all=True)
         self.n_calls += 14
         for v in f_all[0]:
             self._track(v)
@@ -245,7 +261,8 @@ class DoubleHestonJumpCalibrator:
         return minimize(fun=fun_and_grad, x0=x0, jac=True, method='L-BFGS-B',
                         options={'maxiter': maxiter, 'ftol': 1e-9, 'gtol': 1e-6, 'maxfun': maxfun})
 
-    def calibrate(self, maxiter: int = 300, multi_start: int = 3, *, x0=None, gradient: str = "fd") -> CalibrationResult:
+    def calibrate(self, maxiter: int = 300, multi_start: int = 3, *, x0=None, gradient: str = "fd",
+                  objective: str = "price") -> CalibrationResult:
         """Calibrate to the market prices with `multi_start` L-BFGS-B runs; the best (lowest loss) wins.
 
         `x0` (keyword-only extension, not in the reference): optional unconstrained starting points
@@ -255,11 +272,19 @@ class DoubleHestonJumpCalibrator:
         `gradient` (keyword-only extension): "fd" (default) is the reference's forward difference; "analytic" answers
         each scipy request with the exact gradient of the loss (one evaluation, `n_calls` + 1 per request, scipy's
         default maxfun = 15000 requests).
+
+        `objective` (keyword-only extension): "price" (default) is the reference's loss; "iv" fits the Black–Scholes
+        implied vols of the quotes instead: f = mean over the quotes that have an implied vol (status 0) of
+        (sigma_model - sigma_market)^2 + the Feller penalty (DESIGN.md §6e).  It works with both gradients.  With
+        objective="iv", `final_loss` (and `best_loss`) are values of that objective, not of compute_loss; the fields of
+        the result are otherwise the same (model_prices are the model's prices at the optimum).
         """
         if gradient not in ("fd", "analytic"):
             raise ValueError(f"gradient must be 'fd' or 'analytic' (got {gradient!r})")
+        if objective not in ("price", "iv"):
+            raise ValueError(f"objective must be 'price' or 'iv' (got {objective!r})")
         start_time = time.time()
-        market = self._device_market()
+        market = self._device_market(objective)
 
         # initial points in start order: keeps the reference's global-RNG consumption (:252-256)
         if x0 is None:
