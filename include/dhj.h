@@ -160,7 +160,9 @@ DHJ_API int dhj_lbfgs_result(const dhj_lbfgs* opt, double* x, double* f, int32_t
 /* The whole lock-step loop in one call (what dhj.calibrate_many runs per pipeline): ask -> dhj_loss_fd over every
  * state that waits for an evaluation, state i on market state_market[i] (NULL: market 0) -> tell, until all n_states
  * optimisers of `opt` have stopped.  rounds = launches, state_rounds = sum of evaluated states over the rounds,
- * seconds[3] = host time in ask / in the loss calls (copies + launch + wait) / in tell.  Outputs may be NULL. */
+ * seconds[3] = host time in ask / in the loss calls (copies + launch + wait) / in tell.  Outputs may be NULL.
+ * n_states must equal the optimiser's state count (state_market[n_states]) and its dimension must be 13;
+ * otherwise the call fails with DHJ_ERR_ARG before the first ask. */
 DHJ_API int dhj_lbfgs_minimize_fd(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market, const int32_t* state_market,
                                   int64_t n_states, double h, int64_t* rounds, int64_t* state_rounds, double* seconds);
 

@@ -29,35 +29,24 @@ namespace {
 
 char g_init_error[512] = "";
 
-struct DevBuf {
+// A growable buffer of device (DevBuf) or pinned host (PinBuf) memory
+template <cudaError_t (*Alloc)(void**, size_t), cudaError_t (*Free)(void*)>
+struct Buf {
   void* p = nullptr;
   size_t cap = 0;
   cudaError_t reserve(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
-    if (p) cudaFree(p);
+    if (p) Free(p);
     p = nullptr; cap = 0;
     size_t want = std::max(bytes, (size_t)256);
-    cudaError_t e = cudaMalloc(&p, want);
+    cudaError_t e = Alloc(&p, want);
     if (e == cudaSuccess) cap = want;
     return e;
   }
-  void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+  void release() { if (p) Free(p); p = nullptr; cap = 0; }
 };
-
-struct PinBuf {
-  void* p = nullptr;
-  size_t cap = 0;
-  cudaError_t reserve(size_t bytes) {
-    if (bytes <= cap) return cudaSuccess;
-    if (p) cudaFreeHost(p);
-    p = nullptr; cap = 0;
-    size_t want = std::max(bytes, (size_t)256);
-    cudaError_t e = cudaMallocHost(&p, want);
-    if (e == cudaSuccess) cap = want;
-    return e;
-  }
-  void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
-};
+using DevBuf = Buf<cudaMalloc, cudaFree>;
+using PinBuf = Buf<cudaMallocHost, cudaFreeHost>;
 
 // Host description of the option slices (options grouped by maturity, first-appearance order).
 struct BookHost {
@@ -231,6 +220,21 @@ int fail(dhj_ctx* ctx, int code, const char* fmt, ...) {
                   "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e__), __FILE__, __LINE__);     \
   } while (0)
 
+// after every kernel launch: the launch's own error, and the count of dhj_launch_count
+#define DHJ_LAUNCHED(ctx)                    \
+  do {                                       \
+    DHJ_CUDA((ctx), cudaGetLastError());     \
+    (ctx)->launches++;                       \
+  } while (0)
+
+// a 1-D grid of `blocks` blocks, clamped to what one launch takes
+int grid_1d(long long blocks) { return (int)std::max<long long>(1, std::min(blocks, 2147483647LL)); }
+
+// the grid of the grid-stride elementwise kernels (implied vol, Black-Scholes price, IV residual) over n elements
+int grid_stride_blocks(const dhj_ctx* ctx, long long n) {
+  return (int)std::max<long long>(1, std::min<long long>((n + 255) / 256, 32LL * ctx->sm_count));
+}
+
 // staging copies between the caller's pageable memory and the pinned slots: a single thread moves ~10 GB/s, less
 // than the kernel consumes per chunk, so large copies are split over eight host threads (four: 14.75 ms per
 // 1 Mi-set grid from pageable memory, eight: 14.28)
@@ -286,7 +290,6 @@ int launch_price(dhj_ctx* ctx, const SliceView& v, PriceArgs a, int max_slice, c
     const long long batches = (items + a.items_per_batch - 1) / a.items_per_batch;
     // one block per batch: the hardware block scheduler balances the SMs dynamically (a persistent grid with a
     // static batch -> block map measured ~3 % slower: the slowest SM sets the time)
-    const long long cap = 2147483647LL;
     // DHJ_DEBUG_EXTRA_SMEM (bytes): developer knob that pads the launch with unused dynamic shared memory to
     // lower the resident block count (occupancy experiments, profiles/README.md); never set in production
     static const size_t extra = [] {
@@ -295,7 +298,7 @@ int launch_price(dhj_ctx* ctx, const SliceView& v, PriceArgs a, int max_slice, c
       if (b) cudaFuncSetAttribute(k_price_batch<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b);
       return b;
     }();
-    const int grid = (int)std::max<long long>(1, std::min(batches, cap));
+    const int grid = grid_1d(batches);
     if (a.items_per_batch == kPriceItems) k_price_batch<true><<<grid, kBatchThreads, extra, st>>>(v, a);
     else k_price_batch<false><<<grid, kBatchThreads, 0, st>>>(v, a);
   } else {
@@ -305,11 +308,9 @@ int launch_price(dhj_ctx* ctx, const SliceView& v, PriceArgs a, int max_slice, c
                                                          (int)sizeof(DenseSmem));
     DHJ_CUDA(ctx, attr);
     const long long blocks = (items + kDenseWarps - 1) / kDenseWarps;
-    k_price_dense<<<(int)std::max<long long>(1, std::min(blocks, 2147483647LL)), 32 * kDenseWarps, sizeof(DenseSmem),
-                    st>>>(v, a);
+    k_price_dense<<<grid_1d(blocks), 32 * kDenseWarps, sizeof(DenseSmem), st>>>(v, a);
   }
-  DHJ_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
+  DHJ_LAUNCHED(ctx);
   return DHJ_OK;
 }
 
@@ -367,12 +368,59 @@ int book_used(dhj_ctx* ctx, cudaStream_t stream) {
   return DHJ_OK;
 }
 
-int check_common(dhj_ctx* ctx, const void* params, int64_t P, const void* S0, int32_t N, double L, const void* out) {
+int check_arrays(dhj_ctx* ctx, const void* in, int64_t P, const void* S0, const void* out) {
   if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
-  if (!params || !S0 || !out) return fail(ctx, DHJ_ERR_ARG, "null array argument");
+  if (!in || !S0 || !out) return fail(ctx, DHJ_ERR_ARG, "null array argument");
   if (P < 0) return fail(ctx, DHJ_ERR_ARG, "P must be >= 0 (got %lld)", (long long)P);
+  return DHJ_OK;
+}
+
+int check_common(dhj_ctx* ctx, const void* params, int64_t P, const void* S0, int32_t N, double L, const void* out) {
+  int rc = check_arrays(ctx, params, P, S0, out);
+  if (rc) return rc;
   if (N < 1) return fail(ctx, DHJ_ERR_ARG, "N must be >= 1 (got %d)", N);
   if (!(L == L)) return fail(ctx, DHJ_ERR_ARG, "L is NaN");
+  return DHJ_OK;
+}
+
+// The option tables and strides of an option list (dhj_price_list's layout).  *empty: M == 0 or P == 0, nothing to
+// compute; the tables are not looked at then.
+int check_list(dhj_ctx* ctx, int64_t P, int64_t s0_stride, const double* strike, int64_t strike_stride,
+               const double* maturity, const int32_t* is_call, int32_t M, bool* empty) {
+  if (M < 0) return fail(ctx, DHJ_ERR_ARG, "M must be >= 0");
+  *empty = M == 0 || P == 0;
+  if (*empty) return DHJ_OK;
+  if (!strike || !maturity || !is_call) return fail(ctx, DHJ_ERR_ARG, "null option table");
+  if (s0_stride != 0 && s0_stride != 1) return fail(ctx, DHJ_ERR_ARG, "s0_stride must be 0 or 1");
+  if (strike_stride != 0 && strike_stride != M) return fail(ctx, DHJ_ERR_ARG, "strike_stride must be 0 or M");
+  return DHJ_OK;
+}
+
+// An option list priced by dhj_price_list, dhj_price_jacobian and dhj_price_greeks: the maturity book (and a shared
+// strike row) in the book ring and the view over it.  A per-set strike row (strike_stride = M) is the caller's to
+// point the view at.
+struct OptionList {
+  bool empty = true;
+  SliceView v{};
+  int max_slice = 0;
+};
+
+// out_der: the call's second output (dhj_price_list, which has none, passes out again)
+int option_list(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride, double r,
+                double q, const double* strike, int64_t strike_stride, const double* maturity, const int32_t* is_call,
+                int32_t M, int32_t N, double L, const void* out, const void* out_der, OptionList* ol) {
+  int rc = check_common(ctx, params, P, S0, N, L, out);
+  if (rc) return rc;
+  if (!out_der) return fail(ctx, DHJ_ERR_ARG, "null array argument");
+  rc = check_list(ctx, P, s0_stride, strike, strike_stride, maturity, is_call, M, &ol->empty);
+  if (rc || ol->empty) return rc;
+  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
+  BookHost book;
+  book.group(maturity, is_call, M);
+  rc = upload_book(ctx, book, strike_stride ? nullptr : strike, strike_stride ? 0 : M, ctx->stream, &ol->v);
+  if (rc) return rc;
+  ol->v.scale_by_spot = 0; ol->v.n_cos = N; ol->v.r = r; ol->v.q = q; ol->v.L = L;
+  ol->max_slice = book.max_slice;
   return DHJ_OK;
 }
 
@@ -499,6 +547,116 @@ int stage_x(dhj_ctx* ctx, const dhj_market* mk, const double* x, const int32_t* 
   return DHJ_OK;
 }
 
+// The B x staged by stage_x, transformed by k_fd_expand (fd: into the kFdPoints stencil points of each) into d_xv /
+// d_idx, and the arguments of the market's pricing launch over those points (out is the caller's to set).
+int expand_x(dhj_ctx* ctx, const dhj_market* mk, const int* d_index, int64_t B, int fd, double h, PriceArgs* pa) {
+  const int64_t n = B * (fd ? kFdPoints : 1);
+  DHJ_CUDA(ctx, ctx->d_xv.reserve((size_t)n * kNumParams * sizeof(double)));
+  DHJ_CUDA(ctx, ctx->d_idx.reserve((size_t)n * sizeof(int)));
+  k_fd_expand<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>((const double*)ctx->d_x.p, d_index, B, fd, h,
+                                                                   (double*)ctx->d_xv.p, (int*)ctx->d_idx.p);
+  DHJ_LAUNCHED(ctx);
+  pa->params = (const double*)ctx->d_xv.p; pa->S0 = (const double*)mk->d_S0.p; pa->s0_stride = 1;
+  pa->row_index = (const int*)ctx->d_idx.p; pa->P = n; pa->transform = 0; pa->out = nullptr;
+  return DHJ_OK;
+}
+
+// (f, g) of B evaluations from d_fg (kFdPoints doubles each: f, then g) into out_f[B] and out_g[B][13]; out_f_all
+// (may be null) receives the kFdPoints losses per evaluation in d_f
+int download_fg(dhj_ctx* ctx, int64_t B, double* out_f, double* out_g, double* out_f_all) {
+  const size_t bytes = (size_t)B * kFdPoints * sizeof(double);
+  DHJ_CUDA(ctx, ctx->h_res.reserve(bytes * (out_f_all ? 2 : 1)));
+  DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, ctx->d_fg.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (out_f_all)
+    DHJ_CUDA(ctx, cudaMemcpyAsync((unsigned char*)ctx->h_res.p + bytes, ctx->d_f.p, bytes, cudaMemcpyDeviceToHost,
+                                  ctx->stream));
+  DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  const double* res = (const double*)ctx->h_res.p;
+  if (out_f_all) host_copy(out_f_all, res + B * kFdPoints, bytes);
+#pragma omp parallel for schedule(static) num_threads(copy_threads()) if (B >= 4096)
+  for (int64_t c = 0; c < B; ++c) {
+    out_f[c] = res[c * kFdPoints];
+    memcpy(out_g + c * kNumParams, res + c * kFdPoints + 1, kNumParams * sizeof(double));
+  }
+  return DHJ_OK;
+}
+
+// One host array of a synchronous staged call (stage_sync): an input (`in`) or an output (`out`) of `row` bytes per
+// row, or an input of `fixed` bytes that every chunk shares (a shared table, a scalar S0).  A segment without a host
+// array is not staged and its device pointer is null, but its row still counts towards the chunk size.
+struct Seg {
+  const void* in;
+  void* out;
+  size_t row, fixed;
+};
+Seg rows_in(const void* p, size_t row) { return {p, nullptr, row, 0}; }
+Seg rows_out(void* p, size_t row) { return {nullptr, p, row, 0}; }
+Seg table_in(const void* p, size_t bytes) { return {p, nullptr, 0, bytes}; }
+Seg s0_in(const double* S0, int64_t s0_stride) {
+  return s0_stride ? rows_in(S0, sizeof(double)) : table_in(S0, sizeof(double));
+}
+// a strike row per row (strike_stride = M); a shared strike row travels in the book ring instead
+Seg strike_in(const double* strike, int64_t strike_stride) {
+  return rows_in(strike_stride ? strike : nullptr, (size_t)strike_stride * sizeof(double));
+}
+
+constexpr size_t kStageChunkBytes = (size_t)32 << 20;
+constexpr size_t kOneChunk = SIZE_MAX;   // the whole call in one chunk (one launch)
+
+// Host arrays in -> launch(n, d) -> host arrays out, synchronously through the context's staging buffers, for the
+// entry points whose throughput is not a goal.  Rows [0, rows) go in chunks of as many rows as fit in chunk_bytes
+// (at least one); per chunk one upload, the launch callback (d[i]: the device copy of segment i's rows of the chunk)
+// and one download.
+template <size_t N, class Launch>
+int stage_sync(dhj_ctx* ctx, int64_t rows, size_t chunk_bytes, const Seg (&segs)[N], Launch launch) {
+  size_t row = 0;
+  for (const Seg& s : segs) row += s.row;
+  const int64_t chunk =
+      (int64_t)std::max<size_t>(1, std::min<size_t>((size_t)rows, chunk_bytes / std::max<size_t>(row, 1)));
+  // a chunk of n rows: the inputs packed in h_x / d_x, the outputs in d_prices / h_res, 8-byte aligned
+  size_t off[N], bytes[N], in_bytes = 0, out_bytes = 0;
+  auto layout = [&](int64_t n) {
+    in_bytes = out_bytes = 0;
+    for (size_t i = 0; i < N; ++i) {
+      size_t& end = segs[i].out ? out_bytes : in_bytes;
+      off[i] = end;
+      bytes[i] = (segs[i].in || segs[i].out) ? (segs[i].row ? (size_t)n * segs[i].row : segs[i].fixed) : 0;
+      end += BookHost::align8(bytes[i]);
+    }
+  };
+  layout(chunk);
+  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
+  DHJ_CUDA(ctx, ctx->h_x.reserve(in_bytes));
+  DHJ_CUDA(ctx, ctx->d_x.reserve(in_bytes));
+  DHJ_CUDA(ctx, ctx->d_prices.reserve(out_bytes));
+  DHJ_CUDA(ctx, ctx->h_res.reserve(out_bytes));
+  unsigned char* hin = (unsigned char*)ctx->h_x.p;
+  const unsigned char* hout = (const unsigned char*)ctx->h_res.p;
+  for (int64_t lo = 0; lo < rows; lo += chunk) {
+    const int64_t n = std::min(chunk, rows - lo);
+    layout(n);
+    void* d[N];
+    for (size_t i = 0; i < N; ++i) {
+      const Seg& s = segs[i];
+      d[i] = nullptr;
+      if (s.in) {
+        host_copy(hin + off[i], (const unsigned char*)s.in + (size_t)lo * s.row, bytes[i]);
+        d[i] = (unsigned char*)ctx->d_x.p + off[i];
+      } else if (s.out) {
+        d[i] = (unsigned char*)ctx->d_prices.p + off[i];
+      }
+    }
+    DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->d_x.p, hin, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    int rc = launch(n, (void* const*)d);
+    if (rc) return rc;
+    DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, ctx->d_prices.p, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    for (size_t i = 0; i < N; ++i)
+      if (segs[i].out) host_copy((unsigned char*)segs[i].out + (size_t)lo * segs[i].row, hout + off[i], bytes[i]);
+  }
+  return DHJ_OK;
+}
+
 }  // namespace
 
 // ================================================================================================
@@ -599,21 +757,11 @@ int dhj_launch_count(const dhj_ctx* ctx, int64_t* count) {
 int dhj_price_list(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride,
                    double r, double q, const double* strike, int64_t strike_stride, const double* maturity,
                    const int32_t* is_call, int32_t M, int32_t N, double L, double* out) {
-  int rc = check_common(ctx, params, P, S0, N, L, out);
-  if (rc) return rc;
-  if (M < 0) return fail(ctx, DHJ_ERR_ARG, "M must be >= 0");
-  if (M == 0 || P == 0) return DHJ_OK;
-  if (!strike || !maturity || !is_call) return fail(ctx, DHJ_ERR_ARG, "null option table");
-  if (s0_stride != 0 && s0_stride != 1) return fail(ctx, DHJ_ERR_ARG, "s0_stride must be 0 or 1");
-  if (strike_stride != 0 && strike_stride != M) return fail(ctx, DHJ_ERR_ARG, "strike_stride must be 0 or M");
-  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
-  BookHost book;
-  book.group(maturity, is_call, M);
-  SliceView v;
-  rc = upload_book(ctx, book, strike_stride ? nullptr : strike, strike_stride ? 0 : M, ctx->stream, &v);
-  if (rc) return rc;
-  v.scale_by_spot = 0; v.n_cos = N; v.r = r; v.q = q; v.L = L;
-  return run_price_host(ctx, v, book.max_slice, params, P, S0, s0_stride, strike, strike_stride, out);
+  OptionList ol;
+  int rc = option_list(ctx, params, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, N, L, out,
+                       out, &ol);
+  if (rc || ol.empty) return rc;
+  return run_price_host(ctx, ol.v, ol.max_slice, params, P, S0, s0_stride, strike, strike_stride, out);
 }
 
 static int grid_view(dhj_ctx* ctx, const double* strikes, int32_t nK, const double* maturities, int32_t nT,
@@ -738,15 +886,10 @@ static int run_loss(dhj_ctx* ctx, const dhj_market* mk, const double* x, const i
   if (rc) return rc;
   if (!out_f || (fd && !out_g)) return fail(ctx, DHJ_ERR_ARG, "null output");
   if (B == 0) return DHJ_OK;
-  const int per = fd ? kFdPoints : 1;
-  const int64_t n_units = B * per;
+  const int64_t n_units = B * (fd ? kFdPoints : 1);
   if (n_units > 2000000000LL) return fail(ctx, DHJ_ERR_ARG, "batch too large for one launch");
   DHJ_CUDA(ctx, ctx->d_f.reserve((size_t)n_units * sizeof(double)));
-  size_t res_bytes = (size_t)B * sizeof(double);
-  if (fd) {
-    res_bytes = (size_t)n_units * sizeof(double);
-    DHJ_CUDA(ctx, ctx->d_fg.reserve(res_bytes));
-  }
+  if (fd) DHJ_CUDA(ctx, ctx->d_fg.reserve((size_t)n_units * sizeof(double)));
   const SliceView& v = mk->view;
   // Large batches go through the pricing kernel (expand -> k_price_batch -> reduce): its batches of 32 items keep the
   // four warps balanced whatever the number of slices per loss evaluation, which pays for two extra small launches
@@ -776,22 +919,15 @@ static int run_loss(dhj_ctx* ctx, const dhj_market* mk, const double* x, const i
     a.units_per_batch = pick_units_per_batch(n_units, v.n_slices, kPriceItems,
                                              (long long)ctx->sm_count * ctx->loss_blocks_per_sm);
     const long long batches = (n_units + a.units_per_batch - 1) / a.units_per_batch;
-    k_loss_batch<<<(int)std::max<long long>(1, std::min(batches, 2147483647LL)), kBatchThreads, 0, ctx->stream>>>(v, a);
-    DHJ_CUDA(ctx, cudaGetLastError());
-    ctx->launches++;
+    k_loss_batch<<<grid_1d(batches), kBatchThreads, 0, ctx->stream>>>(v, a);
+    DHJ_LAUNCHED(ctx);
   } else {
     // general path: stencil points -> pricing kernel (batch or dense by slice size) -> reduction
-    DHJ_CUDA(ctx, ctx->d_xv.reserve((size_t)n_units * kNumParams * sizeof(double)));
-    DHJ_CUDA(ctx, ctx->d_idx.reserve((size_t)n_units * sizeof(int)));
     DHJ_CUDA(ctx, ctx->d_prices.reserve((size_t)n_units * mk->M * sizeof(double)));
-    const unsigned gb = (unsigned)((n_units + 127) / 128);
-    k_fd_expand<<<gb, 128, 0, ctx->stream>>>((const double*)ctx->d_x.p, d_index, B, fd, h, (double*)ctx->d_xv.p,
-                                             (int*)ctx->d_idx.p);
-    DHJ_CUDA(ctx, cudaGetLastError());
     PriceArgs pa;
-    pa.params = (const double*)ctx->d_xv.p; pa.S0 = (const double*)mk->d_S0.p; pa.s0_stride = 1;
-    pa.row_index = (const int*)ctx->d_idx.p; pa.P = n_units; pa.transform = 0; pa.out = (double*)ctx->d_prices.p;
-    ctx->launches++;
+    rc = expand_x(ctx, mk, d_index, B, fd, h, &pa);
+    if (rc) return rc;
+    pa.out = (double*)ctx->d_prices.p;
     rc = launch_price(ctx, v, pa, mk->book.max_slice, ctx->stream);
     if (rc) return rc;
     if (iv_objective) {
@@ -810,28 +946,14 @@ static int run_loss(dhj_ctx* ctx, const dhj_market* mk, const double* x, const i
           (const double*)mk->d_price.p, v.pos, mk->M, B, fd, h, (const double*)ctx->d_x.p, (double*)ctx->d_f.p,
           fd ? (double*)ctx->d_fg.p : nullptr);
     }
-    DHJ_CUDA(ctx, cudaGetLastError());
-    ctx->launches++;
+    DHJ_LAUNCHED(ctx);
   }
-  const bool want_all = fd && out_f_all;
-  DHJ_CUDA(ctx, ctx->h_res.reserve(res_bytes * (want_all ? 2 : 1)));
-  DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, fd ? ctx->d_fg.p : ctx->d_f.p, res_bytes, cudaMemcpyDeviceToHost,
-                                ctx->stream));
-  if (want_all)
-    DHJ_CUDA(ctx, cudaMemcpyAsync((unsigned char*)ctx->h_res.p + res_bytes, ctx->d_f.p, res_bytes,
-                                  cudaMemcpyDeviceToHost, ctx->stream));
+  if (fd) return download_fg(ctx, B, out_f, out_g, out_f_all);
+  const size_t res_bytes = (size_t)B * sizeof(double);
+  DHJ_CUDA(ctx, ctx->h_res.reserve(res_bytes));
+  DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, ctx->d_f.p, res_bytes, cudaMemcpyDeviceToHost, ctx->stream));
   DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  const double* res = (const double*)ctx->h_res.p;
-  if (want_all) host_copy(out_f_all, (const unsigned char*)ctx->h_res.p + res_bytes, res_bytes);
-  if (!fd) {
-    host_copy(out_f, res, res_bytes);
-  } else {
-#pragma omp parallel for schedule(static) num_threads(copy_threads()) if (B >= 4096)
-    for (int64_t c = 0; c < B; ++c) {
-      out_f[c] = res[c * kFdPoints];
-      memcpy(out_g + c * kNumParams, res + c * kFdPoints + 1, kNumParams * sizeof(double));
-    }
-  }
+  host_copy(out_f, ctx->h_res.p, res_bytes);
   return DHJ_OK;
 }
 
@@ -848,16 +970,23 @@ int dhj_loss_fd(dhj_ctx* ctx, const dhj_market* market, const double* x, const i
   return run_loss(ctx, market, x, market_index, C, 1, h, out_f, out_g, out_f_all);
 }
 
-// The whole lock-step loop of many simultaneous calibrations in one call: ask -> one loss / forward-difference
-// launch over every state that waits for an evaluation -> tell, until every optimiser has stopped.  (The Python
-// host used to drive the three steps itself; with several pipelines per GPU their interpreter work serialised on
-// the GIL — in here a pipeline never touches it.)
-int dhj_lbfgs_minimize_fd(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market, const int32_t* state_market,
-                          int64_t n_states, double h, int64_t* rounds, int64_t* state_rounds, double* seconds) {
+// The whole lock-step loop of many simultaneous calibrations in one call: ask -> evaluate(x, market index, na, f, g)
+// over every state that waits for an evaluation -> tell, until every optimiser has stopped.  (The Python host used
+// to drive the three steps itself; with several pipelines per GPU their interpreter work serialised on the GIL — in
+// here a pipeline never touches it.)
+extern "C++" {
+template <class Evaluate>
+static int run_lockstep(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market, const int32_t* state_market,
+                        int64_t n_states, int64_t* rounds, int64_t* state_rounds, double* seconds, Evaluate evaluate) {
   if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
   if (!opt || !market) return fail(ctx, DHJ_ERR_ARG, "null optimiser or market");
-  if (n_states < 0) return fail(ctx, DHJ_ERR_ARG, "n_states must be >= 0");
-  if (!(h > 0.0)) return fail(ctx, DHJ_ERR_ARG, "h must be > 0");
+  int64_t n_opt = 0;
+  int32_t dim = 0;
+  dhj_lbfgs_shape(opt, &n_opt, &dim);
+  // an ask writes up to every state of the optimiser into the buffers below, and state_market is read at its indices
+  if (n_states != n_opt) return fail(ctx, DHJ_ERR_ARG, "n_states (%lld) != the optimiser's state count (%lld)",
+                                     (long long)n_states, (long long)n_opt);
+  if (dim != kNumParams) return fail(ctx, DHJ_ERR_ARG, "the optimiser's dimension is %d, not %d", dim, kNumParams);
   std::vector<int64_t> idx((size_t)n_states);
   std::vector<int32_t> mi((size_t)n_states);
   std::vector<double> x((size_t)n_states * kNumParams), f((size_t)n_states), g((size_t)n_states * kNumParams);
@@ -868,13 +997,12 @@ int dhj_lbfgs_minimize_fd(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market
     int64_t na = 0;
     int rc = dhj_lbfgs_ask(opt, &na, idx.data(), x.data());
     if (rc) return fail(ctx, rc, "dhj_lbfgs_ask failed (%d)", rc);
-    if (na > n_states) return fail(ctx, DHJ_ERR_ARG, "the optimiser holds more states (%lld) than n_states", (long long)na);
     const double t1 = omp_get_wtime();
     t_ask += t1 - t0;
     if (na == 0) break;
     if (state_market)
       for (int64_t a = 0; a < na; ++a) mi[a] = state_market[idx[a]];
-    rc = run_loss(ctx, market, x.data(), state_market ? mi.data() : nullptr, na, 1, h, f.data(), g.data(), nullptr);
+    rc = evaluate(x.data(), state_market ? mi.data() : nullptr, na, f.data(), g.data());
     if (rc) return rc;
     const double t2 = omp_get_wtime();
     rc = dhj_lbfgs_tell(opt, na, f.data(), g.data());
@@ -889,108 +1017,74 @@ int dhj_lbfgs_minimize_fd(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market
   if (seconds) { seconds[0] = t_ask; seconds[1] = t_loss; seconds[2] = t_tell; }
   return DHJ_OK;
 }
+}  // extern "C++"
+
+int dhj_lbfgs_minimize_fd(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market, const int32_t* state_market,
+                          int64_t n_states, double h, int64_t* rounds, int64_t* state_rounds, double* seconds) {
+  if (ctx && !(h > 0.0)) return fail(ctx, DHJ_ERR_ARG, "h must be > 0");
+  return run_lockstep(opt, ctx, market, state_market, n_states, rounds, state_rounds, seconds,
+                      [&](const double* x, const int32_t* mi, int64_t na, double* f, double* g) {
+                        return run_loss(ctx, market, x, mi, na, 1, h, f, g, nullptr);
+                      });
+}
 
 // ---- analytic parameter gradient (dhj_jac.cuh) -------------------------------------------------------
 static int launch_jac(dhj_ctx* ctx, const SliceView& v, const JacArgs& a, cudaStream_t st) {
   const long long blocks = (a.P * (long long)v.n_slices + kJacWarps - 1) / kJacWarps;
-  k_price_jac<<<(int)std::max<long long>(1, std::min(blocks, 2147483647LL)), 32 * kJacWarps, 0, st>>>(v, a);
-  DHJ_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
+  k_price_jac<<<grid_1d(blocks), 32 * kJacWarps, 0, st>>>(v, a);
+  DHJ_LAUNCHED(ctx);
   return DHJ_OK;
 }
 
-// Prices and n_der derivatives per option of an option list (dhj_price_jacobian, dhj_price_greeks): the argument
-// checks, the maturity book and synchronous chunks of ~32 MB through the staging buffers (throughput of these entry
-// points is not a goal).  launch(view, d_params, d_S0, s0_stride, n, d_price, d_der) enqueues the kernel for n sets.
-extern "C++" {
-template <class Launch>
-static int run_option_list(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride,
-                           double r, double q, const double* strike, int64_t strike_stride, const double* maturity,
-                           const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price, double* out_der,
-                           int n_der, Launch launch) {
-  int rc = check_common(ctx, params, P, S0, N, L, out_price);
-  if (rc) return rc;
-  if (!out_der) return fail(ctx, DHJ_ERR_ARG, "null array argument");
-  if (M < 0) return fail(ctx, DHJ_ERR_ARG, "M must be >= 0");
-  if (M == 0 || P == 0) return DHJ_OK;
-  if (!strike || !maturity || !is_call) return fail(ctx, DHJ_ERR_ARG, "null option table");
-  if (s0_stride != 0 && s0_stride != 1) return fail(ctx, DHJ_ERR_ARG, "s0_stride must be 0 or 1");
-  if (strike_stride != 0 && strike_stride != M) return fail(ctx, DHJ_ERR_ARG, "strike_stride must be 0 or M");
-  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
-  BookHost book;
-  book.group(maturity, is_call, M);
-  SliceView v;
-  rc = upload_book(ctx, book, strike_stride ? nullptr : strike, strike_stride ? 0 : M, ctx->stream, &v);
-  if (rc) return rc;
-  v.scale_by_spot = 0; v.n_cos = N; v.r = r; v.q = q; v.L = L;
-  const size_t row_in = kNumParams + (s0_stride ? 1 : 0) + (strike_stride ? (size_t)M : 0);
-  const size_t row_out = (size_t)M * (1 + n_der);
-  const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(P, (int64_t)(((size_t)1 << 22) / (row_in + row_out))));
-  const size_t in_bytes = (size_t)chunk * row_in * sizeof(double) + sizeof(double);
-  const size_t out_bytes = (size_t)chunk * row_out * sizeof(double);
-  DHJ_CUDA(ctx, ctx->h_x.reserve(in_bytes));
-  DHJ_CUDA(ctx, ctx->d_x.reserve(in_bytes));
-  DHJ_CUDA(ctx, ctx->d_jac.reserve(out_bytes));
-  DHJ_CUDA(ctx, ctx->h_res.reserve(out_bytes));
-  for (int64_t lo = 0; lo < P; lo += chunk) {
-    const int64_t n = std::min(chunk, P - lo);
-    const size_t pb = (size_t)n * kNumParams * sizeof(double);
-    const size_t s0b = s0_stride ? (size_t)n * sizeof(double) : sizeof(double);
-    const size_t kb = strike_stride ? (size_t)n * M * sizeof(double) : 0;
-    unsigned char* hin = (unsigned char*)ctx->h_x.p;
-    unsigned char* din = (unsigned char*)ctx->d_x.p;
-    host_copy(hin, params + lo * kNumParams, pb);
-    host_copy(hin + pb, s0_stride ? S0 + lo : S0, s0b);
-    if (kb) host_copy(hin + pb + s0b, strike + lo * (int64_t)M, kb);
-    DHJ_CUDA(ctx, cudaMemcpyAsync(din, hin, pb + s0b + kb, cudaMemcpyHostToDevice, ctx->stream));
-    SliceView vv = v;
-    if (strike_stride) { vv.strike = (const double*)(din + pb + s0b); vv.strike_stride = M; }
-    double* d_out = (double*)ctx->d_jac.p;
-    rc = launch(vv, (const double*)din, (const double*)(din + pb), s0_stride ? 1 : 0, n, d_out, d_out + n * (int64_t)M);
-    if (rc) return rc;
-    const size_t ob = (size_t)n * row_out * sizeof(double);
-    DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, d_out, ob, cudaMemcpyDeviceToHost, ctx->stream));
-    DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    const double* res = (const double*)ctx->h_res.p;
-    host_copy(out_price + lo * (int64_t)M, res, (size_t)n * M * sizeof(double));
-    host_copy(out_der + lo * (int64_t)M * n_der, res + n * (int64_t)M, (size_t)n * M * n_der * sizeof(double));
-  }
-  return book_used(ctx, ctx->stream);
-}
-}  // extern "C++"
-
+// Prices and derivatives of an option list (dhj_price_jacobian, dhj_price_greeks) come in synchronous chunks through
+// the staging buffers, rows = parameter sets: params | S0 | per-set strikes in, prices | derivatives out.  d[2] is
+// null for a shared strike row (in the book).
 int dhj_price_jacobian(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride, double r,
                        double q, const double* strike, int64_t strike_stride, const double* maturity,
                        const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price, double* out_jac) {
-  return run_option_list(ctx, params, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, N, L,
-                         out_price, out_jac, kNumParams,
-                         [&](const SliceView& vv, const double* d_params, const double* d_S0, long long s0s, int64_t n,
-                             double* d_price, double* d_der) {
-                           JacArgs a;
-                           a.params = d_params; a.S0 = d_S0; a.s0_stride = s0s;
-                           a.row_index = nullptr; a.P = n; a.out_price = d_price; a.out_jac = d_der;
-                           return launch_jac(ctx, vv, a, ctx->stream);
-                         });
+  OptionList ol;
+  int rc = option_list(ctx, params, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, N, L,
+                       out_price, out_jac, &ol);
+  if (rc || ol.empty) return rc;
+  const size_t row = (size_t)M * sizeof(double);
+  rc = stage_sync(ctx, P, kStageChunkBytes,
+                  {rows_in(params, kNumParams * sizeof(double)), s0_in(S0, s0_stride), strike_in(strike, strike_stride),
+                   rows_out(out_price, row), rows_out(out_jac, row * kNumParams)},
+                  [&](int64_t n, void* const* d) {
+                    SliceView v = ol.v;
+                    if (d[2]) { v.strike = (const double*)d[2]; v.strike_stride = M; }
+                    JacArgs a;
+                    a.params = (const double*)d[0]; a.S0 = (const double*)d[1]; a.s0_stride = s0_stride ? 1 : 0;
+                    a.row_index = nullptr; a.P = n; a.out_price = (double*)d[3]; a.out_jac = (double*)d[4];
+                    return launch_jac(ctx, v, a, ctx->stream);
+                  });
+  return rc ? rc : book_used(ctx, ctx->stream);
 }
 
 // ---- Greeks (dhj_greeks.cuh) --------------------------------------------------------------------------
 int dhj_price_greeks(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride, double r,
                      double q, const double* strike, int64_t strike_stride, const double* maturity,
                      const int32_t* is_call, int32_t M, int32_t N, double L, double* out_price, double* out_greeks) {
-  return run_option_list(ctx, params, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, N, L,
-                         out_price, out_greeks, kGreeks,
-                         [&](const SliceView& vv, const double* d_params, const double* d_S0, long long s0s, int64_t n,
-                             double* d_price, double* d_der) {
-                           GreeksArgs a;
-                           a.params = d_params; a.S0 = d_S0; a.s0_stride = s0s;
-                           a.row_index = nullptr; a.P = n; a.out_price = d_price; a.out_greeks = d_der;
-                           const long long blocks = (n * (long long)vv.n_slices + kJacWarps - 1) / kJacWarps;
-                           k_price_greeks<<<(int)std::max<long long>(1, std::min(blocks, 2147483647LL)),
-                                            32 * kJacWarps, 0, ctx->stream>>>(vv, a);
-                           DHJ_CUDA(ctx, cudaGetLastError());
-                           ctx->launches++;
-                           return DHJ_OK;
-                         });
+  OptionList ol;
+  int rc = option_list(ctx, params, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, N, L,
+                       out_price, out_greeks, &ol);
+  if (rc || ol.empty) return rc;
+  const size_t row = (size_t)M * sizeof(double);
+  rc = stage_sync(ctx, P, kStageChunkBytes,
+                  {rows_in(params, kNumParams * sizeof(double)), s0_in(S0, s0_stride), strike_in(strike, strike_stride),
+                   rows_out(out_price, row), rows_out(out_greeks, row * kGreeks)},
+                  [&](int64_t n, void* const* d) {
+                    SliceView v = ol.v;
+                    if (d[2]) { v.strike = (const double*)d[2]; v.strike_stride = M; }
+                    GreeksArgs a;
+                    a.params = (const double*)d[0]; a.S0 = (const double*)d[1]; a.s0_stride = s0_stride ? 1 : 0;
+                    a.row_index = nullptr; a.P = n; a.out_price = (double*)d[3]; a.out_greeks = (double*)d[4];
+                    const long long blocks = (n * (long long)v.n_slices + kJacWarps - 1) / kJacWarps;
+                    k_price_greeks<<<grid_1d(blocks), 32 * kJacWarps, 0, ctx->stream>>>(v, a);
+                    DHJ_LAUNCHED(ctx);
+                    return DHJ_OK;
+                  });
+  return rc ? rc : book_used(ctx, ctx->stream);
 }
 
 // ---- implied volatility (dhj_iv.cuh) ----------------------------------------------------------------
@@ -1017,75 +1111,48 @@ int upload_iv_tables(dhj_ctx* ctx, const double* strike, bool shared_strike, con
 
 // one elementwise launch over a.P x a.M options (grid-stride)
 int launch_iv(dhj_ctx* ctx, const iv::IvArgs& a, bool inverse, cudaStream_t st) {
-  const long long n = a.P * (long long)a.M;
-  const long long blocks = std::max<long long>(1, std::min<long long>((n + 255) / 256, 32LL * ctx->sm_count));
-  if (inverse) iv::k_implied_vol<<<(int)blocks, 256, 0, st>>>(a);
-  else iv::k_bs_price<<<(int)blocks, 256, 0, st>>>(a);
-  DHJ_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
+  const int blocks = grid_stride_blocks(ctx, a.P * (long long)a.M);
+  if (inverse) iv::k_implied_vol<<<blocks, 256, 0, st>>>(a);
+  else iv::k_bs_price<<<blocks, 256, 0, st>>>(a);
+  DHJ_LAUNCHED(ctx);
   return DHJ_OK;
 }
 
 int check_iv(dhj_ctx* ctx, const void* in, int64_t P, const void* S0, int64_t s0_stride, const void* out, int32_t M) {
-  if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
-  if (!in || !S0 || !out) return fail(ctx, DHJ_ERR_ARG, "null array argument");
-  if (P < 0) return fail(ctx, DHJ_ERR_ARG, "P must be >= 0 (got %lld)", (long long)P);
+  int rc = check_arrays(ctx, in, P, S0, out);
+  if (rc) return rc;
   if (M < 0) return fail(ctx, DHJ_ERR_ARG, "M must be >= 0");
   if (s0_stride != 0 && s0_stride != 1) return fail(ctx, DHJ_ERR_ARG, "s0_stride must be 0 or 1");
   return DHJ_OK;
 }
 
-// dhj_implied_vol (inverse) and dhj_bs_price: host arrays, synchronous chunks of ~32 MB through the staging buffers
-// (throughput of these entry points is not a goal)
-int run_iv_host(dhj_ctx* ctx, bool inverse, const double* in, int64_t P, const double* S0, int64_t s0_stride,
-                double r, double q, const double* strike, int64_t strike_stride, const double* maturity,
-                const int32_t* is_call, int32_t M, double* out, int32_t* status) {
+// dhj_implied_vol (inverse) and dhj_bs_price: host arrays in synchronous chunks through the staging buffers, rows =
+// sets: values | S0 | per-set strikes in, results | status out.  The status row counts towards the chunk size
+// whether or not it is asked for (dhj_bs_price has none).
+int run_iv_list(dhj_ctx* ctx, bool inverse, const double* in, int64_t P, const double* S0, int64_t s0_stride, double r,
+                double q, const double* strike, int64_t strike_stride, const double* maturity, const int32_t* is_call,
+                int32_t M, double* out, int32_t* status) {
   int rc = check_iv(ctx, in, P, S0, s0_stride, out, M);
   if (rc) return rc;
-  if (M == 0 || P == 0) return DHJ_OK;
-  if (!strike || !maturity || !is_call) return fail(ctx, DHJ_ERR_ARG, "null option table");
-  if (strike_stride != 0 && strike_stride != M) return fail(ctx, DHJ_ERR_ARG, "strike_stride must be 0 or M");
+  bool empty;
+  rc = check_list(ctx, P, s0_stride, strike, strike_stride, maturity, is_call, M, &empty);
+  if (rc || empty) return rc;
   DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
   iv::IvArgs a{};
   rc = upload_iv_tables(ctx, strike, strike_stride == 0, maturity, is_call, M, ctx->stream, &a);
   if (rc) return rc;
   a.r = r; a.q = q; a.M = M; a.scale_by_spot = 0; a.s0_stride = s0_stride;
-  const size_t row_in = (size_t)M * sizeof(double) + (s0_stride ? sizeof(double) : 0) +
-                        (strike_stride ? (size_t)M * sizeof(double) : 0);
-  const size_t row_out = (size_t)M * (sizeof(double) + sizeof(int32_t));
-  const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(P, (int64_t)(((size_t)1 << 25) / (row_in + row_out))));
-  const size_t in_bytes = (size_t)chunk * row_in + sizeof(double);
-  const size_t out_bytes = (size_t)chunk * row_out;
-  DHJ_CUDA(ctx, ctx->h_x.reserve(in_bytes));
-  DHJ_CUDA(ctx, ctx->d_x.reserve(in_bytes));
-  DHJ_CUDA(ctx, ctx->d_jac.reserve(out_bytes));
-  DHJ_CUDA(ctx, ctx->h_res.reserve(out_bytes));
-  for (int64_t lo = 0; lo < P; lo += chunk) {
-    const int64_t n = std::min(chunk, P - lo);
-    const size_t vb = (size_t)n * M * sizeof(double);
-    const size_t s0b = s0_stride ? (size_t)n * sizeof(double) : sizeof(double);
-    const size_t kb = strike_stride ? vb : 0;
-    unsigned char* hin = (unsigned char*)ctx->h_x.p;
-    unsigned char* din = (unsigned char*)ctx->d_x.p;
-    host_copy(hin, in + lo * (int64_t)M, vb);
-    host_copy(hin + vb, s0_stride ? S0 + lo : S0, s0b);
-    if (kb) host_copy(hin + vb + s0b, strike + lo * (int64_t)M, kb);
-    DHJ_CUDA(ctx, cudaMemcpyAsync(din, hin, vb + s0b + kb, cudaMemcpyHostToDevice, ctx->stream));
-    unsigned char* dout = (unsigned char*)ctx->d_jac.p;
-    a.in = (const double*)din; a.S0 = (const double*)(din + vb); a.P = n;
-    if (kb) { a.strike = (const double*)(din + vb + s0b); a.strike_stride = M; }
-    a.out = (double*)dout;
-    a.status = (inverse && status) ? (int32_t*)(dout + vb) : nullptr;
-    rc = launch_iv(ctx, a, inverse, ctx->stream);
-    if (rc) return rc;
-    const size_t ob = vb + (a.status ? (size_t)n * M * sizeof(int32_t) : 0);
-    DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, dout, ob, cudaMemcpyDeviceToHost, ctx->stream));
-    DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    const unsigned char* res = (const unsigned char*)ctx->h_res.p;
-    host_copy(out + lo * (int64_t)M, res, vb);
-    if (a.status) host_copy(status + lo * (int64_t)M, res + vb, (size_t)n * M * sizeof(int32_t));
-  }
-  return book_used(ctx, ctx->stream);
+  const size_t row = (size_t)M * sizeof(double);
+  rc = stage_sync(ctx, P, kStageChunkBytes,
+                  {rows_in(in, row), s0_in(S0, s0_stride), strike_in(strike, strike_stride), rows_out(out, row),
+                   rows_out(inverse ? status : nullptr, (size_t)M * sizeof(int32_t))},
+                  [&](int64_t n, void* const* d) {
+                    a.in = (const double*)d[0]; a.S0 = (const double*)d[1]; a.P = n;
+                    if (d[2]) { a.strike = (const double*)d[2]; a.strike_stride = M; }
+                    a.out = (double*)d[3]; a.status = (int32_t*)d[4];
+                    return launch_iv(ctx, a, inverse, ctx->stream);
+                  });
+  return rc ? rc : book_used(ctx, ctx->stream);
 }
 
 }  // namespace
@@ -1093,14 +1160,14 @@ int run_iv_host(dhj_ctx* ctx, bool inverse, const double* in, int64_t P, const d
 int dhj_implied_vol(dhj_ctx* ctx, const double* price, int64_t P, const double* S0, int64_t s0_stride, double r,
                     double q, const double* strike, int64_t strike_stride, const double* maturity,
                     const int32_t* is_call, int32_t M, double* out_vol, int32_t* out_status) {
-  return run_iv_host(ctx, true, price, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, out_vol,
+  return run_iv_list(ctx, true, price, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, out_vol,
                      out_status);
 }
 
 int dhj_bs_price(dhj_ctx* ctx, const double* vol, int64_t P, const double* S0, int64_t s0_stride, double r, double q,
                  const double* strike, int64_t strike_stride, const double* maturity, const int32_t* is_call,
                  int32_t M, double* out_price) {
-  return run_iv_host(ctx, false, vol, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, out_price,
+  return run_iv_list(ctx, false, vol, P, S0, s0_stride, r, q, strike, strike_stride, maturity, is_call, M, out_price,
                      nullptr);
 }
 
@@ -1109,8 +1176,9 @@ int dhj_implied_vol_dev(dhj_ctx* ctx, const double* d_price, int64_t P, const do
                         const int32_t* is_call, int32_t M, double* d_out_vol, int32_t* d_out_status, void* stream) {
   int rc = check_iv(ctx, d_price, P, d_S0, s0_stride, d_out_vol, M);
   if (rc) return rc;
-  if (M == 0 || P == 0) return DHJ_OK;
-  if (!strike || !maturity || !is_call) return fail(ctx, DHJ_ERR_ARG, "null option table");
+  bool empty;
+  rc = check_list(ctx, P, s0_stride, strike, 0, maturity, is_call, M, &empty);
+  if (rc || empty) return rc;
   DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = (cudaStream_t)stream;   // NULL = the default stream
   iv::IvArgs a{};
@@ -1139,25 +1207,19 @@ static int run_loss_grad(dhj_ctx* ctx, const dhj_market* mk, const double* x, co
   const int M = mk->M;
   const bool iv_objective = mk->objective == DHJ_OBJECTIVE_IV;
   const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(B, (int64_t)(((size_t)1 << 27) / ((size_t)M * kJacChannels))));
-  DHJ_CUDA(ctx, ctx->d_xv.reserve((size_t)B * kNumParams * sizeof(double)));
-  DHJ_CUDA(ctx, ctx->d_idx.reserve((size_t)B * sizeof(int)));
   DHJ_CUDA(ctx, ctx->d_fg.reserve((size_t)B * kFdPoints * sizeof(double)));
   DHJ_CUDA(ctx, ctx->d_prices.reserve((size_t)2 * chunk * M * sizeof(double)));   // pricing kernel | k_price_jac
   DHJ_CUDA(ctx, ctx->d_jac.reserve((size_t)chunk * M * kNumParams * sizeof(double)));
   if (iv_objective) DHJ_CUDA(ctx, ctx->d_ivres.reserve((size_t)2 * chunk * M * sizeof(double)));   // vol | 1/vega
-  double* pv = (double*)ctx->d_xv.p;
-  int* idx = (int*)ctx->d_idx.p;
+  PriceArgs all;
+  rc = expand_x(ctx, mk, d_index, B, 0, 0.0, &all);
+  if (rc) return rc;
   double* fg = (double*)ctx->d_fg.p;
-  k_fd_expand<<<(unsigned)((B + 127) / 128), 128, 0, ctx->stream>>>((const double*)ctx->d_x.p, d_index, B, 0, 0.0, pv,
-                                                                   idx);
-  DHJ_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
   for (int64_t lo = 0; lo < B; lo += chunk) {
     const int64_t n = std::min(chunk, B - lo);
     double* prices = (double*)ctx->d_prices.p;
-    PriceArgs pa;
-    pa.params = pv + lo * kNumParams; pa.S0 = (const double*)mk->d_S0.p; pa.s0_stride = 1; pa.row_index = idx + lo;
-    pa.P = n; pa.transform = 0; pa.out = prices;
+    PriceArgs pa = all;
+    pa.params += lo * kNumParams; pa.row_index += lo; pa.P = n; pa.out = prices;
     rc = launch_price(ctx, mk->view, pa, mk->book.max_slice, ctx->stream);
     if (rc) return rc;
     JacArgs a;
@@ -1178,20 +1240,9 @@ static int run_loss_grad(dhj_ctx* ctx, const dhj_market* mk, const double* x, co
           prices, a.out_jac, a.params, a.row_index, (const double*)mk->d_price.p, mk->view.pos, M, n,
           fg + lo * kFdPoints);
     }
-    DHJ_CUDA(ctx, cudaGetLastError());
-    ctx->launches++;
+    DHJ_LAUNCHED(ctx);
   }
-  const size_t res_bytes = (size_t)B * kFdPoints * sizeof(double);
-  DHJ_CUDA(ctx, ctx->h_res.reserve(res_bytes));
-  DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, fg, res_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-  DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  const double* res = (const double*)ctx->h_res.p;
-#pragma omp parallel for schedule(static) num_threads(copy_threads()) if (B >= 4096)
-  for (int64_t c = 0; c < B; ++c) {
-    out_f[c] = res[c * kFdPoints];
-    memcpy(out_g + c * kNumParams, res + c * kFdPoints + 1, kNumParams * sizeof(double));
-  }
-  return DHJ_OK;
+  return download_fg(ctx, B, out_f, out_g, nullptr);
 }
 
 int dhj_loss_grad(dhj_ctx* ctx, const dhj_market* market, const double* x, const int32_t* market_index, int64_t C,
@@ -1202,44 +1253,10 @@ int dhj_loss_grad(dhj_ctx* ctx, const dhj_market* market, const double* x, const
 
 int dhj_lbfgs_minimize_grad(dhj_lbfgs* opt, dhj_ctx* ctx, const dhj_market* market, const int32_t* state_market,
                             int64_t n_states, int64_t* rounds, int64_t* state_rounds, double* seconds) {
-  if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
-  if (!opt || !market) return fail(ctx, DHJ_ERR_ARG, "null optimiser or market");
-  int64_t n_opt = 0;
-  int32_t dim = 0;
-  dhj_lbfgs_shape(opt, &n_opt, &dim);
-  // the buffers below receive up to every state of the optimiser per ask
-  if (n_states != n_opt) return fail(ctx, DHJ_ERR_ARG, "n_states (%lld) != the optimiser's state count (%lld)",
-                                     (long long)n_states, (long long)n_opt);
-  if (dim != kNumParams) return fail(ctx, DHJ_ERR_ARG, "the optimiser's dimension is %d, not %d", dim, kNumParams);
-  std::vector<int64_t> idx((size_t)n_states);
-  std::vector<int32_t> mi((size_t)n_states);
-  std::vector<double> x((size_t)n_states * kNumParams), f((size_t)n_states), g((size_t)n_states * kNumParams);
-  int64_t n_rounds = 0, n_state_rounds = 0;
-  double t_ask = 0.0, t_loss = 0.0, t_tell = 0.0;
-  for (;;) {
-    const double t0 = omp_get_wtime();
-    int64_t na = 0;
-    int rc = dhj_lbfgs_ask(opt, &na, idx.data(), x.data());
-    if (rc) return fail(ctx, rc, "dhj_lbfgs_ask failed (%d)", rc);
-    const double t1 = omp_get_wtime();
-    t_ask += t1 - t0;
-    if (na == 0) break;
-    if (state_market)
-      for (int64_t a = 0; a < na; ++a) mi[a] = state_market[idx[a]];
-    rc = run_loss_grad(ctx, market, x.data(), state_market ? mi.data() : nullptr, na, f.data(), g.data());
-    if (rc) return rc;
-    const double t2 = omp_get_wtime();
-    rc = dhj_lbfgs_tell(opt, na, f.data(), g.data());
-    if (rc) return fail(ctx, rc, "dhj_lbfgs_tell failed (%d)", rc);
-    t_loss += t2 - t1;
-    t_tell += omp_get_wtime() - t2;
-    ++n_rounds;
-    n_state_rounds += na;
-  }
-  if (rounds) *rounds = n_rounds;
-  if (state_rounds) *state_rounds = n_state_rounds;
-  if (seconds) { seconds[0] = t_ask; seconds[1] = t_loss; seconds[2] = t_tell; }
-  return DHJ_OK;
+  return run_lockstep(opt, ctx, market, state_market, n_states, rounds, state_rounds, seconds,
+                      [&](const double* x, const int32_t* mi, int64_t na, double* f, double* g) {
+                        return run_loss_grad(ctx, market, x, mi, na, f, g);
+                      });
 }
 
 int dhj_market_prices(dhj_ctx* ctx, const dhj_market* mk, const double* x, const int32_t* market_index,
@@ -1301,11 +1318,8 @@ static int launch_iv_residual(dhj_ctx* ctx, const dhj_market* mk, const double* 
   a.is_call = (const int32_t*)((const unsigned char*)mk->d_ivtab.p + (size_t)mk->M * sizeof(double));
   a.mvol = (const double*)mk->d_mvol.p; a.r = mk->r; a.n_units = n_units; a.M = mk->M; a.n_markets = mk->n_markets;
   a.vol = vol; a.inv_vega = inv_vega; a.status = status;
-  const long long n = n_units * (long long)mk->M;
-  const long long blocks = std::max<long long>(1, std::min<long long>((n + 255) / 256, 32LL * ctx->sm_count));
-  k_iv_residual<<<(int)blocks, 256, 0, ctx->stream>>>(a);
-  DHJ_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
+  k_iv_residual<<<grid_stride_blocks(ctx, n_units * (long long)mk->M), 256, 0, ctx->stream>>>(a);
+  DHJ_LAUNCHED(ctx);
   return DHJ_OK;
 }
 
@@ -1375,18 +1389,13 @@ int dhj_market_implied_vols(dhj_ctx* ctx, const dhj_market* market, const double
   if (rc) return rc;
   const int M = mk->M;
   const size_t nb = (size_t)B * M;
-  DHJ_CUDA(ctx, ctx->d_xv.reserve((size_t)B * kNumParams * sizeof(double)));
-  DHJ_CUDA(ctx, ctx->d_idx.reserve((size_t)B * sizeof(int)));
   DHJ_CUDA(ctx, ctx->d_prices.reserve(nb * sizeof(double)));
   DHJ_CUDA(ctx, ctx->d_ivres.reserve(nb * (sizeof(double) + sizeof(int32_t))));
   DHJ_CUDA(ctx, ctx->h_res.reserve(nb * (sizeof(double) + sizeof(int32_t))));
-  k_fd_expand<<<(unsigned)((B + 127) / 128), 128, 0, ctx->stream>>>((const double*)ctx->d_x.p, d_index, B, 0, 0.0,
-                                                                   (double*)ctx->d_xv.p, (int*)ctx->d_idx.p);
-  DHJ_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
   PriceArgs pa;
-  pa.params = (const double*)ctx->d_xv.p; pa.S0 = (const double*)mk->d_S0.p; pa.s0_stride = 1;
-  pa.row_index = (const int*)ctx->d_idx.p; pa.P = B; pa.transform = 0; pa.out = (double*)ctx->d_prices.p;
+  rc = expand_x(ctx, mk, d_index, B, 0, 0.0, &pa);
+  if (rc) return rc;
+  pa.out = (double*)ctx->d_prices.p;
   rc = launch_price(ctx, mk->view, pa, mk->book.max_slice, ctx->stream);
   if (rc) return rc;
   double* vol = (double*)ctx->d_ivres.p;
@@ -1402,55 +1411,22 @@ int dhj_market_implied_vols(dhj_ctx* ctx, const dhj_market* market, const double
 }
 
 // ---- the remaining public methods of DoubleHeston --------------------------------------------
-// small synchronous helper: host arrays in -> kernel -> host arrays out through the loss staging buffers
-namespace {
-struct Staged {
-  dhj_ctx* ctx;
-  size_t in_bytes = 0, out_bytes = 0;
-  int begin(size_t in_b, size_t out_b) {
-    in_bytes = BookHost::align8(in_b); out_bytes = out_b;
-    DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
-    DHJ_CUDA(ctx, ctx->h_x.reserve(in_bytes));
-    DHJ_CUDA(ctx, ctx->d_x.reserve(in_bytes));
-    DHJ_CUDA(ctx, ctx->d_prices.reserve(out_bytes));
-    DHJ_CUDA(ctx, ctx->h_res.reserve(out_bytes));
-    return DHJ_OK;
-  }
-  unsigned char* hin() { return (unsigned char*)ctx->h_x.p; }
-  unsigned char* din() { return (unsigned char*)ctx->d_x.p; }
-  int upload() {
-    DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->d_x.p, ctx->h_x.p, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    return DHJ_OK;
-  }
-  int download() {
-    DHJ_CUDA(ctx, cudaGetLastError());
-    ctx->launches++;
-    DHJ_CUDA(ctx, cudaMemcpyAsync(ctx->h_res.p, ctx->d_prices.p, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    DHJ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return DHJ_OK;
-  }
-};
-}  // namespace
-
+// one synchronous staged launch each (stage_sync, one chunk)
 int dhj_cf(dhj_ctx* ctx, const double* params, double r, double q, double tau, const double* u, int32_t n,
            double* out_re, double* out_im) {
   if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
   if (!params || !u || !out_re || !out_im || n < 0) return fail(ctx, DHJ_ERR_ARG, "bad arguments");
   if (n == 0) return DHJ_OK;
-  Staged st{ctx};
-  const size_t pb = kNumParams * sizeof(double), ub = (size_t)n * sizeof(double);
-  int rc = st.begin(pb + ub, 2 * ub);
-  if (rc) return rc;
-  memcpy(st.hin(), params, pb);
-  memcpy(st.hin() + pb, u, ub);
-  if ((rc = st.upload())) return rc;
-  double* dout = (double*)ctx->d_prices.p;
-  k_cf<<<(n + 127) / 128, 128, 0, ctx->stream>>>((const double*)st.din(), r, q, tau, (const double*)(st.din() + pb),
-                                                  n, dout, dout + n);
-  if ((rc = st.download())) return rc;
-  memcpy(out_re, ctx->h_res.p, ub);
-  memcpy(out_im, (unsigned char*)ctx->h_res.p + ub, ub);
-  return DHJ_OK;
+  return stage_sync(ctx, n, kOneChunk,
+                    {table_in(params, kNumParams * sizeof(double)), rows_in(u, sizeof(double)),
+                     rows_out(out_re, sizeof(double)), rows_out(out_im, sizeof(double))},
+                    [&](int64_t, void* const* d) {
+                      k_cf<<<(n + 127) / 128, 128, 0, ctx->stream>>>((const double*)d[0], r, q, tau,
+                                                                      (const double*)d[1], n, (double*)d[2],
+                                                                      (double*)d[3]);
+                      DHJ_LAUNCHED(ctx);
+                      return DHJ_OK;
+                    });
 }
 
 int dhj_cf_complex(dhj_ctx* ctx, const double* params, double r, double q, double tau, const double* u_re,
@@ -1458,22 +1434,17 @@ int dhj_cf_complex(dhj_ctx* ctx, const double* params, double r, double q, doubl
   if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
   if (!params || !u_re || !u_im || !out_re || !out_im || n < 0) return fail(ctx, DHJ_ERR_ARG, "bad arguments");
   if (n == 0) return DHJ_OK;
-  Staged st{ctx};
-  const size_t pb = kNumParams * sizeof(double), ub = (size_t)n * sizeof(double);
-  int rc = st.begin(pb + 2 * ub, 2 * ub);
-  if (rc) return rc;
-  memcpy(st.hin(), params, pb);
-  memcpy(st.hin() + pb, u_re, ub);
-  memcpy(st.hin() + pb + ub, u_im, ub);
-  if ((rc = st.upload())) return rc;
-  double* dout = (double*)ctx->d_prices.p;
-  k_cf_complex<<<(n + 127) / 128, 128, 0, ctx->stream>>>((const double*)st.din(), r, q, tau,
-                                                          (const double*)(st.din() + pb),
-                                                          (const double*)(st.din() + pb + ub), n, dout, dout + n);
-  if ((rc = st.download())) return rc;
-  memcpy(out_re, ctx->h_res.p, ub);
-  memcpy(out_im, (unsigned char*)ctx->h_res.p + ub, ub);
-  return DHJ_OK;
+  return stage_sync(ctx, n, kOneChunk,
+                    {table_in(params, kNumParams * sizeof(double)), rows_in(u_re, sizeof(double)),
+                     rows_in(u_im, sizeof(double)), rows_out(out_re, sizeof(double)),
+                     rows_out(out_im, sizeof(double))},
+                    [&](int64_t, void* const* d) {
+                      k_cf_complex<<<(n + 127) / 128, 128, 0, ctx->stream>>>(
+                          (const double*)d[0], r, q, tau, (const double*)d[1], (const double*)d[2], n, (double*)d[3],
+                          (double*)d[4]);
+                      DHJ_LAUNCHED(ctx);
+                      return DHJ_OK;
+                    });
 }
 
 int dhj_truncation_range(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride,
@@ -1484,23 +1455,18 @@ int dhj_truncation_range(dhj_ctx* ctx, const double* params, int64_t P, const do
   if (s0_stride != 0 && s0_stride != 1) return fail(ctx, DHJ_ERR_ARG, "s0_stride must be 0 or 1");
   if (P == 0 || M == 0) return DHJ_OK;
   if (P * (int64_t)M > (int64_t)1 << 28) return fail(ctx, DHJ_ERR_ARG, "P*M too large for this helper");
-  Staged st{ctx};
-  const size_t pb = (size_t)P * kNumParams * sizeof(double), sb = (s0_stride ? (size_t)P : 1) * sizeof(double);
   const size_t mb = (size_t)M * sizeof(double);
-  int rc = st.begin(pb + sb + 2 * mb, (size_t)P * M * 2 * sizeof(double));
-  if (rc) return rc;
-  memcpy(st.hin(), params, pb);
-  memcpy(st.hin() + pb, S0, sb);
-  memcpy(st.hin() + pb + sb, strike, mb);
-  memcpy(st.hin() + pb + sb + mb, maturity, mb);
-  if ((rc = st.upload())) return rc;
-  const long long n = P * (long long)M;
-  k_truncation_range<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(
-      (const double*)st.din(), P, (const double*)(st.din() + pb), s0_stride, (const double*)(st.din() + pb + sb),
-      (const double*)(st.din() + pb + sb + mb), M, r, L, (double*)ctx->d_prices.p);
-  if ((rc = st.download())) return rc;
-  memcpy(out_ab, ctx->h_res.p, st.out_bytes);
-  return DHJ_OK;
+  return stage_sync(ctx, P, kOneChunk,
+                    {rows_in(params, kNumParams * sizeof(double)), s0_in(S0, s0_stride), table_in(strike, mb),
+                     table_in(maturity, mb), rows_out(out_ab, 2 * mb)},
+                    [&](int64_t, void* const* d) {
+                      const long long n = P * (long long)M;
+                      k_truncation_range<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(
+                          (const double*)d[0], P, (const double*)d[1], s0_stride, (const double*)d[2],
+                          (const double*)d[3], M, r, L, (double*)d[4]);
+                      DHJ_LAUNCHED(ctx);
+                      return DHJ_OK;
+                    });
 }
 
 int dhj_chi_psi(dhj_ctx* ctx, const int32_t* k, int32_t n, double c, double d, double a, double b,
@@ -1508,18 +1474,14 @@ int dhj_chi_psi(dhj_ctx* ctx, const int32_t* k, int32_t n, double c, double d, d
   if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
   if (!k || !out_chi || !out_psi || n < 0) return fail(ctx, DHJ_ERR_ARG, "bad arguments");
   if (n == 0) return DHJ_OK;
-  Staged st{ctx};
-  const size_t kb = (size_t)n * sizeof(int), ob = (size_t)n * sizeof(double);
-  int rc = st.begin(kb, 2 * ob);
-  if (rc) return rc;
-  memcpy(st.hin(), k, kb);
-  if ((rc = st.upload())) return rc;
-  double* dout = (double*)ctx->d_prices.p;
-  k_chi_psi<<<(n + 127) / 128, 128, 0, ctx->stream>>>((const int*)st.din(), n, c, d, a, b, dout, dout + n);
-  if ((rc = st.download())) return rc;
-  memcpy(out_chi, ctx->h_res.p, ob);
-  memcpy(out_psi, (unsigned char*)ctx->h_res.p + ob, ob);
-  return DHJ_OK;
+  return stage_sync(ctx, n, kOneChunk,
+                    {rows_in(k, sizeof(int32_t)), rows_out(out_chi, sizeof(double)), rows_out(out_psi, sizeof(double))},
+                    [&](int64_t, void* const* dev) {
+                      k_chi_psi<<<(n + 127) / 128, 128, 0, ctx->stream>>>((const int*)dev[0], n, c, d, a, b,
+                                                                           (double*)dev[1], (double*)dev[2]);
+                      DHJ_LAUNCHED(ctx);
+                      return DHJ_OK;
+                    });
 }
 
 }  // extern "C"
@@ -1556,8 +1518,7 @@ int enqueue_generate(dhj_ctx* ctx, const GenConfig& c, int64_t first, int64_t n,
   const long long q_first = first / g.path_len, q_last = (first + n - 1) / g.path_len;
   const long long paths = q_last - q_first + 1;
   k_gen_draws<<<(unsigned)((paths + kGenWarps - 1) / kGenWarps), 32 * kGenWarps, 0, st>>>(g, d_params, d_spots);
-  DHJ_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
+  DHJ_LAUNCHED(ctx);
   SliceView v;
   int rc = grid_view(ctx, c.strikes_rel, c.nK, c.maturities, c.nT, /*scale_by_spot=*/1, /*is_call=*/1, c.N, c.r, 0.0,
                      c.L, st, &v);
@@ -1574,8 +1535,7 @@ int enqueue_generate(dhj_ctx* ctx, const GenConfig& c, int64_t first, int64_t n,
     const size_t smem = (size_t)kGenMarketSamples * (M | 1) * sizeof(double);
     k_gen_market<<<(unsigned)((n + kGenMarketSamples - 1) / kGenMarketSamples), kGenMarketSamples, smem, st>>>(
         g.seed, first, n, M, g.noise_sd, d_model, d_market, d_loss);
-    DHJ_CUDA(ctx, cudaGetLastError());
-    ctx->launches++;
+    DHJ_LAUNCHED(ctx);
   }
   return DHJ_OK;
 }
@@ -1708,8 +1668,7 @@ int dhj_fp64_peak(dhj_ctx* ctx, int32_t iters, double* tflops, double* milliseco
     DHJ_CUDA(ctx, cudaEventRecord(e0, ctx->stream));
     if (rep < 4) k_fp64_peak<false><<<blocks, threads, 0, ctx->stream>>>((double*)ctx->d_peak.p, iters, 0.999999, 1e-7);
     else k_fp64_peak<true><<<blocks, threads, 0, ctx->stream>>>((double*)ctx->d_peak.p, iters, 0.999999, 1e-7);
-    DHJ_CUDA(ctx, cudaGetLastError());
-    ctx->launches++;
+    DHJ_LAUNCHED(ctx);
     DHJ_CUDA(ctx, cudaEventRecord(e1, ctx->stream));
     DHJ_CUDA(ctx, cudaEventSynchronize(e1));
     float ms = 0.f;

@@ -148,6 +148,46 @@ def _ptr(a: np.ndarray) -> int:
     return a.ctypes.data
 
 
+def _is_call(is_call, M):
+    return np.ascontiguousarray(np.broadcast_to(np.asarray(is_call), (M,)).astype(bool).astype(np.int32))
+
+
+def _strikes(strike, is_call, rows, M, what="P"):
+    """(strike, strike_stride, is_call) of an option list: strike [M] (stride 0) or [rows, M] (stride M), is_call
+    broadcast to int32[M]."""
+    strike = _f64(strike)
+    if strike.size == M:
+        strike, k_stride = strike.reshape(M), 0
+    elif strike.size == rows * M:
+        strike, k_stride = strike.reshape(rows, M), M
+    else:
+        raise ValueError(f"strike must be [M] or [{what}, M]")
+    return strike, k_stride, _is_call(is_call, M)
+
+
+def _option_list(values, S0, strike, maturity, is_call, per_option=False):
+    """(values, P, S0, s0_stride, strike, strike_stride, maturity, M, is_call) of an option list in dhj_price_list's
+    layout: values are parameter sets [P, 13] or, per_option, one value per option ([M] or [P, M]); S0 a scalar or
+    [P]; strike [M] or [P, M]."""
+    maturity = _f64(maturity).reshape(-1)
+    M = maturity.shape[0]
+    values = _f64(values)
+    if not per_option:
+        values = values.reshape(-1, N_PARAMS)
+    elif values.ndim == 2 and values.shape[1] == M:
+        pass
+    elif M and values.size % M == 0:
+        values = values.reshape(-1, M)
+    else:
+        raise ValueError("values must be [M] or [P, M]")
+    P = values.shape[0]
+    S0 = _f64(S0).reshape(-1)
+    if S0.size not in (1, P):
+        raise ValueError("S0 must be a scalar or have one entry per row")
+    strike, k_stride, call = _strikes(strike, is_call, P, M)
+    return values, P, S0, 0 if S0.size == 1 else 1, strike, k_stride, maturity, M, call
+
+
 class Context:
     """One libdhj context = one CUDA device.  Calls are serialised with a lock (the C side is not re-entrant)."""
 
@@ -198,8 +238,8 @@ class Context:
         """(prices float64[P, M], jac float64[P, M, 13]) of P parameter sets on an option list: jac[p, o, i] =
         d price / d param_i with the truncation range held at its value for the current parameters
         (dhj_price_jacobian)."""
-        params, P, S0, s0_stride, strike, k_stride, maturity, M, call = self._option_list(params, S0, strike, maturity,
-                                                                                        is_call)
+        params, P, S0, s0_stride, strike, k_stride, maturity, M, call = _option_list(params, S0, strike, maturity,
+                                                                                   is_call)
         prices, jac = np.empty((P, M)), np.empty((P, M, N_PARAMS))
         with self._lock:
             self._check(self._lib.dhj_price_jacobian(self._h, params, P, S0, s0_stride, float(r), float(q), strike,
@@ -211,8 +251,8 @@ class Context:
         """(prices float64[P, M], greeks float64[P, M, 5]) of P parameter sets on an option list: greeks[p, o] =
         (delta, gamma, theta, rho, rho_q) = (dV/dS0, d2V/dS0^2, -dV/dT, dV/dr, dV/dq), exact with the truncation
         range held at its value for the current inputs (dhj_price_greeks)."""
-        params, P, S0, s0_stride, strike, k_stride, maturity, M, call = self._option_list(params, S0, strike, maturity,
-                                                                                        is_call)
+        params, P, S0, s0_stride, strike, k_stride, maturity, M, call = _option_list(params, S0, strike, maturity,
+                                                                                   is_call)
         prices, greeks = np.empty((P, M)), np.empty((P, M, N_GREEKS))
         with self._lock:
             self._check(self._lib.dhj_price_greeks(self._h, params, P, S0, s0_stride, float(r), float(q), strike,
@@ -221,37 +261,12 @@ class Context:
         return prices, greeks
 
     # -- implied volatility -----------------------------------------------------------------------
-    @staticmethod
-    def _iv_list(values, S0, strike, maturity, is_call):
-        maturity = _f64(maturity).reshape(-1)
-        M = maturity.shape[0]
-        values = _f64(values)
-        if values.ndim == 2 and values.shape[1] == M:
-            P = values.shape[0]
-        elif M and values.size % M == 0:
-            P = values.size // M
-        else:
-            raise ValueError("values must be [M] or [P, M]")
-        values = values.reshape(P, M)
-        S0 = _f64(S0).reshape(-1)
-        if S0.size not in (1, P):
-            raise ValueError("S0 must be a scalar or have one entry per row")
-        strike = _f64(strike)
-        if strike.size == M:
-            strike, k_stride = strike.reshape(M), 0
-        elif strike.size == P * M:
-            strike, k_stride = strike.reshape(P, M), M
-        else:
-            raise ValueError("strike must be [M] or [P, M]")
-        call = np.ascontiguousarray(np.broadcast_to(np.asarray(is_call), (M,)).astype(bool).astype(np.int32))
-        return values, P, S0, 0 if S0.size == 1 else 1, strike, k_stride, maturity, M, call
-
     def implied_vol(self, price, S0, strike, maturity, is_call, r, q=0.0, return_status=False):
         """Black–Scholes implied vols float64[P, M] of prices [P, M] (or [M]) on an option list in price_list's layout:
         S0 scalar or [P], strike [M] or [P, M] (dhj_implied_vol).  NaN outside the no-arbitrage bounds; with
         return_status also the int32[P, M] status codes (IV_STATUS names them)."""
-        price, P, S0, s0_stride, strike, k_stride, maturity, M, call = self._iv_list(price, S0, strike, maturity,
-                                                                                     is_call)
+        price, P, S0, s0_stride, strike, k_stride, maturity, M, call = _option_list(price, S0, strike, maturity,
+                                                                                    is_call, per_option=True)
         vol, status = np.empty((P, M)), np.empty((P, M), dtype=np.int32)
         with self._lock:
             self._check(self._lib.dhj_implied_vol(self._h, price, P, S0, s0_stride, float(r), float(q), strike,
@@ -267,7 +282,7 @@ class Context:
         M = maturity.size
         if strike.size != M:
             raise ValueError("strike must be [M]")
-        call = np.ascontiguousarray(np.broadcast_to(np.asarray(is_call), (M,)).astype(bool).astype(np.int32))
+        call = _is_call(is_call, M)
         with self._lock:
             self._check(self._lib.dhj_implied_vol_dev(self._h, d_price, int(P), d_S0, int(s0_stride), float(r),
                                                       float(q), strike, int(bool(scale_by_spot)), maturity, call, M,
@@ -276,51 +291,18 @@ class Context:
 
     def bs_price(self, vol, S0, strike, maturity, is_call, r, q=0.0):
         """Black–Scholes prices float64[P, M] of vols [P, M] (or [M]) in implied_vol's layout (dhj_bs_price)."""
-        vol, P, S0, s0_stride, strike, k_stride, maturity, M, call = self._iv_list(vol, S0, strike, maturity, is_call)
+        vol, P, S0, s0_stride, strike, k_stride, maturity, M, call = _option_list(vol, S0, strike, maturity, is_call,
+                                                                                  per_option=True)
         out = np.empty((P, M))
         with self._lock:
             self._check(self._lib.dhj_bs_price(self._h, vol, P, S0, s0_stride, float(r), float(q), strike, k_stride,
                                                maturity, call, M, _ptr(out)), "dhj_bs_price")
         return out
 
-    @staticmethod
-    def _option_list(params, S0, strike, maturity, is_call):
-        params = _f64(params).reshape(-1, N_PARAMS)
-        P = params.shape[0]
-        maturity = _f64(maturity).reshape(-1)
-        M = maturity.shape[0]
-        S0 = _f64(S0).reshape(-1)
-        if S0.size not in (1, P):
-            raise ValueError("S0 must be a scalar or have one entry per parameter set")
-        s0_stride = 0 if S0.size == 1 else 1
-        strike = _f64(strike)
-        if strike.size == M:
-            strike, k_stride = strike.reshape(M), 0
-        elif strike.size == P * M:
-            strike, k_stride = strike.reshape(P, M), M
-        else:
-            raise ValueError("strike must be [M] or [P, M]")
-        call = np.ascontiguousarray(np.broadcast_to(np.asarray(is_call), (M,)).astype(bool).astype(np.int32))
-        return params, P, S0, s0_stride, strike, k_stride, maturity, M, call
-
     def price_list(self, params, S0, strike, maturity, is_call, r, q=0.0, N=128, L=10.0) -> np.ndarray:
         """Prices float64[P, M] of P parameter sets on an option list (dhj_price_list)."""
-        params = _f64(params).reshape(-1, N_PARAMS)
-        P = params.shape[0]
-        maturity = _f64(maturity).reshape(-1)
-        M = maturity.shape[0]
-        S0 = _f64(S0).reshape(-1)
-        if S0.size not in (1, P):
-            raise ValueError("S0 must be a scalar or have one entry per parameter set")
-        s0_stride = 0 if S0.size == 1 else 1
-        strike = _f64(strike)
-        if strike.size == M:
-            strike, k_stride = strike.reshape(M), 0
-        elif strike.size == P * M:
-            strike, k_stride = strike.reshape(P, M), M
-        else:
-            raise ValueError("strike must be [M] or [P, M]")
-        call = np.ascontiguousarray(np.broadcast_to(np.asarray(is_call), (M,)).astype(bool).astype(np.int32))
+        params, P, S0, s0_stride, strike, k_stride, maturity, M, call = _option_list(params, S0, strike, maturity,
+                                                                                   is_call)
         out = np.empty((P, M), dtype=np.float64)
         with self._lock:
             self._check(self._lib.dhj_price_list(self._h, params, P, S0, s0_stride, float(r), float(q), strike,
@@ -465,14 +447,7 @@ class Market:
         S0 = _f64(S0).reshape(-1)
         n = S0.size
         price = _f64(price).reshape(n, M)
-        strike = _f64(strike)
-        if strike.size == M:
-            strike, k_stride = strike.reshape(M), 0
-        elif strike.size == n * M:
-            strike, k_stride = strike.reshape(n, M), M
-        else:
-            raise ValueError("strike must be [M] or [n_markets, M]")
-        call = np.ascontiguousarray(np.broadcast_to(np.asarray(is_call), (M,)).astype(bool).astype(np.int32))
+        strike, k_stride, call = _strikes(strike, is_call, n, M, "n_markets")
         self.n_markets, self.M, self.N = n, M, int(N)
         self.objective = "price"
         self._h = _c_vp()
@@ -492,16 +467,17 @@ class Market:
             pass
 
     @staticmethod
-    def _index(market_index, B):
-        if market_index is None:
-            return None, None
-        idx = np.ascontiguousarray(np.asarray(market_index, dtype=np.int32).reshape(B))
-        return idx, idx.ctypes.data
-
-    def loss_batch(self, x, market_index=None) -> np.ndarray:
+    def _batch(x, market_index):
+        """(x float64[B, 13], B, market index int32[B] or None, its pointer or None)"""
         x = _f64(x).reshape(-1, N_PARAMS)
         B = x.shape[0]
-        idx, pidx = self._index(market_index, B)
+        if market_index is None:
+            return x, B, None, None
+        idx = np.ascontiguousarray(np.asarray(market_index, dtype=np.int32).reshape(B))
+        return x, B, idx, idx.ctypes.data
+
+    def loss_batch(self, x, market_index=None) -> np.ndarray:
+        x, B, idx, pidx = self._batch(x, market_index)
         out = np.empty(B)
         c = self.ctx
         with c._lock:
@@ -510,9 +486,7 @@ class Market:
 
     def loss_fd(self, x, h=1e-8, market_index=None, want_all=False):
         """(f[C], g[C,13][, f_all[C,14]]) in one launch (dhj_loss_fd)."""
-        x = _f64(x).reshape(-1, N_PARAMS)
-        C = x.shape[0]
-        idx, pidx = self._index(market_index, C)
+        x, C, idx, pidx = self._batch(x, market_index)
         f, g = np.empty(C), np.empty((C, N_PARAMS))
         f_all = np.empty((C, FD_POINTS)) if want_all else None
         c = self.ctx
@@ -524,9 +498,7 @@ class Market:
     def loss_grad(self, x, market_index=None):
         """(f[C], g[C,13]): the loss and its exact gradient in the unconstrained x (dhj_loss_grad; truncation range
         held fixed, g = 0 where f is the 1e10 sentinel)."""
-        x = _f64(x).reshape(-1, N_PARAMS)
-        C = x.shape[0]
-        idx, pidx = self._index(market_index, C)
+        x, C, idx, pidx = self._batch(x, market_index)
         f, g = np.empty(C), np.empty((C, N_PARAMS))
         c = self.ctx
         with c._lock:
@@ -556,9 +528,7 @@ class Market:
     def implied_vols(self, x, market_index=None):
         """(vol[B, M], status[B, M]): Black–Scholes implied vols (q = 0) of the model prices at the unconstrained x
         and their IV_STATUS codes, every option (dhj_market_implied_vols)."""
-        x = _f64(x).reshape(-1, N_PARAMS)
-        B = x.shape[0]
-        idx, pidx = self._index(market_index, B)
+        x, B, idx, pidx = self._batch(x, market_index)
         vol, status = np.empty((B, self.M)), np.empty((B, self.M), dtype=np.int32)
         c = self.ctx
         with c._lock:
@@ -567,9 +537,7 @@ class Market:
         return vol, status
 
     def prices(self, x, market_index=None) -> np.ndarray:
-        x = _f64(x).reshape(-1, N_PARAMS)
-        B = x.shape[0]
-        idx, pidx = self._index(market_index, B)
+        x, B, idx, pidx = self._batch(x, market_index)
         out = np.empty((B, self.M))
         c = self.ctx
         with c._lock:
@@ -635,26 +603,20 @@ class BatchLBFGS:
         `market` over all states that wait for an evaluation (state i uses market `state_market[i]`), until every
         optimiser has stopped.  Returns (rounds, state_rounds, (seconds in ask, loss, tell)).  The GIL is released for
         the whole call."""
-        sm = None if state_market is None else np.ascontiguousarray(np.asarray(state_market, dtype=np.int32).reshape(self.n))
-        rounds, state_rounds, secs = _c_i64(), _c_i64(), np.zeros(3)
-        c = market.ctx
-        with c._lock:
-            c._check(self._lib.dhj_lbfgs_minimize_fd(self._h, c._h, market._h, None if sm is None else sm.ctypes.data,
-                                                     self.n, float(h), ctypes.byref(rounds), ctypes.byref(state_rounds),
-                                                     secs), "dhj_lbfgs_minimize_fd")
-        return rounds.value, state_rounds.value, tuple(secs)
+        return self._minimize("dhj_lbfgs_minimize_fd", market, state_market, float(h))
 
     def minimize_grad(self, market: "Market", state_market=None):
         """minimize_fd with the analytic gradient (dhj_lbfgs_minimize_grad): every round one `dhj_loss_grad` call,
         one loss evaluation per request.  Returns (rounds, state_rounds, (seconds in ask, loss, tell))."""
+        return self._minimize("dhj_lbfgs_minimize_grad", market, state_market)
+
+    def _minimize(self, name, market, state_market, *args):
         sm = None if state_market is None else np.ascontiguousarray(np.asarray(state_market, dtype=np.int32).reshape(self.n))
         rounds, state_rounds, secs = _c_i64(), _c_i64(), np.zeros(3)
         c = market.ctx
         with c._lock:
-            c._check(self._lib.dhj_lbfgs_minimize_grad(self._h, c._h, market._h,
-                                                       None if sm is None else sm.ctypes.data, self.n,
-                                                       ctypes.byref(rounds), ctypes.byref(state_rounds), secs),
-                     "dhj_lbfgs_minimize_grad")
+            c._check(getattr(self._lib, name)(self._h, c._h, market._h, None if sm is None else sm.ctypes.data, self.n,
+                                              *args, ctypes.byref(rounds), ctypes.byref(state_rounds), secs), name)
         return rounds.value, state_rounds.value, tuple(secs)
 
     def result(self):
