@@ -129,11 +129,20 @@ def test_greeks_nan_and_empty(ctx):
 
 
 def test_checked_build_greeks():
+    """Zero violations and the product build's bits on the binding family, the surface and the multi-chunk slices of
+    test_gpu_derivative_edges (449 strikes with binding strikes at the 224 boundary, ragged N, per-set rows, and the
+    reversed and one-option compositions)."""
     import dhj
+    import test_gpu_derivative_edges as E
+    edge = [E._greeks_case(n)[:8] for n in ("bind224-128", "bind224-33", "n449", "per_set")]
+    pe, Se, Ke, Te, ce, re, qe, Ne = edge[0]
+    edge.append((pe, Se, Ke[::-1], Te[::-1], ce[::-1], re, qe, Ne))
+    edge.append((pe, Se, Ke[224:225], Te[224:225], ce[224:225], re, qe, Ne))
     outs = []
     for lib in (None, CHECKED):
         c = dhj.Context(0, library=lib)
         res = [c.price_greeks(*_families()[f][1:]) for f in (3, 4)]
+        res += [c.price_greeks(p, s, k, t, cc, rr, qq, N=n) for p, s, k, t, cc, rr, qq, n in edge]
         if lib:
             enabled, counts = c.debug_checks()
             assert enabled and not counts.any(), counts

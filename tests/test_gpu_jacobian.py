@@ -139,23 +139,35 @@ def test_loss_grad_deterministic(ctx):
 
 
 def test_checked_build_jacobian():
+    """Zero violations and the product build's bits on: the binding family, the multi-chunk slices of
+    test_gpu_derivative_edges (129 strikes with binding strikes at the chunk boundary, every strike binding, 200
+    strikes, ragged N, per-set rows, and the reversed and one-option compositions), the dense market's loss_grad and
+    loss_grad over 16 markets with a shuffled market_index."""
     import dhj
+    import test_gpu_derivative_edges as E
     name, params, S0, K, T, call, r = _families()[2]
     tag, S0m, rm, Km, Tm, callm, mk, x = _markets()[2]
+    edge_cases = [E._jac_case(n)[:9] for n in ("bind_edges-128", "bind_edges-33", "all_bind", "n200", "per_set_L12")]
+    pe, Se, Ke, Te, ce, re, qe, Ne, Le = edge_cases[0]
+    edge_cases.append((pe, Se, Ke[::-1], Te[::-1], ce[::-1], re, qe, Ne, Le))
+    edge_cases.append((pe, Se, Ke[64:65], Te[64:65], ce[64:65], re, qe, Ne, Le))
+    many = None
     outs = []
     for lib in (None, CHECKED):
         c = dhj.Context(0, library=lib)
-        pj = c.price_jacobian(params, S0, K, T, call, r)
-        fg = c.market(S0m, rm, Km, Tm, callm, mk).loss_grad(x)
+        if many is None:
+            many = E._multi_market(c, 16, 3)
+        Sm, rmm, Kmm, Tmm, cm, mkm, xm, im = many
+        res = [c.price_jacobian(params, S0, K, T, call, r), c.market(S0m, rm, Km, Tm, callm, mk).loss_grad(x),
+               c.market(Sm, rmm, Kmm, Tmm, cm, mkm).loss_grad(xm, im)]
+        res += [c.price_jacobian(p, s, k, t, cc, rr, qq, N=n, L=l) for p, s, k, t, cc, rr, qq, n, l in edge_cases]
         if lib:
             enabled, counts = c.debug_checks()
             assert enabled and not counts.any(), counts
-        outs.append((pj, fg))
+        outs.append(res)
         c.close()
-    (pa, ja), (fa, ga) = outs[0]
-    (pb, jb), (fb, gb) = outs[1]
-    assert np.array_equal(pa, pb) and np.array_equal(ja, jb)
-    assert np.array_equal(fa, fb) and np.array_equal(ga, gb)
+    for a, b in zip(*outs):
+        assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1])
 
 
 # ---- calibrations driven by the analytic gradient ---------------------------------------------------------------

@@ -126,24 +126,51 @@ def emu_jac():
     lib.emu_price_jacobian.argtypes = [D, D, D, D, I, ctypes.c_double, ctypes.c_double, ctypes.c_long, ctypes.c_int,
                                        ctypes.c_int, ctypes.c_double, D, D]
 
-    def run(params, S0, K, T, call, r, N=128):
+    def run(params, S0, K, T, call, r, N=128, q=0.0, L=10.0):
+        """S0 a scalar or [P], K [M] or [P, M] (per-set strike rows)."""
         params = np.ascontiguousarray(params, dtype=np.float64).reshape(-1, 13)
         P, M = len(params), len(T)
         prices, jac = np.empty((P, M)), np.empty((P, M, 13))
-        lib.emu_price_jacobian(params, np.full(P, float(S0)), np.ascontiguousarray(np.tile(K, (P, 1)), dtype=np.float64),
-                               np.ascontiguousarray(T, dtype=np.float64), np.asarray(call).astype(np.int32), r, 0.0, P,
-                               M, N, 10.0, prices, jac)
+        S0 = np.ascontiguousarray(np.broadcast_to(np.asarray(S0, dtype=np.float64), (P,)))
+        K = np.ascontiguousarray(np.broadcast_to(np.asarray(K, dtype=np.float64), (P, M)))
+        lib.emu_price_jacobian(params, S0, K, np.ascontiguousarray(T, dtype=np.float64),
+                               np.asarray(call).astype(np.int32), r, q, P, M, N, L, prices, jac)
         return prices, jac
     return run
 
 
-@pytest.mark.parametrize("N", [128, 256])
-@pytest.mark.parametrize("case", range(3))
+def _emu_cases():
+    """(name, params, S0, K, T, call, r, q, L): _cases() with q = 0 and L = 10; a 129-strike slice at T = 0.05 with
+    K 40-160 (many binding strikes), calls and puts; per-set spots 80 / 100 / 130 with per-set strike rows (65
+    strikes at T = 0.1, 13 at T = 1), r = 0.02, q = 0.015 and L = 8 or 12."""
+    out = [c + (0.0, 10.0) for c in _cases()]
+    rng = np.random.default_rng(3)
+    lo, hi = O.GENERATOR_RANGES[:, 0], O.GENERATOR_RANGES[:, 1]
+    params = lo + (hi - lo) * rng.random((3, 13))
+    Kw = np.linspace(40.0, 160.0, 129)
+    out.append(("wide129", params, 100.0, Kw, np.full(129, 0.05), np.arange(129) % 2 == 0, 0.03, 0.0, 10.0))
+    S0 = np.array([80.0, 100.0, 130.0])
+    Kp = S0[:, None] * np.linspace(0.6, 1.45, 65)[None, :] * (1 + 0.01 * rng.standard_normal((3, 65)))
+    Kp = np.concatenate([Kp, Kp[:, ::5]], axis=1)
+    Tp = np.concatenate([np.full(65, 0.1), np.full(13, 1.0)])
+    for L in (8.0, 12.0):
+        out.append((f"per_set_L{L:g}", params, S0, Kp, Tp, np.arange(78) % 2 == 1, 0.02, 0.015, L))
+    return out
+
+
+@pytest.mark.parametrize("N", [128, 256, 2, 33, 1000])
+@pytest.mark.parametrize("case", range(6))
 def test_emulated_device_jacobian(emu_jac, case, N):
-    """Device arithmetic vs the oracle: <= 1e-10 of the column scale (measured worst 1e-11, sigma / kappa columns)."""
-    name, params, S0, K, T, call, r = _cases()[case]
-    prices, jac = emu_jac(params, S0, K, T, call, r, N)
-    want_p, want_j = J.price_jacobian_batch(params, S0, K, T, call, r, N=N)
+    """Device arithmetic vs the oracle: <= 1e-10 of the column scale (measured worst 3.0e-11 for N >= 33, c5_calls),
+    also at a one-block and ragged N, with binding strikes, per-set rows, q != 0 and L != 10."""
+    name, params, S0, K, T, call, r, q, L = _emu_cases()[case]
+    prices, jac = emu_jac(params, S0, K, T, call, r, N, q, L)
+    want_p, want_j = J.price_jacobian_batch(params, S0, K, T, call, r, q, N=N, L=L, chunk=1)
     scale = np.abs(want_j).max(axis=1, keepdims=True)
-    assert (np.abs(jac - want_j) / scale).max() <= 1e-10, name
-    assert np.abs(prices - want_p).max() <= 1e-11 * S0
+    err = (np.abs(jac - want_j) / scale).max()
+    print(f"{name} N={N}: worst |jac - oracle| / column scale {err:.2e}")
+    # at N = 2 the series has two terms: a column's largest entry falls up to 9x below its N = 128 value while the
+    # rounding of a deep in-the-money binding strike's S0-sized terms does not (measured 1.6e-10 on wide129, sigma2
+    # column, K = 45.6; every other case <= 7.8e-11)
+    assert err <= (3e-10 if N == 2 else 1e-10), name
+    assert np.abs(prices - want_p).max() <= 1e-11 * np.max(S0)
