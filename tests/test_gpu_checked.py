@@ -17,6 +17,7 @@ import pytest
 
 from conftest import PKG
 from oracle import cos_oracle as O
+from test_gpu_derivative_edges import _bind_slice
 
 pytestmark = pytest.mark.gpu
 
@@ -40,6 +41,12 @@ def _workload(ctx):
     out["slices"] = ctx.price_list(params[:50], 100.0, np.full(40, 100.0), np.linspace(0.1, 2.0, 40), np.ones(40), 0.03)
     # dense kernel: regular and binding strikes, two chunks (300 strikes), N = 256
     out["dense"] = ctx.price_grid(params[:64], 100.0, np.linspace(50.0, 150.0, 300), np.array([0.02, 0.25, 1.0]), 0.03, N=256)
+    # dense kernel at N = 1000: 449 strikes binding at lane and chunk edges; batch kernel at N = 257: an 8-strike slice
+    # binding at 1 and 6 (the extra passes' rotation steps through the pointer shift)
+    Kb, cb = _bind_slice(449, (0, 31, 32, 63, 64, 223, 224, 448))
+    out["dense_bind"] = ctx.price_list(params[:6], 100.0, Kb, np.full(449, 0.05), cb, 0.03, N=1000)
+    Kb, cb = _bind_slice(8, (1, 6))
+    out["batch_bind"] = ctx.price_list(params[:200], 100.0, Kb, np.full(8, 0.05), cb, 0.03, N=257)
     # loss: fused kernel (small), split path (large), dense market
     Km = np.tile(O.GENERATOR_STRIKES_REL, 3); Tm = np.repeat(O.GENERATOR_MATURITIES, 5)
     market = out["grid"][0].reshape(-1) * (1 + 0.02 * rng.standard_normal(15))
@@ -53,6 +60,14 @@ def _workload(ctx):
     mk2 = ctx.market(100.0, 0.02, K2, T2, np.ones(15), np.full(15, 5.0))
     out["fd_dense"] = np.concatenate(mk2.loss_fd(x[:20]), axis=None)
     mk2.close()
+    # fused loss with 32 maturities (one unit per block); FD on a Market with N = 257
+    T32 = np.repeat(np.linspace(0.1, 2.0, 32), 2); K32 = np.tile([95.0, 105.0], 32)
+    mk3 = ctx.market(100.0, 0.03, K32, T32, np.arange(64) % 2 == 0, np.full(64, 5.0))
+    out["fd_slices32"] = np.concatenate(mk3.loss_fd(x[:30]), axis=None)
+    mk3.close()
+    mk4 = ctx.market(float(spots[0]), 0.03, Km * spots[0] / 100.0, Tm, np.ones(15), market, N=257)
+    out["fd_n257"] = np.concatenate(mk4.loss_fd(x[:40]), axis=None)
+    mk4.close()
     # dataset sweep
     g = ctx.generate(3, 250, 2100, 500, lo, hi, 0.9, 100.0, 0.0003, 0.01, 0.02, O.GENERATOR_STRIKES_REL,
                      O.GENERATOR_MATURITIES, 0.03)

@@ -286,7 +286,7 @@ def test_loss_general_path(ctx):
 
 
 def test_many_strikes_and_slices(ctx):
-    """300 strikes on one slice (two 256-strike chunks) and 40 maturities (more slices than a block batch)."""
+    """300 strikes on one slice (chunks of 224 and 76 strikes) and 40 maturities (more slices than a block batch)."""
     rng = np.random.default_rng(10)
     params = rng.uniform(O.GENERATOR_RANGES[:, 0], O.GENERATOR_RANGES[:, 1], size=(3, 13))
     K = np.linspace(70, 130, 300); T = np.full(300, 0.75)

@@ -13,6 +13,7 @@ from numpy.ctypeslib import ndpointer
 from conftest import PKG, ROOT, rel_err
 
 EMU_DIR = os.path.join(ROOT, "tests", "host_emu")
+WALKS = ("r01", "batch", "dense")
 
 
 @pytest.fixture(scope="module")
@@ -40,6 +41,22 @@ def emu():
         lib.emu_price_list(params, S0, 1, strike, M, mat, call, r, q, P, M, N, L, out, ab)
         return out, ab
 
+    U8 = ndpointer(np.uint8, flags="C")
+    lib.emu_price_walk.argtypes = [ctypes.c_int, D, D, D, D, I, ctypes.c_double, ctypes.c_double, ctypes.c_long,
+                                   ctypes.c_int, ctypes.c_int, ctypes.c_double, D, U8]
+
+    def price_walk(walk, params, S0, strike, mat, call, r, q=0.0, N=128, L=10.0):
+        """(prices[P, M], binding[P, M]) in the order of walk "r01", "batch" or "dense"."""
+        params = np.ascontiguousarray(params, dtype=np.float64).reshape(-1, 13)
+        P, M = len(params), len(mat)
+        S0 = np.ascontiguousarray(np.broadcast_to(np.asarray(S0, dtype=np.float64), (P,)))
+        strike = np.ascontiguousarray(np.broadcast_to(np.asarray(strike, dtype=np.float64), (P, M)))
+        call = np.ascontiguousarray(np.broadcast_to(np.asarray(call), (M,)).astype(np.int32))
+        out, bind = np.empty((P, M)), np.empty((P, M), dtype=np.uint8)
+        lib.emu_price_walk(WALKS.index(walk), params, S0, strike, np.ascontiguousarray(mat, dtype=np.float64), call,
+                           r, q, P, M, N, L, out, bind)
+        return out, bind.astype(bool)
+
     def loss(x, S0, r, strike, mat, call, market, N=128):
         x = np.ascontiguousarray(x, dtype=np.float64).reshape(-1, 13)
         out = np.empty(len(x))
@@ -49,6 +66,7 @@ def emu():
                      np.ascontiguousarray(market, dtype=np.float64), len(mat), N, out)
         return out
 
+    price_list.walk = price_walk
     return price_list, loss
 
 
@@ -99,3 +117,41 @@ def test_emu_loss(emu, golden):
         want = g[f"{tag}_loss"]
         assert np.array_equal(got == 1e10, want == 1e10)
         assert (np.abs(got - want) <= 1e-9 * np.maximum(1.0, np.abs(want))).all()
+
+
+# ---- the current kernels' orders (k_price_batch, k_price_dense) on families b and c of test_gpu_price_edges ----------
+@pytest.mark.parametrize("walk", ["batch", "dense"])
+@pytest.mark.parametrize("N", [2, 33, 256, 257, 1000, 2048])
+def test_emu_walks_binding_positions(emu, walk, N):
+    """Binding strikes at every position of 8-strike slices (their own pass, (a, b) and jump recurrences) through
+    both kernels' orders, against the C oracle at the GPU test's bounds; the emulation finds the same binding
+    strikes as the oracle."""
+    from test_gpu_price_edges import _batch_binding_list, _check
+    params, K, T, call, mask = _batch_binding_list()
+    got, bind = emu[0].walk(walk, params, 100.0, K, T, call, 0.03, 0.01, N)
+    assert (bind == mask).all()
+    _check(f"emulated {walk} walk, binding positions N={N}", got, params, 100.0, K, T, call, 0.03, 0.01, N)
+
+
+@pytest.mark.parametrize("walk", ["batch", "dense"])
+@pytest.mark.parametrize("N", [255, 256, 257, 512, 1000, 2048])
+def test_emu_walks_recurrence_family(emu, walk, N):
+    """Low-diffusion, jump-dominated sets whose blocks beyond k = 256 carry weight: the jump term's rotation and
+    Gaussian ratio and the segment starts' rotation between the exact blocks, against the C oracle."""
+    from test_gpu_price_edges import REC_STRIKES, _check, _rec_case
+    params, K, T, call, mask = _rec_case(REC_STRIKES[walk])
+    got, bind = emu[0].walk(walk, params, 100.0, K, T, call, 0.03, 0.0, N)
+    assert (bind == mask).all()
+    _check(f"emulated {walk} walk, recurrence family N={N}", got, params, 100.0, K, T, call, 0.03, 0.0, N)
+
+
+def test_emu_walks_agree_with_r01_order(emu):
+    """The three orders price the C2 grid alike to 1e-12 relative (the arithmetic is the same up to summation order
+    and the recurrences)."""
+    from test_gpu_derivative_edges import _params
+    params = _params(20, 27)
+    K, T = np.tile(np.linspace(90.0, 110.0, 5), 3), np.repeat([0.25, 0.5, 1.0], 5)
+    ref, _ = emu[0].walk("r01", params, 100.0, K, T, np.arange(15) % 2 == 0, 0.03)
+    for walk in ("batch", "dense"):
+        got, _ = emu[0].walk(walk, params, 100.0, K, T, np.arange(15) % 2 == 0, 0.03)
+        assert rel_err(got, ref).max() <= 1e-12, walk
