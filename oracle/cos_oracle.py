@@ -459,13 +459,18 @@ def counter_draws(seed, first, n, path_len, lo=None, hi=None, persistence=0.9, s
     return params[cut:], spots[cut:], noise[cut:]
 
 
-def counter_generate(seed, first, n, path_len, r=GENERATOR_RATE, N=128, **kw):
-    """Full restatement of the sweep: draws, C-oracle prices on the generator grid (K = K_rel * spot / 100,
-    :123-138), market = price + noise * price (:141-142), loss = mean(((model - market) / market)^2) (:154-157)."""
-    params, spots, noise = counter_draws(seed, first, n, path_len, **kw)
-    K = np.tile(GENERATOR_STRIKES_REL[None, :] * spots[:, None] / 100.0, (1, GENERATOR_MATURITIES.size))
-    T = np.repeat(GENERATOR_MATURITIES, GENERATOR_STRIKES_REL.size)
-    model = c_price_batch(params, spots, K, T, np.ones(T.size), r, 0.0, N)
+def counter_generate(seed, first, n, path_len, r=GENERATOR_RATE, N=128, strikes_rel=None, maturities=None, L=10,
+                     **kw):
+    """Full restatement of the sweep: draws, C-oracle prices of calls on the nT x nK grid (maturity-major,
+    K = K_rel * spot / 100, :123-138; the generator's 3 x 5 grid by default), market = price + noise * price
+    (:141-142), loss = mean(((model - market) / market)^2) (:154-157).  One noise factor per option (slots
+    8 .. 8 + (M - 1) / 2)."""
+    strikes_rel = GENERATOR_STRIKES_REL if strikes_rel is None else np.asarray(strikes_rel, dtype=np.float64).ravel()
+    maturities = GENERATOR_MATURITIES if maturities is None else np.asarray(maturities, dtype=np.float64).ravel()
+    params, spots, noise = counter_draws(seed, first, n, path_len, n_noise=strikes_rel.size * maturities.size, **kw)
+    K = np.tile(strikes_rel[None, :] * spots[:, None] / 100.0, (1, maturities.size))
+    T = np.repeat(maturities, strikes_rel.size)
+    model = c_price_batch(params, spots, K, T, np.ones(T.size), r, 0.0, N, L)
     market = model + noise * model
     loss = np.mean(((model - market) / market) ** 2, axis=1)
     return {"params": params, "spots": spots, "noise": noise, "model": model, "market": market, "loss": loss}

@@ -72,6 +72,10 @@ def _workload(ctx):
     g = ctx.generate(3, 250, 2100, 500, lo, hi, 0.9, 100.0, 0.0003, 0.01, 0.02, O.GENERATOR_STRIKES_REL,
                      O.GENERATOR_MATURITIES, 0.03)
     out.update({"gen_" + k: v for k, v in g.items()})
+    # the sweep's dense pricing with per-sample spots: a 1 x 32 grid at N = 257, 33-step paths, first inside a tile
+    g = ctx.generate(5, 33 * 4 + 9, 700, 33, lo, hi, 0.9, 100.0, 0.0003, 0.01, 0.02, np.linspace(80.0, 120.0, 32),
+                     [0.5], 0.03, N=257)
+    out.update({"gen32_" + k: v for k, v in g.items()})
     return out
 
 

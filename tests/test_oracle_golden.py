@@ -280,3 +280,59 @@ def test_counter_stream_known_answers():
     assert np.array_equal(p2, p[700:800]) and np.array_equal(s2, s[700:800]) and np.array_equal(n2, nz[700:800])
     big = O.counter_draws(3, 0, 20000, 1)[2]
     assert abs(big.std() - 0.02) < 3e-4 and abs(big.mean()) < 3e-4
+
+
+def test_counter_generate_grid():
+    """counter_generate on any nT x nK grid: the default is the generator's 3 x 5 grid, bit for bit; an option's noise
+    slot depends on its column only, so the first 15 noise columns of a 32-option grid are the 15-option noise."""
+    g = O.counter_generate(9, 480, 40, 500)
+    e = O.counter_generate(9, 480, 40, 500, strikes_rel=O.GENERATOR_STRIKES_REL, maturities=O.GENERATOR_MATURITIES,
+                           L=10)
+    for key in g:
+        assert np.array_equal(g[key], e[key]), key
+    assert g["model"].shape == (40, 15) and g["noise"].shape == (40, 15)
+    w = O.counter_generate(9, 480, 40, 500, strikes_rel=np.linspace(80.0, 120.0, 32), maturities=[0.5])
+    assert w["model"].shape == (40, 32) and w["noise"].shape == (40, 32)
+    assert np.array_equal(w["noise"][:, :15], g["noise"]) and np.array_equal(w["params"], g["params"])
+    assert np.array_equal(w["market"], w["model"] + w["noise"] * w["model"])
+    assert np.array_equal(w["loss"], np.mean(((w["model"] - w["market"]) / w["market"]) ** 2, axis=1))
+
+
+def test_counter_stream_exact_invariants():
+    """persistence = 0 gives the raw draws, persistence = 1 repeats each path's head row, noise_sd = 0 gives
+    market == model and a zero loss; all bit for bit."""
+    raw = O.counter_draws(5, 0, 300, 1)[0]
+    assert np.array_equal(O.counter_draws(5, 0, 300, 100, persistence=0.0)[0], raw)
+    p1 = O.counter_draws(5, 30, 270, 100, persistence=1.0)[0]                 # paths start at 100 and 200
+    heads = np.repeat(raw[[0, 100, 200]], 100, axis=0)[30:]
+    assert np.array_equal(p1, heads)
+    g = O.counter_generate(5, 30, 20, 100, noise_sd=0.0)
+    assert np.array_equal(g["market"], g["model"]) and (g["loss"] == 0.0).all()
+
+
+def test_counter_stream_64bit_words():
+    """The key's high word (seed >> 32) and the counter's high word (index >> 32) reach the draws; a path that
+    straddles index 2^32 continues its recurrences across it."""
+    p7, s7, n7 = O.counter_draws(7, 0, 64, 1)
+    for seed in (2 ** 32 + 7, 2 ** 63 + 7):                                   # same low word as seed 7
+        p, s, nz = O.counter_draws(seed, 0, 64, 1)
+        assert (p != p7).all(axis=1).all() and (nz != n7).all()
+    w_lo = O.counter_words(7, np.array([5], dtype=np.uint64), 0)
+    w_hi = O.counter_words(7, np.array([2 ** 32 + 5], dtype=np.uint64), 0)
+    assert w_lo[0][0] != w_hi[0][0] and w_lo[1][0] != w_hi[1][0]
+    c = 2 ** 32
+    assert c % 500 not in (0, 1)                                              # index 2^32 is inside a path
+    first = c - 700
+    p, s, nz = O.counter_draws(7, first, 1400, 500)
+    raw = O.counter_draws(7, first, 1400, 1)[0]
+    z0, _ = O.counter_normal_pair(7, np.arange(first, first + 1400, dtype=np.uint64), 7)
+    ret = 0.0003 + 0.01 * z0
+    t = np.arange(first, first + 1400) % 500
+    for k in range(1, 1400):
+        if t[k] == 0:
+            assert np.array_equal(p[k], raw[k]) and s[k] == 100.0
+        else:
+            assert np.array_equal(p[k], 0.9 * p[k - 1] + (1 - 0.9) * raw[k]), k
+            assert s[k] == s[k - 1] * (1.0 + ret[k]), k
+    straddle = np.flatnonzero((np.arange(first, first + 1400) // 500) == c // 500)
+    assert straddle[0] + first < c < straddle[-1] + first                   # the path around 2^32 is all there
