@@ -315,6 +315,40 @@ DHJ_API int dhj_generate(dhj_ctx* ctx, uint64_t seed, int64_t first, int64_t n, 
                          double r, int32_t N, double L, double* params, double* spots, double* model, double* market,
                          double* loss);
 
+/* ---- Monte Carlo pricing of path-dependent options ---------------------------------------------
+ * dhj_mc_price: P parameter sets params[P][13] (calibrator order), one spot S0[0] (s0_stride 0) or S0[P] (1), one
+ * maturity T, continuous rates r and q, and M <= DHJ_MC_MAX_OPTIONS options: kind[M] (DHJ_MC_*), is_call[M] (nonzero:
+ * call), strike[M] (finite, >= 0) and barrier[M] (finite, > 0 for the barrier kinds; ignored otherwise; the whole
+ * array may be NULL when no option has a barrier).  n_paths paths per set; out_price[P][M] = e^{-rT} x the mean payoff,
+ * out_stderr[P][M] (may be NULL) = its standard error e^{-rT} sqrt(sample variance / n_paths) (NaN for n_paths = 1).
+ *
+ * Scheme: n_steps equal steps dt = T / n_steps, full-truncation Euler for the two variances (Lord, Koekkoek, van Dijk
+ * 2010) and log-Euler for the spot with Poisson(lambda dt) Merton jumps per step; e^{-(r-q)t} S_t is an exact
+ * martingale of the scheme, so the forward is unbiased, but the variance paths are discretised and the price is NOT an
+ * unbiased estimate of the continuous-time price: the bias shrinks with dt (measured against the COS price in
+ * DESIGN.md §6f) and barriers are monitored at the observation dates only (no continuity correction).  n_obs divides
+ * n_steps; the observations are the ends of steps i n_steps / n_obs, i = 1..n_obs (S0 is not one):
+ *   DHJ_MC_EUROPEAN  max(+-(S_T - K), 0)               DHJ_MC_ASIAN    max(+-(A - K), 0), A = mean of S at the dates
+ *   DHJ_MC_UP_OUT    European payoff if max S < B      DHJ_MC_UP_IN    ... if max S >= B
+ *   DHJ_MC_DOWN_OUT  ... if min S > B                  DHJ_MC_DOWN_IN  ... if min S <= B
+ * Random numbers: Philox4x32-10 keyed by `seed`, a function of (seed, path, step) only (stream in csrc/dhj_mc.cuh):
+ * every parameter set of a call sees the same numbers, and the outputs have the same bits from run to run and do not
+ * depend on the other sets or options of the call.  Model parameters are not validated (a NaN gives NaN).
+ * DHJ_ERR_ARG: P, M, n_steps, n_obs or n_paths < 1, n_steps > 2^28, n_steps not a multiple of n_obs, T not finite and
+ * > 0, M > DHJ_MC_MAX_OPTIONS, an unknown kind, a strike not finite and >= 0, a barrier option without a finite
+ * barrier > 0, a null array (other than barrier / out_stderr), s0_stride not 0 or 1.  Host arrays, synchronous. */
+#define DHJ_MC_EUROPEAN 0
+#define DHJ_MC_ASIAN 1
+#define DHJ_MC_UP_OUT 2
+#define DHJ_MC_UP_IN 3
+#define DHJ_MC_DOWN_OUT 4
+#define DHJ_MC_DOWN_IN 5
+#define DHJ_MC_MAX_OPTIONS 64
+DHJ_API int dhj_mc_price(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride,
+                         double r, double q, double T, int32_t n_steps, int32_t n_obs, int32_t M,
+                         const int32_t* kind, const int32_t* is_call, const double* strike, const double* barrier,
+                         uint64_t seed, int64_t n_paths, double* out_price, double* out_stderr);
+
 /* ---- checked build -----------------------------------------------------------------------------
  * lib/libdhj_checked.so is the same library compiled with -DDHJ_CHECKED: the kernels verify their own shared-memory
  * protocol (a stage of coefficients read before it was written / overwritten before it was consumed, an item record

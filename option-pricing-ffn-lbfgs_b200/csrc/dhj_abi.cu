@@ -19,6 +19,7 @@
 #include "dhj_generate.cuh"
 #include "dhj_iv.cuh"
 #include "dhj_ivloss.cuh"
+#include "dhj_mc.cuh"
 
 using namespace dhj;
 
@@ -165,6 +166,7 @@ struct dhj_ctx {
   PinBuf h_x, h_res;
   size_t counters_zeroed = 0;
   DevBuf d_peak;
+  DevBuf d_mc_in, d_mc_part, d_mc_out;          // dhj_mc_price: inputs, chunk partials + carried sums, outputs
   // device buffers of destroyed markets, kept for the next dhj_market_create: cudaMalloc / cudaFree synchronise the
   // whole device, which stalls the other lock-step pipelines of a calibrate_many call every time a market comes or goes
   std::vector<DevBuf> pool;
@@ -738,6 +740,7 @@ int dhj_destroy(dhj_ctx* ctx) {
   ctx->d_x.release(); ctx->d_xv.release(); ctx->d_idx.release(); ctx->d_f.release(); ctx->d_fg.release();
   ctx->d_counters.release(); ctx->d_prices.release(); ctx->d_jac.release(); ctx->h_x.release(); ctx->h_res.release();
   ctx->d_peak.release(); ctx->d_ivres.release();
+  ctx->d_mc_in.release(); ctx->d_mc_part.release(); ctx->d_mc_out.release();
   for (DevBuf& b : ctx->pool) b.release();
   ctx->pool.clear();
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -1629,6 +1632,114 @@ int dhj_generate(dhj_ctx* ctx, uint64_t seed, int64_t first, int64_t n, int32_t 
     DHJ_CUDA(ctx, cudaEventSynchronize(sl.done));
     sl.drain_pieces(host_copy);
   }
+  return DHJ_OK;
+}
+
+}  // extern "C"
+
+// ---- Monte Carlo pricing of path-dependent options (dhj_mc.cuh) ------------------------------------
+namespace {
+
+int check_mc(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride, double T,
+             int32_t n_steps, int32_t n_obs, int32_t M, const int32_t* kind, const int32_t* is_call,
+             const double* strike, const double* barrier, int64_t n_paths, const double* out_price) {
+  if (!ctx) return fail(nullptr, DHJ_ERR_ARG, "null context");
+  if (!params || !S0 || !kind || !is_call || !strike || !out_price) return fail(ctx, DHJ_ERR_ARG, "null array");
+  if (P < 1 || M < 1 || n_paths < 1)
+    return fail(ctx, DHJ_ERR_ARG, "P, M and n_paths must be >= 1 (got %lld, %d, %lld)", (long long)P, M,
+                (long long)n_paths);
+  if (M > mc::kMcMaxOptions) return fail(ctx, DHJ_ERR_ARG, "M must be <= %d (got %d)", mc::kMcMaxOptions, M);
+  if (s0_stride != 0 && s0_stride != 1) return fail(ctx, DHJ_ERR_ARG, "s0_stride must be 0 or 1");
+  if (n_steps < 1 || n_obs < 1 || n_steps > mc::kMcMaxSteps || n_steps % n_obs != 0)
+    return fail(ctx, DHJ_ERR_ARG, "need 1 <= n_obs, n_obs | n_steps, n_steps <= %d (got n_steps %d, n_obs %d)",
+                mc::kMcMaxSteps, n_steps, n_obs);
+  if (!(std::isfinite(T) && T > 0.0)) return fail(ctx, DHJ_ERR_ARG, "T must be finite and > 0 (got %g)", T);
+  for (int m = 0; m < M; ++m) {
+    if (kind[m] < 0 || kind[m] >= mc::kMcKinds) return fail(ctx, DHJ_ERR_ARG, "option %d: unknown kind %d", m, kind[m]);
+    if (!(std::isfinite(strike[m]) && strike[m] >= 0.0))
+      return fail(ctx, DHJ_ERR_ARG, "option %d: strike must be finite and >= 0 (got %g)", m, strike[m]);
+    if (kind[m] >= mc::kUpOut && !(barrier && std::isfinite(barrier[m]) && barrier[m] > 0.0))
+      return fail(ctx, DHJ_ERR_ARG, "option %d: a barrier option needs a finite barrier > 0", m);
+  }
+  return DHJ_OK;
+}
+
+// (chunk, option) partials the scratch holds at once; DHJ_MC_SCRATCH_ENTRIES (developer knob) lowers it so that the
+// split paths of the host loop can be exercised at small sizes
+int64_t mc_scratch_entries() {
+  const char* e = getenv("DHJ_MC_SCRATCH_ENTRIES");
+  const long long v = e ? atoll(e) : 0;
+  return v > 0 ? (int64_t)v : ((int64_t)1 << 22);
+}
+
+}  // namespace
+
+extern "C" {
+
+int dhj_mc_price(dhj_ctx* ctx, const double* params, int64_t P, const double* S0, int64_t s0_stride, double r,
+                 double q, double T, int32_t n_steps, int32_t n_obs, int32_t M, const int32_t* kind,
+                 const int32_t* is_call, const double* strike, const double* barrier, uint64_t seed, int64_t n_paths,
+                 double* out_price, double* out_stderr) {
+  int rc = check_mc(ctx, params, P, S0, s0_stride, T, n_steps, n_obs, M, kind, is_call, strike, barrier, n_paths,
+                    out_price);
+  if (rc) return rc;
+  DHJ_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  // inputs: params[P][13] | S0 | options (kind, is_call)[M] | (strike, barrier)[M]
+  const size_t pb = (size_t)P * kNumParams * sizeof(double), sb = (size_t)(s0_stride ? P : 1) * sizeof(double);
+  const size_t ob = (size_t)M * 2 * sizeof(int32_t), kb = (size_t)M * 2 * sizeof(double);
+  std::vector<int32_t> opt((size_t)2 * M);
+  std::vector<double> kbar((size_t)2 * M);
+  for (int m = 0; m < M; ++m) {
+    opt[2 * m] = kind[m]; opt[2 * m + 1] = is_call[m] ? 1 : 0;
+    kbar[2 * m] = strike[m]; kbar[2 * m + 1] = (kind[m] >= mc::kUpOut) ? barrier[m] : 0.0;
+  }
+  DHJ_CUDA(ctx, ctx->d_mc_in.reserve(pb + sb + ob + kb));
+  unsigned char* din = (unsigned char*)ctx->d_mc_in.p;
+  DHJ_CUDA(ctx, cudaMemcpyAsync(din, params, pb, cudaMemcpyHostToDevice, st));
+  DHJ_CUDA(ctx, cudaMemcpyAsync(din + pb, S0, sb, cudaMemcpyHostToDevice, st));
+  DHJ_CUDA(ctx, cudaMemcpyAsync(din + pb + sb, opt.data(), ob, cudaMemcpyHostToDevice, st));
+  DHJ_CUDA(ctx, cudaMemcpyAsync(din + pb + sb + ob, kbar.data(), kb, cudaMemcpyHostToDevice, st));
+  // pieces: groups of whole sets while a set's partials fit the scratch, else one set at a time in runs of chunks
+  const int64_t n_chunks = (n_paths + mc::kMcChunk - 1) / mc::kMcChunk;
+  const int64_t cap = std::max<int64_t>(mc::kMcChunk, mc_scratch_entries());
+  const int64_t per_set = n_chunks * M;
+  const int64_t group = per_set <= cap ? std::min<int64_t>(P, cap / per_set) : 1;
+  const int64_t run = per_set <= cap ? n_chunks : std::max<int64_t>(1, cap / M);
+  const size_t part_bytes = (size_t)group * run * M * sizeof(double2);
+  const size_t acc_bytes = (size_t)group * M * 3 * sizeof(double);
+  DHJ_CUDA(ctx, ctx->d_mc_part.reserve(part_bytes + acc_bytes));
+  DHJ_CUDA(ctx, ctx->d_mc_out.reserve((size_t)P * M * 2 * sizeof(double)));
+  double2* d_part = (double2*)ctx->d_mc_part.p;
+  double* d_acc = (double*)((unsigned char*)ctx->d_mc_part.p + part_bytes);
+  double* d_price = (double*)ctx->d_mc_out.p;
+  double* d_stderr = d_price + (size_t)P * M;
+  mc::McArgs a{};
+  a.s0_stride = s0_stride; a.opt = (const int*)(din + pb + sb); a.opt_kb = (const double*)(din + pb + sb + ob);
+  a.r = r; a.q = q; a.dt = T / (double)n_steps; a.n_steps = n_steps; a.n_obs = n_obs; a.M = M; a.seed = seed;
+  a.n_paths = n_paths; a.partial = d_part;
+  mc::McFinalArgs f{};
+  f.partial = d_part; f.acc = d_acc; f.n_paths = n_paths; f.M = M; f.disc = exp(-r * T);
+  for (int64_t p0 = 0; p0 < P; p0 += group) {
+    const int64_t g = std::min(group, P - p0);
+    a.params = (const double*)din + p0 * kNumParams;
+    a.S0 = (const double*)(din + pb) + p0 * s0_stride;
+    a.sets = (int)g;
+    f.sets = (int)g; f.price = d_price + p0 * M; f.stderr_ = d_stderr + p0 * M;
+    for (int64_t c0 = 0; c0 < n_chunks; c0 += run) {
+      const int64_t cn = std::min(run, n_chunks - c0);
+      a.chunk0 = c0; a.chunks = cn;
+      mc::k_mc_paths<<<grid_1d(g * cn), mc::kMcChunk, 0, st>>>(a);
+      DHJ_LAUNCHED(ctx);
+      f.chunk0 = c0; f.chunks = cn; f.first = c0 == 0; f.last = c0 + cn == n_chunks;
+      mc::k_mc_finalize<<<grid_1d((g * M + 127) / 128), 128, 0, st>>>(f);
+      DHJ_LAUNCHED(ctx);
+    }
+  }
+  DHJ_CUDA(ctx, cudaMemcpyAsync(out_price, d_price, (size_t)P * M * sizeof(double), cudaMemcpyDeviceToHost, st));
+  if (out_stderr)
+    DHJ_CUDA(ctx, cudaMemcpyAsync(out_stderr, d_stderr, (size_t)P * M * sizeof(double), cudaMemcpyDeviceToHost, st));
+  DHJ_CUDA(ctx, cudaStreamSynchronize(st));
   return DHJ_OK;
 }
 

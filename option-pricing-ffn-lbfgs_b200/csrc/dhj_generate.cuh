@@ -63,17 +63,23 @@ DHJ_HD void counter_words(uint64_t seed, uint64_t i, uint32_t slot, uint64_t* w0
 DHJ_HD double counter_uniform(uint64_t w) { return (double)(w >> 11) * 1.1102230246251565e-16; }          // 2^-53
 DHJ_HD double counter_uniform_open0(uint64_t w) { return (double)((w >> 11) + 1) * 1.1102230246251565e-16; }
 
-#if defined(__CUDACC__)
-
-// Box-Muller pair of (sample i, slot).  The library's own branch-free log / sqrt / sincos (dhj_fastmath.cuh, <= 1-2 ulp):
-// with libdevice's the noise epilogue was bound by their instruction count at 2.5 TB/s, 38 % of the HBM rate.
-__device__ __forceinline__ void counter_normal_pair(uint64_t seed, uint64_t i, uint32_t slot, double* z0, double* z1) {
-  uint64_t w0, w1;
-  counter_words(seed, i, slot, &w0, &w1);
+// Box-Muller pair of two stream words.  The library's own branch-free log / sqrt / sincos (dhj_fastmath.cuh,
+// <= 1-2 ulp): with libdevice's the noise epilogue was bound by their instruction count at 2.5 TB/s, 38 % of the HBM
+// rate.  Host-compilable, so that the test suite's g++ emulations run the device's arithmetic.
+DHJ_HD void box_muller(uint64_t w0, uint64_t w1, double* z0, double* z1) {
   const double R = fm::sqrt_(-2.0 * fm::log_(counter_uniform_open0(w0)));
   double sn, cs;
   fm::sincos_(6.283185307179586 * counter_uniform(w1), &sn, &cs);
   *z0 = R * cs; *z1 = R * sn;
+}
+
+#if defined(__CUDACC__)
+
+// Box-Muller pair of (sample i, slot)
+__device__ __forceinline__ void counter_normal_pair(uint64_t seed, uint64_t i, uint32_t slot, double* z0, double* z1) {
+  uint64_t w0, w1;
+  counter_words(seed, i, slot, &w0, &w1);
+  box_muller(w0, w1, z0, z1);
 }
 
 struct GenArgs {

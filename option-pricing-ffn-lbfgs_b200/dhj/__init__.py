@@ -8,10 +8,10 @@ The drop-in replacements for the reference's modules live beside this package un
 (src/models/double_heston.py, src/calibration/lbfgs_calibrator.py, src/data/synthetic_generator.py).
 """
 from ._native import (BatchLBFGS, Context, Market, NativeError, default_context, generator_draws, load_library, set_host_threads, EXPORTS,
-                      LIB_PATH, N_PARAMS, N_GREEKS, GREEKS, IV_STATUS, FD_POINTS)
+                      LIB_PATH, N_PARAMS, N_GREEKS, GREEKS, IV_STATUS, FD_POINTS, MC_KINDS)
 
 __all__ = ["BatchLBFGS", "Context", "Market", "NativeError", "default_context", "generator_draws", "load_library", "set_host_threads",
-           "EXPORTS", "LIB_PATH", "N_PARAMS", "N_GREEKS", "GREEKS", "IV_STATUS", "FD_POINTS"]
+           "EXPORTS", "LIB_PATH", "N_PARAMS", "N_GREEKS", "GREEKS", "IV_STATUS", "FD_POINTS", "MC_KINDS"]
 from .calibrate_many import calibrate_many, calibrate_many_sharded, initial_guesses  # noqa: E402
 
 __all__ += ["calibrate_many", "calibrate_many_sharded", "initial_guesses"]

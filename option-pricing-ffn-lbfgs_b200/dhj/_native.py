@@ -32,10 +32,12 @@ EXPORTS = (
     "dhj_generator_draws", "dhj_generate_dev", "dhj_generate", "dhj_set_host_threads", "dhj_debug_checks",
     "dhj_price_jacobian", "dhj_loss_grad", "dhj_lbfgs_minimize_grad", "dhj_price_greeks",
     "dhj_implied_vol", "dhj_implied_vol_dev", "dhj_bs_price",
-    "dhj_market_set_objective", "dhj_market_implied_vols",
+    "dhj_market_set_objective", "dhj_market_implied_vols", "dhj_mc_price",
 )
 # calibration objectives of a Market (dhj_market_set_objective)
 OBJECTIVES = {"price": 0, "iv": 1}
+# option kinds of mc_price, in the order of their codes (DHJ_MC_* in include/dhj.h)
+MC_KINDS = ("european", "asian", "up-and-out", "up-and-in", "down-and-out", "down-and-in")
 
 
 class NativeError(RuntimeError):
@@ -126,6 +128,8 @@ def load_library(path: str | None = None) -> ctypes.CDLL:
         lib.dhj_generate_dev.argtypes = gen_head + [_c_vp] * 6
         lib.dhj_generate.argtypes = gen_head + [_c_vp] * 5
         lib.dhj_set_host_threads.argtypes = [_c_i32]
+        lib.dhj_mc_price.argtypes = [_c_vp, _F64, _c_i64, _F64, _c_i64, _c_f64, _c_f64, _c_f64, _c_i32, _c_i32, _c_i32,
+                                     _I32, _I32, _F64, _c_vp, _c_u64, _c_i64, _F64, _c_vp]
         lib.dhj_debug_checks.argtypes = [_c_vp, ctypes.POINTER(_c_i32), ndpointer(dtype=np.uint64, flags="C_CONTIGUOUS")]
         for name in EXPORTS:
             if name not in ("dhj_last_error",):
@@ -344,6 +348,44 @@ class Context:
                                                      float(q), strikes, strikes.size, maturities, maturities.size,
                                                      int(bool(scale_by_spot)), int(bool(is_call)), int(N), float(L),
                                                      d_out, stream or None), "dhj_price_grid_dev")
+
+    # -- Monte Carlo pricing of path-dependent options -------------------------------------------
+    def mc_price(self, params, S0, T, kind, is_call, strike, r, q=0.0, barrier=None, n_paths=1 << 20, n_steps=252,
+                 n_obs=None, seed=0):
+        """(price float64[P, M], stderr float64[P, M]): Monte Carlo prices of M options of one maturity T under P
+        parameter sets (dhj_mc_price).  kind[M]: names from MC_KINDS or their codes; is_call[M], strike[M] and
+        barrier[M] (needed for the barrier kinds; NaN or anything elsewhere) broadcast to M; S0 a scalar or [P].
+        n_steps equal time steps, n_obs equally spaced observation dates (None: every step; must divide n_steps).
+        The draws depend on (seed, path, step) only, so all sets share them and the result is reproducible."""
+        params = _f64(params).reshape(-1, N_PARAMS)
+        P = params.shape[0]
+        S0 = _f64(S0).reshape(-1)
+        if S0.size not in (1, P):
+            raise ValueError("S0 must be a scalar or have one entry per parameter set")
+        kinds = np.atleast_1d(np.asarray(kind, dtype=object))
+        strike = np.atleast_1d(_f64(strike))
+        M = max(kinds.size, strike.size, np.size(is_call), 1 if barrier is None else np.size(barrier))
+        codes = np.empty(kinds.size, dtype=np.int32)
+        for i, k in enumerate(kinds):
+            if isinstance(k, str):
+                if k not in MC_KINDS:
+                    raise ValueError(f"unknown option kind {k!r}: expected one of {MC_KINDS}")
+                codes[i] = MC_KINDS.index(k)
+            else:
+                codes[i] = int(k)
+        codes = np.ascontiguousarray(np.broadcast_to(codes, (M,)))
+        strike = np.ascontiguousarray(np.broadcast_to(strike, (M,)))
+        call = _is_call(is_call, M)
+        bar = None if barrier is None else np.ascontiguousarray(np.broadcast_to(_f64(barrier), (M,)))
+        n_steps = int(n_steps)
+        n_obs = n_steps if n_obs is None else int(n_obs)
+        price, err = np.empty((P, M)), np.empty((P, M))
+        with self._lock:
+            self._check(self._lib.dhj_mc_price(self._h, params, P, S0, 0 if S0.size == 1 else 1, float(r), float(q),
+                                               float(T), n_steps, n_obs, M, codes, call, strike,
+                                               None if bar is None else _ptr(bar), int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                               int(n_paths), price, _ptr(err)), "dhj_mc_price")
+        return price, err
 
     # -- synthetic dataset sweep (counter stream) ------------------------------------------------
     @staticmethod

@@ -5,6 +5,9 @@ Same class, constructor signature, attribute names and method names as the refer
 libdhj.so (ctypes, include/dhj.h); there is no NumPy re-implementation here and no CPU fallback: if
 the library or the device is missing, construction of the first object raises `dhj.NativeError`.
 
+`monte_carlo` (extension) prices the same option's path-dependent variants (Asian, discretely monitored barriers) by
+simulation on the device.
+
 One object still prices ONE option, as in the reference; batches should use `dhj.Context.price_grid`
 / `price_list` (or the calibrator / generator drop-ins, which batch internally).
 """
@@ -113,3 +116,15 @@ class DoubleHeston():
         price = self._ctx.price_list(self._params(), self.S0, [self.K], [self.T], [self._is_call()], self.r, self.q, N)
         vol = self._ctx.implied_vol(price, self.S0, [self.K], [self.T], [self._is_call()], self.r, self.q)
         return np.float64(vol[0, 0])
+
+    def monte_carlo(self, kind="european", barrier=None, n_paths=1 << 20, n_steps=None, n_obs=None, seed=0):
+        """(price, stderr): Monte Carlo price of a path-dependent option at the same S0, K, T, r, q and option type
+        (extension, not in the reference).  kind: one of dhj.MC_KINDS ("european", "asian", "up-and-out",
+        "up-and-in", "down-and-out", "down-and-in"); barrier B for the barrier kinds; n_steps equal steps of the
+        full-truncation Euler scheme (default ceil(252 T)); n_obs observation dates for the average and the barrier
+        (default every step; must divide n_steps).  The scheme is discrete: see dhj.Context.mc_price."""
+        if n_steps is None:
+            n_steps = max(1, int(np.ceil(252 * self.T)))
+        price, err = self._ctx.mc_price(self._params(), self.S0, self.T, [kind], [self._is_call()], [self.K], self.r,
+                                        self.q, None if barrier is None else [barrier], n_paths, n_steps, n_obs, seed)
+        return np.float64(price[0, 0]), np.float64(err[0, 0])
