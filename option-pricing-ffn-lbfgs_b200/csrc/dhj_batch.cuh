@@ -80,16 +80,24 @@ struct BatchSmemT {
   ItemRec items[ITEMS];
   ExtraPass extra[kBatchWarps];
   CoefStage stage[kBatchWarps];
-  fm::Tables ltab;                 // fm::log_tab / exp_tab / atan2_tab tables (per-lane index: shared memory, not the constant bank)
+  fm::TrigTables ltab;             // fm::log_tab / exp_tab / atan2_tab / sincos_tab tables (per-lane index: shared memory, not the constant bank)
 };
 using PriceSmem = BatchSmemT<kPriceItems>;
 
 struct PriceArgs;                  // dhj_kernels.cuh
 
-// every block copies the lookup tables into its shared memory once
+// every block copies the lookup tables into its shared memory once (THREADS: the block size)
+template <int THREADS>
 __device__ __forceinline__ void load_log_table(fm::Tables* dst, int tid) {
-  if (tid < 64) { dst->log[tid] = fm::kTables.log[tid]; dst->exp2[tid] = fm::kTables.exp2[tid]; }
-  if (tid < 65) dst->atan64[tid] = fm::kTables.atan64[tid];
+  for (int i = tid; i < 65; i += THREADS) {
+    if (i < 64) { dst->log[i] = fm::kTables.log[i]; dst->exp2[i] = fm::kTables.exp2[i]; }
+    dst->atan64[i] = fm::kTables.atan64[i];
+  }
+}
+template <int THREADS>
+__device__ __forceinline__ void load_log_table(fm::TrigTables* dst, int tid) {
+  load_log_table<THREADS>(static_cast<fm::Tables*>(dst), tid);
+  for (int i = tid; i < fm::kSinCosTab; i += THREADS) dst->sincos[i] = fm::kTables.sincos[i];
 }
 
 // checked build: the stage's epoch bookkeeping starts at zero
@@ -159,9 +167,9 @@ __device__ __forceinline__ void tag_item(ItemRec& rec, unsigned long long batch_
 }
 
 // The quantities that are trigonometric functions of an angle LINEAR in k — the jump term's (cos, sin)(u_k mu)
-// and the contraction segments' start (cos, sin)(k theta_j) — are evaluated exactly in the first block of 32 k
-// and then advanced from block to block by one plane rotation (4 FP64 instructions instead of a 19 + 17
-// instruction sincos); every kReseed-th block starts from an exact evaluation again (error growth <= kReseed ulp).
+// and the contraction segments' start (cos, sin)(k theta_j) — are evaluated in full in the first block of 32 k
+// (fm::sincos_tab) and then advanced from block to block by one plane rotation (4 FP64 instructions instead of a
+// 17-instruction sincos_tab); every kReseed-th block starts from an exact evaluation again (error growth <= kReseed ulp).
 constexpr int kReseed = 8;
 
 __device__ __forceinline__ void rotate(double& c, double& s, double cr, double sr) {
@@ -178,7 +186,7 @@ __device__ __forceinline__ void contract_pass(const ItemRec& it, const PassConst
                                               const double* __restrict__ sth, const double* __restrict__ c32,
                                               const double* __restrict__ s32, const double* __restrict__ cmu_smu,
                                               unsigned mask, int n_cos, int lane, CoefStage& st,
-                                              const fm::Tables* __restrict__ ltab, double& acc) {
+                                              const fm::TrigTables* __restrict__ ltab, double& acc) {
   constexpr int kSeg = 8, kNumSeg = 32 / kSeg;
   const int slot_pq = lane + (lane >> 3), slot_r = lane + 2 * (lane >> 3);      // padded stage slots of this lane's k
   // A1, A2 feed calls, A3 puts (uniform per pass)
@@ -196,7 +204,7 @@ __device__ __forceinline__ void contract_pass(const ItemRec& it, const PassConst
     const double u = u_of_k(pc, k);
     KTerm t = make_kterm_f(it.set, pc, k, ltab, u, [&](double* cj_out, double* sj_out, double* ej_out) {
       if (exact) {
-        fm::sincos_(u * it.set.mu, &sj, &cj);
+        fm::sincos_tab(u * it.set.mu, ltab, &sj, &cj);
         ej = jump_gauss(it.set, u, ltab);
         rho = fm::exp_tab_neg(-(jump_alpha(pc, it.set.hsj2) * (double)(64 * k + 1024)), ltab);
       } else {
@@ -228,7 +236,7 @@ __device__ __forceinline__ void contract_pass(const ItemRec& it, const PassConst
     for (int i = 0; i < kSeg; ++i) DHJ_CHECK(st.wtag[s * kSeg + i] == epoch, kChkReadBeforeWrite);
 #endif
     if ((mask >> j) & 1u) {
-      if (exact) fm::sincos_(u_of_k(pc, k0 + s * kSeg) * (it.x[j] - pc.a), &sn, &cs);
+      if (exact) fm::sincos_tab(u_of_k(pc, k0 + s * kSeg) * (it.x[j] - pc.a), ltab, &sn, &cs);
       else rotate(cs, sn, c32[j], s32[j]);
       double spq, sr;
       segment_sums<kSeg>(st.PQ + s * (kSeg + 1), reinterpret_cast<const Pair*>(st.R + s * (kSeg + 2)), cs, sn, cth[j],

@@ -41,7 +41,7 @@ struct DenseWarp {
 
 struct DenseSmem {
   DenseWarp w[kDenseWarps];
-  fm::Tables ltab;
+  fm::TrigTables ltab;
 };
 
 // prologue of one item by its warp (see the header)
@@ -99,14 +99,14 @@ struct JumpState { double cj = 1.0, sj = 0.0, ej = 1.0, rho = 1.0; };
 // shares of A1, A2, A3 accumulate in a1, a2, a3; g0 (k = 0 only) is broadcast in the first block
 __device__ __forceinline__ void dense_coefficients(DenseWarp& W, const PassConsts& pc, const double* __restrict__ jrot,
                                                    JumpState& js, int k0, int n_cos, int lane,
-                                                   const fm::Tables* __restrict__ ltab, double& a1, double& a2,
+                                                   const fm::TrigTables* __restrict__ ltab, double& a1, double& a2,
                                                    double& a3, double& g0) {
   const int k = k0 + lane;
   const bool exact = ((k0 >> 5) % kReseed) == 0;        // uniform
   const double u = u_of_k(pc, k);
   KTerm t = make_kterm_f(W.set, pc, k, ltab, u, [&](double* cj_out, double* sj_out, double* ej_out) {
     if (exact) {
-      fm::sincos_(u * W.set.mu, &js.sj, &js.cj);
+      fm::sincos_tab(u * W.set.mu, ltab, &js.sj, &js.cj);
       js.ej = jump_gauss(W.set, u, ltab);
       js.rho = fm::exp_tab_neg(-(jump_alpha(pc, W.set.hsj2) * (double)(64 * k + 1024)), ltab);
     } else {
@@ -143,7 +143,7 @@ __device__ __forceinline__ void dense_consumed(DenseWarp& W, int lane) {
 
 // regular pass: all strikes of the chunk whose widening does not bind, a lane per strike, rounds of 32
 __device__ __forceinline__ void dense_pass(DenseWarp& W, int cnt, int n_cos, int lane,
-                                           const fm::Tables* __restrict__ ltab) {
+                                           const fm::TrigTables* __restrict__ ltab) {
   const PassConsts& pc = W.pass;
   double a1 = 0.0, a2 = 0.0, a3 = 0.0, g0 = 0.0;
   JumpState js;
@@ -158,8 +158,8 @@ __device__ __forceinline__ void dense_pass(DenseWarp& W, int cnt, int n_cos, int
     for (; t + 32 < cnt; t += 64) {
       const int tb = t + 32;
       double sna, csa, snb, csb, spqa, sra, spqb, srb;
-      fm::sincos_(u0 * (W.x[t] - pc.a), &sna, &csa);
-      fm::sincos_(u0 * (W.x[tb] - pc.a), &snb, &csb);
+      fm::sincos_tab(u0 * (W.x[t] - pc.a), ltab, &sna, &csa);
+      fm::sincos_tab(u0 * (W.x[tb] - pc.a), ltab, &snb, &csb);
       segment_sums2<32>(W.stage.PQ, reinterpret_cast<const Pair*>(W.stage.R), csa, sna, W.cth[t], W.sth[t], csb, snb,
                         W.cth[tb], W.sth[tb], &spqa, &sra, &spqb, &srb);
       if (!W.bind[t]) W.part[t] += fma(W.K[t], sra, -(W.sex[t] * spqa));
@@ -167,7 +167,7 @@ __device__ __forceinline__ void dense_pass(DenseWarp& W, int cnt, int n_cos, int
     }
     if (t < cnt && !W.bind[t]) {
       double sn, cs, spq, sr;
-      fm::sincos_(u0 * (W.x[t] - pc.a), &sn, &cs);
+      fm::sincos_tab(u0 * (W.x[t] - pc.a), ltab, &sn, &cs);
       segment_sums<32>(W.stage.PQ, reinterpret_cast<const Pair*>(W.stage.R), cs, sn, W.cth[t], W.sth[t], &spq, &sr);
       W.part[t] += fma(W.K[t], sr, -(W.sex[t] * spq));
     }
@@ -181,7 +181,7 @@ __device__ __forceinline__ void dense_pass(DenseWarp& W, int cnt, int n_cos, int
 
 // pass of ONE strike with its own (a, b): four lanes contract 8-term segments, as in the batch kernel
 __device__ __forceinline__ void dense_pass_single(DenseWarp& W, int t, int n_cos, int lane,
-                                                  const fm::Tables* __restrict__ ltab) {
+                                                  const fm::TrigTables* __restrict__ ltab) {
   if (lane == 0) {
     W.extra_pass = make_pass_consts(W.set, py_min(W.a0, W.x[t] - 0.1), py_max(W.b0, W.x[t] + 0.1), W.pass.T);
     fm::sincos_(u_one(W.extra_pass) * (W.x[t] - W.extra_pass.a), &W.extra_sth, &W.extra_cth);
@@ -198,7 +198,7 @@ __device__ __forceinline__ void dense_pass_single(DenseWarp& W, int t, int n_cos
     double val = 0.0;
     if (lane < 4) {
       double sn, cs, spq, sr;
-      fm::sincos_(u_of_k(pc, k0 + 8 * lane) * (W.x[t] - pc.a), &sn, &cs);
+      fm::sincos_tab(u_of_k(pc, k0 + 8 * lane) * (W.x[t] - pc.a), ltab, &sn, &cs);
       segment_sums<8>(W.stage.PQ + 8 * lane, reinterpret_cast<const Pair*>(W.stage.R + 8 * lane), cs, sn, W.extra_cth,
                       W.extra_sth, &spq, &sr);
       val = fma(W.K[t], sr, -(W.sex[t] * spq));

@@ -221,11 +221,7 @@ template <class Ch>
 __device__ __forceinline__ void chan_items(const SliceView& v, const typename Ch::Args& a) {
   __shared__ ChanSmem<Ch> sm;
   const int tid = threadIdx.x;
-  // (load_log_table assumes >= 65 threads: the block has 64, so the tables are copied in a strided loop)
-  for (int i = tid; i < 65; i += 32 * kJacWarps) {
-    if (i < 64) { sm.ltab.log[i] = fm::kTables.log[i]; sm.ltab.exp2[i] = fm::kTables.exp2[i]; }
-    sm.ltab.atan64[i] = fm::kTables.atan64[i];
-  }
+  load_log_table<32 * kJacWarps>(&sm.ltab, tid);
 #if defined(DHJ_CHECKED)
   sm.w[tid >> 5].wtag[tid & 31] = 0u; sm.w[tid >> 5].rtag[tid & 31] = 0u;
   if ((tid & 31) == 0) sm.w[tid >> 5].epoch = 0u;

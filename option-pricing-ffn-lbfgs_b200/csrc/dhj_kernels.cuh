@@ -37,7 +37,7 @@ template <bool FULL>
 __global__ void __launch_bounds__(kBatchThreads, DHJ_BATCH_MINB) k_price_batch(SliceView v, PriceArgs a) {
   __shared__ PriceSmem sm;
   const int tid = threadIdx.x;
-  load_log_table(&sm.ltab, tid);
+  load_log_table<kBatchThreads>(&sm.ltab, tid);
   stage_check_init(sm.stage[tid >> 5], tid & 31);
   const long long n_items = a.P * (long long)v.n_slices;
   const int ipb = FULL ? kPriceItems : a.items_per_batch;
@@ -86,7 +86,7 @@ __global__ void __launch_bounds__(32 * kDenseWarps, DHJ_DENSE_MINB) k_price_dens
   extern __shared__ __align__(16) unsigned char dense_smem_raw[];
   DenseSmem& sm = *reinterpret_cast<DenseSmem*>(dense_smem_raw);
   const int tid = threadIdx.x;
-  load_log_table(&sm.ltab, tid);
+  load_log_table<32 * kDenseWarps>(&sm.ltab, tid);
   stage_check_init(sm.w[tid >> 5].stage, tid & 31);
   __syncthreads();
   const int warp = __shfl_sync(kFullMask, tid >> 5, 0), lane = tid & 31;
@@ -164,7 +164,7 @@ __global__ void __launch_bounds__(kBatchThreads, DHJ_BATCH_MINB) k_loss_batch(Sl
   __shared__ PriceSmem sm;
   __shared__ double s_feller[kPriceItems];
   const int tid = threadIdx.x;
-  load_log_table(&sm.ltab, tid);
+  load_log_table<kBatchThreads>(&sm.ltab, tid);
   stage_check_init(sm.stage[tid >> 5], tid & 31);
   const int nS = v.n_slices;
   const long long n_batches = (a.n_units + a.units_per_batch - 1) / a.units_per_batch;

@@ -183,7 +183,7 @@ DHJ_HD PassConsts make_pass_consts(const SetConsts& s, double a, double b, doubl
 // resource): aR, aI += A_j without its -2 c_j i arg(.) part, which goes to sli += c_j arg(.);
 // xbr, xbi += B_j v0_j.  Scalars are folded: B_j v0_j = -(v0 u) (u + i) (1-E) conj(D) |D|^-2 (m pl = -sigma^2 u (u+i)), and
 // -2 log|D/(2d)| = log(4 |z| / |D|^2) comes straight from the table-driven log (the 4 is an exponent offset).
-DHJ_HD void heston_factor(const SetConsts& s, int j, double u, double T, const fm::Tables* __restrict__ ltab,
+DHJ_HD void heston_factor(const SetConsts& s, int j, double u, double T, const fm::TrigTables* __restrict__ ltab,
                           double& aR, double& aI, double& sli, double& xbr, double& xbi) {
   const double kap = s.kappa[j];
   const double bi = -(s.rs[j] * u);                 // Im beta
@@ -217,7 +217,7 @@ DHJ_HD void heston_factor(const SetConsts& s, int j, double u, double T, const f
   // (integer underflow test: if -dr T is NaN so is beta - d, and with it D and the factor's whole contribution)
   const double er = fm::exp_tab_neg_ix(-dr * T, ltab);
   double sn, cs;
-  fm::sincos_(-di * T, &sn, &cs);
+  fm::sincos_tab(-di * T, ltab, &sn, &cs);
   const double Er = er * cs, Ei = er * sn;
   const double mr = kap - dr, mi = bi - di;         // beta - d
   const double pr = kap + dr, pi_ = bi + di;        // beta + d
@@ -258,7 +258,7 @@ DHJ_HD double jump_gauss(const SetConsts& s, double u, const fm::Tables* __restr
 }
 
 template <class JumpTrig>
-DHJ_HD void cf_exponent_f(const SetConsts& s, double u, double T, double lamT, const fm::Tables* __restrict__ ltab,
+DHJ_HD void cf_exponent_f(const SetConsts& s, double u, double T, double lamT, const fm::TrigTables* __restrict__ ltab,
                           JumpTrig jump_trig, double* xr_out, double* xi_out) {
   double aR = 0.0, aI = (s.drift * u) * T, sli = 0.0, xbr = 0.0, xbi = 0.0;
 #pragma unroll
@@ -272,7 +272,7 @@ DHJ_HD void cf_exponent_f(const SetConsts& s, double u, double T, double lamT, c
   *xr_out = xr; *xi_out = xi;
 }
 
-DHJ_HD void cf_exponent(const SetConsts& s, double u, double T, double lamT, const fm::Tables* __restrict__ ltab,
+DHJ_HD void cf_exponent(const SetConsts& s, double u, double T, double lamT, const fm::TrigTables* __restrict__ ltab,
                         double* xr_out, double* xi_out) {
   cf_exponent_f(s, u, T, lamT, ltab, [&](double* cj, double* sj, double* ej) {
     fm::sincos_(u * s.mu, sj, cj);
@@ -473,7 +473,7 @@ DHJ_HD double u_of_k(const PassConsts& p, int k) {
 
 // u = u_k; jump_trig as in cf_exponent_f
 template <class JumpTrig>
-DHJ_HD KTerm make_kterm_f(const SetConsts& s, const PassConsts& p, int k, const fm::Tables* __restrict__ ltab,
+DHJ_HD KTerm make_kterm_f(const SetConsts& s, const PassConsts& p, int k, const fm::TrigTables* __restrict__ ltab,
                           double u, JumpTrig jump_trig) {
   KTerm t;
   t.u = u;
@@ -481,7 +481,7 @@ DHJ_HD KTerm make_kterm_f(const SetConsts& s, const PassConsts& p, int k, const 
   cf_exponent_f(s, u, p.T, p.lamT, ltab, jump_trig, &xr, &xi);
   // Re( cf_heston * cf_jump * e^{-i u a} ) with the three exponentials merged
   // (the k = 0 weight 1/2 of double_heston.py:188 is folded in here: scaling by 2^-1 commutes exactly)
-  t.G = (fm::exp_tab(xr, ltab) * fm::cos_(fma(-u, p.a, xi))) * ((k == 0) ? 0.5 : 1.0);
+  t.G = (fm::exp_tab(xr, ltab) * fm::cos_tab(fma(-u, p.a, xi), ltab)) * ((k == 0) ? 0.5 : 1.0);
   // sin / cos of fl(u (b-a)) = k pi + delta, |delta| <~ 1e-13: sin = (-1)^k delta, cos = (-1)^k exactly in
   // double (what libm returns for this argument), with delta from a two-term pi
   const double kf = (double)k;
@@ -495,7 +495,7 @@ DHJ_HD KTerm make_kterm_f(const SetConsts& s, const PassConsts& p, int k, const 
   return t;
 }
 
-DHJ_HD KTerm make_kterm(const SetConsts& s, const PassConsts& p, int k, const fm::Tables* __restrict__ ltab) {
+DHJ_HD KTerm make_kterm(const SetConsts& s, const PassConsts& p, int k, const fm::TrigTables* __restrict__ ltab) {
   const double u = u_of_k(p, k);
   return make_kterm_f(s, p, k, ltab, u, [&](double* cj, double* sj, double* ej) {
     fm::sincos_(u * s.mu, sj, cj);

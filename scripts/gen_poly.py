@@ -91,6 +91,12 @@ def imm_main():
     fc = lambda z: ((mp.cos(sq(z)) - 1 + z / 2) / z ** 2) if z > mp.mpf("1e-12") else mp.mpf(1) / 24 - z / 720 + z * z / 40320
     c, e = refit_with_fixed_top(fc, mp.mpf(0), Z, 5, 2)
     show("cos: (cos(r) - 1 + z/2)/z^2, top 2 coefficients 32-bit", c, e)
+    # sincos_tab: |r| <= pi/512 after the 512-entry table
+    Zt = (mp.pi / 512) ** 2 * mp.mpf("1.02")
+    c, e = refit_with_fixed_top(fs, mp.mpf(0), Zt, 1, 1)
+    show("sincos_tab sin: (sin(r)/r - 1)/z, z <= (pi/512)^2, top coefficient 32-bit (times z: relative error)", c, e * Zt)
+    c, e = refit_with_fixed_top(fc, mp.mpf(0), Zt, 1, 1)
+    show("sincos_tab cos: (cos(r) - 1 + z/2)/z^2, top coefficient 32-bit (times z^2: absolute error)", c, e * Zt * Zt)
     L = mp.log(2) / 128
     q = lambda r: (mp.exp(r) - 1 - r) / r ** 2 if abs(r) > mp.mpf('1e-15') else mp.mpf(1) / 2 + r / 6 + r * r / 24
     c, e = refit_with_fixed_top(q, -L, L, 3, 1)
